@@ -12,7 +12,10 @@ total): every step's inputs come from HBM.
 
 The headline spreads the rotation's independent batches over two streams (a batch keeps its stream): one
 batch's last envs -- a few worlds with long contact islands -- finish while the next batch's blocks take over
-the SMs.  Short driver windows (--steps 20) are repeated and the per-rank median taken.
+the SMs.  --steps is the number of timed steps; --windows splits them into windows and the per-rank median of
+the time per step is taken.  --dump-outputs DIR writes what the last timed step returned (obs, rewards, done,
+nearest-agent ids, collided flags of the batch it stepped) as .npy files: the inputs are seeded, so two builds
+run with the same arguments can be compared output for output.
 
 N > 1 (torchrun, one rank per GPU): each rank owns its own 4096 envs (weak scaling); envs are
 independent, so the data path has no collective.  Legs beside the headline: the same steps on one stream,
@@ -236,10 +239,11 @@ def default_damping():
 
 
 class Timer(object):
-    """Device timing of step sequences: windows of exactly K steps, each bracketed by a barrier over the ranks and
-    a device synchronisation on both sides and timed with CUDA events on the stream the steps are enqueued from
-    (side streams fork after the start event and join before the stop event).  A rank's figure is the MEDIAN of
-    its windows; the job's figure is the MAX over the ranks."""
+    """Device timing of step sequences: K steps in all, split into windows as evenly as possible, each window
+    bracketed by a barrier over the ranks and a device synchronisation on both sides and timed with CUDA events on
+    the stream the steps are enqueued from (side streams fork after the start event and join before the stop
+    event).  A rank's figure is the MEDIAN over its windows of the time per step; the job's figure is the MAX over
+    the ranks."""
 
     def __init__(self, torch, dist, dev, world):
         self.torch, self.dist, self.dev, self.world = torch, dist, dev, world
@@ -253,9 +257,12 @@ class Timer(object):
         return x
 
     def windows(self, issue, K, n_windows, streams=(), k0=0, after=None):
+        """Issue steps k0 .. k0 + K - 1; returns (ms per step, [ms of each window], next k)."""
         torch = self.torch
+        n_windows = max(1, min(n_windows, K))
+        sizes = [K // n_windows + (w < K % n_windows) for w in range(n_windows)]
         ms, k = [], k0
-        for w in range(n_windows):
+        for n in sizes:
             torch.cuda.synchronize()
             if self.world > 1:
                 self.dist.barrier()
@@ -264,7 +271,7 @@ class Timer(object):
             e0.record()
             for st in streams:
                 st.wait_stream(self.main)      # every stream starts after the start event ...
-            for j in range(K):
+            for j in range(n):
                 issue(k)
                 k += 1
             for st in streams:
@@ -274,13 +281,31 @@ class Timer(object):
             e1.record()
             torch.cuda.synchronize()
             ms.append(e0.elapsed_time(e1))
-        med = statistics.median(ms)
+        med = statistics.median(m / n for m, n in zip(ms, sizes))
         return self.max_over_ranks(med), ms, k
 
 
-def n_windows_for(K):
-    # short driver windows (K = 20 is 0.4 ms) are repeated and the median taken; long ones stand alone
-    return 1 if K >= 400 else max(3, min(25, 500 // max(K, 1)))
+DUMP_LIMIT = 64 << 20   # bytes written by --dump-outputs in all
+
+
+def dump_outputs(path, batch):
+    """The per-step outputs of `batch` (what a caller of the stepped batch reads) as DIR/<name>.npy: float outputs
+    in float32, integer ones in float64 (exact).  Past DUMP_LIMIT a fixed, seeded sample of envs is written;
+    env_index.npy names the envs written either way."""
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+    out = {}
+    for name in batch.engine.OUTPUTS:
+        a = batch.state[name].cpu().numpy()
+        out[name] = a.astype(np.float32 if a.dtype.kind == "f" else np.float64)
+    E = batch.engine.E
+    per_env = sum(a.nbytes for a in out.values()) // E + 8
+    keep = np.arange(E)
+    if per_env * E > DUMP_LIMIT:
+        keep = np.sort(np.random.default_rng(0).choice(E, (DUMP_LIMIT - 4096) // per_env, replace=False))   # 4 KB: .npy headers
+    out["env_index"] = keep.astype(np.float64)
+    for name, a in out.items():
+        np.save(os.path.join(path, name + ".npy"), a if name == "env_index" else a[keep])
 
 
 def main():
@@ -296,7 +321,8 @@ def main():
     ap.add_argument("--streams", type=int, default=2,
                     help="streams the independent batches of the rotation are spread over (a batch keeps its stream); "
                          "2 = a batch's last envs finish while the next batch starts")
-    ap.add_argument("--windows", type=int, default=0, help="timed windows of --steps steps (0 = 25 for short windows, 1 for long)")
+    ap.add_argument("--windows", type=int, default=1,
+                    help="timed windows the --steps steps are split into (the median time per step is reported)")
     ap.add_argument("--no-legs", action="store_true", help="headline + e2e only (no other configs, no exchange legs)")
     ap.add_argument("--cpu-seconds", type=float, default=12.0)
     ap.add_argument("--e2e-steps", type=int, default=240)
@@ -304,7 +330,13 @@ def main():
     ap.add_argument("--policy", default="random", choices=["random", "flock"])
     ap.add_argument("--settle", type=int, default=64, help="untimed steps per batch after the random spawn")
     ap.add_argument("--max-touching", type=int, default=0, help="experiment: capacity of the touching-contact stage (0 = default)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the outputs of the last one to DIR/<name>.npy (float32/float64)")
     args = ap.parse_args()
+    if args.steps < 1 or args.windows < 1:
+        ap.error("--steps and --windows must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the CUDA path's outputs; --impl reference has none to write")
 
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -342,7 +374,7 @@ def main():
             os.close(keep)
     E, N, ROT = args.envs, N_AGENTS, args.rot
     K = args.steps
-    NW = args.windows if args.windows > 0 else n_windows_for(K)
+    NW = min(args.windows, K)
     sampler = ClockSampler(local) if rank == 0 else None   # started early: it is warm when the timed region begins
     T = Timer(torch, dist, dev, world)
     main_stream = T.main
@@ -406,14 +438,15 @@ def main():
         pool.k = 0
     launches0 = sum(s.engine.launch_count for s in sims)
     t0 = time.time()
-    ms_win, ms_all, knext = T.windows(issue, K, NW, streams)
+    ms_per_step, ms_all, knext = T.windows(issue, K, NW, streams)
     t1 = time.time()
     launches = sum(s.engine.launch_count for s in sims) - launches0
     clocks = sampler.stop(t0, t1) if sampler else None
     torch.cuda.synchronize()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, sims[(K - 1) % ROT])   # the batch the last timed step stepped
     for s_ in sims:                  # the legs below name their streams themselves
         s_.engine.stream = None
-    ms_per_step = ms_win / K
     value = world * E * N / (ms_per_step * 1e-3)
 
     legs = {}
@@ -423,7 +456,7 @@ def main():
     if plain and NS > 1:
         T.windows(issue1, min(K, 200), 1)     # warm-up of this shape
         ms1, all1, _ = T.windows(issue1, K, NW)
-        legs["one_stream"] = {"value": world * E * N * K / (ms1 * 1e-3), "unit": UNIT, "ms_per_step": ms1 / K,
+        legs["one_stream"] = {"value": world * E * N / (ms1 * 1e-3), "unit": UNIT, "ms_per_step": ms1,
                                "windows": NW, "note": "the same steps on one stream: no overlap between a batch's "
                                "tail (a few envs with long contact islands) and the next batch"}
     # (2) one launch alone on an idle GPU (synchronised on both sides): the kernel's own duration, read from the
@@ -450,14 +483,14 @@ def main():
     if plain and args.rollout > 0:
         R = min(args.rollout, POOL)
         outs = [sims[0].engine.rollout_buffers(R) for _ in range(2)]
-        n_launch = max(ROT, (min(K * NW, 2000) // R) // ROT * ROT)
+        n_launch = max(ROT, (min(K, 2000) // R) // ROT * ROT)
 
         def roll(j):
             sims[j % ROT].engine.rollout(acts[:R], R, None, 0, outs[j & 1])
         T.windows(roll, ROT, 1)
-        msr, _, _ = T.windows(roll, n_launch, 1)
-        legs["rollout"] = {"value": world * E * N * n_launch * R / (msr * 1e-3), "unit": UNIT,
-                            "ms_per_step": msr / (n_launch * R), "steps_per_launch": R, "launches": n_launch,
+        msr, _, _ = T.windows(roll, n_launch, 1)      # ms per launch of R steps
+        legs["rollout"] = {"value": world * E * N * R / (msr * 1e-3), "unit": UNIT,
+                            "ms_per_step": msr / R, "steps_per_launch": R, "launches": n_launch,
                             "note": "macm_rollout, per-step outputs written every step; bit-identical to single steps "
                                     "(tests/test_gpu_rollout.py)"}
         del outs
@@ -489,9 +522,9 @@ def main():
             s.engine.rollout(act_of(k), 1, None, 0, peer.mine[k & 1], st)
         T.windows(peer_step, min(K, 100), 1, streams)
         msp, _, _ = T.windows(peer_step, K, NW, streams)
-        legs["gather_peer"] = {"value": world * E * N * K / (msp * 1e-3), "unit": UNIT, "ms_per_step": msp / K,
+        legs["gather_peer"] = {"value": world * E * N / (msp * 1e-3), "unit": UNIT, "ms_per_step": msp,
                                 "bytes_into_learner_per_step": nbytes_in,
-                                "learner_ingress_GBps": nbytes_in / (msp / K * 1e-3) / 1e9, "windows": NW,
+                                "learner_ingress_GBps": nbytes_in / (msp * 1e-3) / 1e9, "windows": NW,
                                 "note": "obs+rewards+done of every rank stored into rank 0's buffers by the step kernel "
                                         "itself (gym_macm.dist.PeerGather: NVLink peer stores through CUDA IPC, no collective)"}
         # (b) NCCL all-gather of obs + rewards on a side stream: the next batch steps while this one's outputs travel
@@ -510,10 +543,10 @@ def main():
         def join():
             main_stream.wait_stream(gstream)
         T.windows(nccl_step, min(K, 50), 1, after=join)
-        msn, _, _ = T.windows(nccl_step, K, max(3, NW // 3), after=join)
-        legs["gather_nccl"] = {"value": world * E * N * K / (msn * 1e-3), "unit": UNIT, "ms_per_step": msn / K,
+        msn, _, _ = T.windows(nccl_step, K, NW, after=join)
+        legs["gather_nccl"] = {"value": world * E * N / (msn * 1e-3), "unit": UNIT, "ms_per_step": msn,
                                 "bytes_into_every_rank_per_step": (world - 1) * E * N * 20,
-                                "ingress_GBps": (world - 1) * E * N * 20 / (msn / K * 1e-3) / 1e9,
+                                "ingress_GBps": (world - 1) * E * N * 20 / (msn * 1e-3) / 1e9,
                                 "note": "NCCL all_gather_into_tensor of obs and rewards to every rank, on a side stream"}
         peer.close()
         del gathered, peer
@@ -624,7 +657,8 @@ def main():
             "warmup": args.warmup, "ms_per_step": ms_per_step, "higher_is_better": True, "scaling": "weak",
             "vs_baseline": None, "dtype": "f32", "data": "synthetic",
             "windows": NW, "window_ms": ms_all,
-            "window_agg": "each window = %d steps between barrier+synchronize; per-rank median of %d windows, max over ranks" % (K, NW),
+            "window_agg": "%d steps in %d window(s) between barrier+synchronize; per-rank median of the time per step "
+                          "over the windows, max over ranks" % (K, NW),
             "config": {"workload": WORKLOAD, "envs_per_gpu": E, "agents_per_env": N, "reward_mode": "linear",
                        "actions": "pre-generated on device, U{0,1,2}^3" if args.policy == "random" else "bots.flock on device",
                        "l2": "inputs larger than L2: rotation over %d independent batches (%.0f MB of state+outputs)"
@@ -667,15 +701,14 @@ def other_configs(torch, gym_macm, T, dev, world, rank, K, NW, peak, settle):
             sims[k % ROT].engine.step(acts[(k // ROT + 7 * (k % ROT)) % POOL])
         torch.cuda.synchronize()
         T.windows(issue, min(steps, 4 * ROT), 1, st2)
-        ms, _, _ = T.windows(issue, steps, NW, st2)
+        per, win_ms, _ = T.windows(issue, steps, NW, st2)
         c_bar = float(sum(float(s.state["contact_count"].sum()) for s in sims) / (ROT * E * n_agents))
         b = b_alg_fn(c_bar)
-        per = ms / steps
         ach = b * E * n_agents / (per * 1e-3) / 1e9
         foot = sum(sum(t.numel() * t.element_size() for t in s.state.values()) for s in sims)
         ov = [sum(x) for x in zip(*[s.overflow_count() for s in sims])]
         out[name] = {"workload": workload, "value": world * E * n_agents / (per * 1e-3), "unit": UNIT,
-                     "ms_per_step": per, "steps": steps, "windows": NW, "envs_per_gpu": E, "agents_per_env": n_agents,
+                     "ms_per_step": per, "steps": steps, "windows": len(win_ms), "envs_per_gpu": E, "agents_per_env": n_agents,
                      "batches_in_rotation": ROT, "footprint_MB": foot / 1e6, "contacts_per_agent": c_bar,
                      "bytes_per_agent_step": b, "envs_with_contact_overflow": ov,
                      "roofline": {"bound": "hbm", "achieved": ach, "peak": peak, "unit": "GB/s", "frac": ach / peak}}
@@ -714,11 +747,11 @@ def other_configs(torch, gym_macm, T, dev, world, rank, K, NW, peak, settle):
         def peer_step(k):
             sims[k % 2].engine.rollout(acts[(k // 2 + 7 * (k % 2)) % 31], 1, None, 0, peer.mine[k & 1], st2[k & 1])
         T.windows(peer_step, 4, 1, st2)
-        msp, _, _ = T.windows(peer_step, steps, max(3, NW // 3), st2)
+        msp, _, _ = T.windows(peer_step, steps, NW, st2)
         nb = (world - 1) * (E5 * N5 * 20 + E5)
         out["config5_32768_envs_per_gpu"]["gather_peer"] = {
-            "value": world * E5 * N5 * steps / (msp * 1e-3), "unit": UNIT, "ms_per_step": msp / steps,
-            "bytes_into_learner_per_step": nb, "learner_ingress_GBps": nb / (msp / steps * 1e-3) / 1e9}
+            "value": world * E5 * N5 / (msp * 1e-3), "unit": UNIT, "ms_per_step": msp,
+            "bytes_into_learner_per_step": nb, "learner_ingress_GBps": nb / (msp * 1e-3) / 1e9}
         gathered = [torch.empty((world,) + tuple(sims[0].state[k_].shape), dtype=sims[0].state[k_].dtype, device=dev)
                     for k_ in ("obs", "rewards")]
         gstream = torch.cuda.Stream(device=dev)
@@ -734,11 +767,11 @@ def other_configs(torch, gym_macm, T, dev, world, rank, K, NW, peak, settle):
         def join():
             T.main.wait_stream(gstream)
         T.windows(nccl_step, 4, 1, after=join)
-        msn, _, _ = T.windows(nccl_step, steps, 3, after=join)
+        msn, _, _ = T.windows(nccl_step, steps, NW, after=join)
         out["config5_32768_envs_per_gpu"]["gather_nccl"] = {
-            "value": world * E5 * N5 * steps / (msn * 1e-3), "unit": UNIT, "ms_per_step": msn / steps,
+            "value": world * E5 * N5 / (msn * 1e-3), "unit": UNIT, "ms_per_step": msn,
             "bytes_into_every_rank_per_step": (world - 1) * E5 * N5 * 20,
-            "ingress_GBps": (world - 1) * E5 * N5 * 20 / (msn / steps * 1e-3) / 1e9}
+            "ingress_GBps": (world - 1) * E5 * N5 * 20 / (msn * 1e-3) / 1e9}
         peer.close()
         del gathered, peer
     return out

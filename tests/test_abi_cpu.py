@@ -1,9 +1,10 @@
 """CPU-side checks: libmacm.so loads and exports every symbol include/macm.h declares, the ctypes
 structs match the header, and the host marshalling helpers do what the reference's dict API does.
 No compute call is made (there is no GPU here)."""
-import ctypes as C
 import os
 import re
+import subprocess
+import sys
 
 import numpy as np
 import pytest
@@ -58,21 +59,30 @@ def test_defaults_are_the_reference_settings(built):
     assert (t.cooldown_atk, t.cooldown_mov_penalty, t.melee_range, t.melee_dmg) == (1.0, 0.5, 2.0, 0.25)
 
 
+_NO_DEVICE = r"""
+import ctypes as C
+import pytest
+import gym_macm
+from gym_macm import _lib as built
+with pytest.raises(built.MacmError):
+    gym_macm.BatchedFlock(4, n_agents=[4])
+with pytest.raises(built.MacmError):
+    gym_macm.make("gym_macm:cm-flock-v0", n_agents=[4])
+# macm_create itself refuses without a device
+p = built.default_params(built.FLOCK)
+h = C.c_void_p()
+assert built.lib().macm_create(C.byref(h), C.byref(p), 0) == -2 and not h
+p.n_agents = 129      # MACM_MAX_AGENTS is 128
+assert built.lib().macm_create(C.byref(h), C.byref(p), 0) == -1
+"""
+
+
 def test_no_cpu_fallback(built):
-    import torch
-    if torch.cuda.is_available():
-        pytest.skip("GPU present")
-    import gym_macm
-    with pytest.raises(built.MacmError):
-        gym_macm.BatchedFlock(4, n_agents=[4])
-    with pytest.raises(built.MacmError):
-        gym_macm.make("gym_macm:cm-flock-v0", n_agents=[4])
-    # macm_create itself refuses without a device
-    p = built.default_params(built.FLOCK)
-    h = C.c_void_p()
-    assert built.lib().macm_create(C.byref(h), C.byref(p), 0) == -2 and not h
-    p.n_agents = 129      # MACM_MAX_AGENTS is 128
-    assert built.lib().macm_create(C.byref(h), C.byref(p), 0) == -1
+    # in a child process that sees no CUDA device, so that the check also runs where a GPU is present
+    env = dict(os.environ, CUDA_VISIBLE_DEVICES="",
+               PYTHONPATH=os.pathsep.join([ROOT, os.path.join(ROOT, "gym-macm_b200")]))
+    r = subprocess.run([sys.executable, "-c", _NO_DEVICE], capture_output=True, text=True, env=env, timeout=300)
+    assert r.returncode == 0, r.stderr
 
 
 def test_settings_bag():
