@@ -90,10 +90,14 @@ struct Lay {
     static constexpr int STACK = LABEL + 4 * NC;  // u8     [NC]  DFS stack (intrusive next-pointers on the common path)
     static constexpr int COMP = STACK + NC;       // u8     [NC]  seed body of the k-th island that has contacts
     static constexpr int SOLVED = COMP + NC;      // u8     [NC]  position solver converged for the island seeded here
-    // dense piles only (more touching contacts than lanes, *_big below):
+    // dense piles only (more touching contacts than lanes, dense_* below):
     static constexpr int LASTLVL = SOLVED + NC, ISLACT = LASTLVL + NC, ISLBAD = ISLACT + NC;
     static constexpr int HEAD = ISLBAD + NC;      // u8     [NC]  newest touching contact of a body
-    static constexpr int MISC = (HEAD + NC + 15) / 16 * 16;  // 4 x u32
+    // 4 x u32, used by phases that never overlap in time:
+    //   phase 0 (MACM_BULK_STAGE build)  two mbarriers of the bulk state copies
+    //   phases 5-7 (macm_kernels_huge.cu)  word 0: contacts of a dense pile in the global-memory stage (0: the env is in
+    //                                      the shared-memory stage), from the velocity to the position part
+    static constexpr int MISC = (HEAD + NC + 15) / 16 * 16;
     static constexpr int FIXED = MISC + 16;
     // per touching contact (capacity TC, a multiple of 16):
     //   float2 normal ; float2 impulses ; u32 edge word ; u16 slot ; u16 ord|lvl<<8    = 24 bytes
@@ -891,322 +895,93 @@ __device__ void tdm_observe(const Grp<G>& g, const EnvS<G * APL>& S, const SimCo
     }
 }
 
-#if MACM_HUGE_BUILD
 // ------------------------------------------------------------------------------------------
-// Envs with more touching contacts than the shared-memory stage holds (tc > TC <= 240: overlapping spawn piles; bodies
-// that do not overlap cannot touch more than ~3N others).  With a global-memory stage bound (macm_buffers.touch_scratch,
-// max_touching > 240) such an env is solved here, exactly, in Box2D's island order like the dense-pile path above --
-// 16-bit contact indices and levels, every array in global memory, one lane replaying the traversal.  Cold and slow
-// by design; without the stage the env is flagged MACM_ENV_TOUCH_OVERFLOW instead.
+// Dense piles: environments with more touching contacts than lanes (tc > G).  One lane replays Box2D's depth-first
+// island traversal over per-body edge lists (head-inserted in birth order, like b2ContactManager::AddPair builds them);
+// every contact gets its position in the island order and a level = 1 + max(level of the previous contact of either
+// body).  Contacts of one level share no body and run across lanes.  Rare, and kept out of line so that the common path
+// stays small in the instruction cache.
+//
+// The solver is written once, on a STAGE: where the env's touching contacts live while they are ordered and solved.
+//   SmemStage  the shared-memory stage that phase 2 fills (capacity TC <= 240): the next-links of a contact are bytes of
+//              its edge word, order and level a u16 t | lvl<<8, head / lastlvl a byte per body.
+//   GmemStage  the global-memory stage (macm_buffers.touch_scratch, max_touching > 240; only in the kernels of
+//              macm_kernels_huge.cu): 16-bit links, order and levels.  It takes envs with more than TC touching contacts
+//              -- overlapping spawn piles; bodies that do not overlap cannot touch more than ~3N others.  Without it such
+//              an env is flagged MACM_ENV_TOUCH_OVERFLOW instead.
+// A stage provides edge(t) -> w, a(w) / b(w), next(w, t, body) (the next edge at `body`), link(t, w, next-of-a,
+// next-of-b), taken(w) / take(t, w), ord(k) -> (t, lvl) / set_ord(k, t, lvl), the arrays n, imp (normal and impulses of
+// contact t) and slot (its HBM list index), head / lastlvl (per body), and NONE (end of an edge list).
 // ------------------------------------------------------------------------------------------
-struct HugeStage {
-    float2* n; float2* imp; uint32_t* ew; uint16_t* na; uint16_t* nb; uint16_t* slot; uint32_t* ord; int cap;
-    __device__ HugeStage(const SimConst& P, int env)
-    {
-        unsigned char* b = P.scratch + (size_t)env * P.TCH * 32;
-        const size_t T = (size_t)P.TCH;
-        n = (float2*)b; imp = (float2*)(b + 8 * T); ew = (uint32_t*)(b + 16 * T); na = (uint16_t*)(b + 20 * T);
-        nb = (uint16_t*)(b + 22 * T); slot = (uint16_t*)(b + 24 * T); ord = (uint32_t*)(b + 28 * T); cap = P.TCH;
-    }
+template <int NC>
+struct SmemStage {
+    typedef EW<NC> E;
+    static constexpr int NONE = EW_NONE;
+    uint32_t* ew; uint16_t* ol; float2* n; float2* imp; uint16_t* slot; uint8_t* head; uint8_t* lastlvl;
+    __device__ explicit SmemStage(const EnvS<NC>& S)
+        : ew(S.t_ew()), ol(S.ordlvl()), n(S.t_n()), imp(S.t_imp()), slot(S.t_slot()), head(S.head()), lastlvl(S.lastlvl()) {}
+    __device__ uint32_t edge(int t) const { return ew[t]; }
+    __device__ static int a(uint32_t w) { return E::a(w); }
+    __device__ static int b(uint32_t w) { return E::b(w); }
+    __device__ int next(uint32_t w, int, int body) const { return a(w) == body ? E::na(w) : E::nb(w); }
+    __device__ void link(int t, uint32_t w, int na, int nb) const { ew[t] = w | ((uint32_t)na << E::SH_NA) | ((uint32_t)nb << E::SH_NB); }
+    __device__ static bool taken(uint32_t w) { return (w & E::TAKEN) != 0u; }
+    __device__ void take(int t, uint32_t w) const { ew[t] = w | E::TAKEN; }
+    __device__ int2 ord(int k) const { const int v = ol[k]; return make_int2(v & 0xff, v >> 8); }
+    __device__ void set_ord(int k, int t, int l) const { ol[k] = (uint16_t)(t | (l << 8)); }
 };
-#define HUGE_NONE 0xffffu
-#define HUGE_TAKEN 0x80000000u
 
-// Stages every touching contact of the env's HBM list (birth order), replays the island traversal, solves the velocity
-// constraints and stores the impulses.  Returns the number of levels (bit 30 set when even the global-memory stage
-// was too small), or 0 when the env fits the shared-memory stage after all (exactly TC touching contacts) and nothing
-// was done.
-template <int G, int APL>
-__device__ __noinline__ int solve_velocity_huge(const Grp<G>& g, const EnvS<G * APL>& S, const SimConst& P, int env, int cnt,
-                                                const uint32_t* c_ab, float2* c_imp, float ratio)
-{
-    bool overflow = false;
-    constexpr int NC = G * APL;
-    const float2* pos = S.pos(); float2* vel = S.vel();
-    uint32_t* label = S.label();
-    const HugeStage H(P, env);
-    // 1. stage: edges, HBM slots, impulses (the first TC were staged in shared memory by phase 2, the rest kept theirs in
-    //    the HBM list), world normals at the pre-integration positions, impulses scaled by dtRatio
-    int ht = 0;
-    for (int base = 0; base < cnt; base += G) {
-        const int k = base + g.gl;
-        const uint32_t ab = k < cnt ? c_ab[k] : 0u;
-        const bool touch = (ab >> 16) & 1u;
-        const unsigned tm = g.ballot(touch);
-        const int t = ht + __popc(tm & g.below());
-        if (touch) {
-            if (t < H.cap) {
-                const int a = ab & 0xff, b = (ab >> 8) & 0xff;
-                H.ew[t] = (uint32_t)a | ((uint32_t)b << 8);
-                H.slot[t] = (uint16_t)k;
-                float2 im = t < P.TC ? S.t_imp()[t] : c_imp[k];
-                const float2 pa = pos[a], pb = pos[b];
-                float nx = 1.0f, ny = 0.0f;
-                const float dx = pb.x - pa.x, dy = pb.y - pa.y;
-                if ((dx * dx + dy * dy) > B2_EPSILON * B2_EPSILON) { nx = dx; ny = dy; b2normalize(nx, ny); }
-                if (P.warm_starting) { im.x = ratio * im.x; im.y = ratio * im.y; } else im = make_float2(0.0f, 0.0f);
-                H.n[t] = make_float2(nx, ny);
-                H.imp[t] = im;
-            } else {
-                overflow = true;
-            }
-        }
-        ht += __popc(tm);
+#if MACM_HUGE_BUILD
+// An env's TCH x 32 bytes of touch_scratch: float2 n [TCH] ; float2 imp [TCH] ; u32 edge word a | b<<8 | taken<<31 [TCH] ;
+// u16 next-of-a [TCH] ; u16 next-of-b [TCH] ; u16 slot [TCH] ; (2 x TCH bytes unused) ; u32 t | lvl<<16 [TCH].
+// head / lastlvl are u16 per body in the env's NEW region (shared memory).
+struct GmemStage {
+    static constexpr int NONE = 0xffff;
+    static constexpr uint32_t TAKEN = 0x80000000u;
+    float2* n; float2* imp; uint32_t* ew; uint16_t* na; uint16_t* nb; uint16_t* slot; uint32_t* ol; uint16_t* head; uint16_t* lastlvl;
+    template <int NC>
+    __device__ GmemStage(const EnvS<NC>& S, const SimConst& P, int env)
+    {
+        unsigned char* p = P.scratch + (size_t)env * P.TCH * 32;
+        const size_t T = (size_t)P.TCH;
+        n = (float2*)p; imp = (float2*)(p + 8 * T); ew = (uint32_t*)(p + 16 * T); na = (uint16_t*)(p + 20 * T);
+        nb = (uint16_t*)(p + 22 * T); slot = (uint16_t*)(p + 24 * T); ol = (uint32_t*)(p + 28 * T);
+        head = reinterpret_cast<uint16_t*>(S.nw()); lastlvl = head + NC;
     }
-    if (ht <= P.TC) return 0;   // (uniform) the shared-memory path takes it
-    const int tc = ht < H.cap ? ht : H.cap;
-    // 2. islands: per-body edge lists (head-inserted in birth order), depth-first from the highest body left, edges
-    //    newest-first; every contact gets its place in the island order and a level
-    uint16_t* head = reinterpret_cast<uint16_t*>(S.nw());
-    uint16_t* lastlvl = head + NC;
+    __device__ uint32_t edge(int t) const { return ew[t]; }
+    __device__ static int a(uint32_t w) { return (int)(w & 0xffu); }
+    __device__ static int b(uint32_t w) { return (int)((w >> 8) & 0xffu); }
+    __device__ int next(uint32_t w, int t, int body) const { return a(w) == body ? na[t] : nb[t]; }
+    __device__ void link(int t, uint32_t, int na_, int nb_) const { na[t] = (uint16_t)na_; nb[t] = (uint16_t)nb_; }
+    __device__ static bool taken(uint32_t w) { return (w & TAKEN) != 0u; }
+    __device__ void take(int t, uint32_t w) const { ew[t] = w | TAKEN; }
+    __device__ int2 ord(int k) const { const uint32_t v = ol[k]; return make_int2((int)(v & 0xffffu), (int)(v >> 16)); }
+    __device__ void set_ord(int k, int t, int l) const { ol[k] = (uint32_t)t | ((uint32_t)l << 16); }
+};
+#endif   // MACM_HUGE_BUILD
+
+// Islands of the tc staged contacts: labels (seed body of each body's island), island order and levels.  Returns the
+// number of levels.
+template <int G, int APL, class St>
+__device__ __forceinline__ int dense_islands(const Grp<G>& g, const EnvS<G * APL>& S, const St& st, int tc)
+{
+    uint32_t* label = S.label();
 #pragma unroll
-    for (int s = 0; s < APL; ++s) { head[g.gl + s * G] = HUGE_NONE; lastlvl[g.gl + s * G] = 0; }
+    for (int s = 0; s < APL; ++s) { st.lastlvl[g.gl + s * G] = 0; st.head[g.gl + s * G] = St::NONE; }
     g.sync();
     int L = 1;
     if (g.gl == 0) {
         uint8_t* stack = S.stack();
-        constexpr int W = NC > 64 ? 4 : 2;
-        uint32_t rem[W];
-#pragma unroll
-        for (int w = 0; w < W; ++w) rem[w] = 0u;
-        for (int t = 0; t < tc; ++t) {
-            const uint32_t ew = H.ew[t];
-            const int a = ew & 0xff, b = (ew >> 8) & 0xff;
-            H.na[t] = head[a]; H.nb[t] = head[b];
-            head[a] = (uint16_t)t; head[b] = (uint16_t)t;
-            rem[a >> 5] |= 1u << (a & 31);
-            rem[b >> 5] |= 1u << (b & 31);
-        }
-        int nord = 0;
-        for (;;) {
-            int seed = -1;
-#pragma unroll
-            for (int w = W - 1; w >= 0; --w)
-                if (seed < 0 && rem[w]) seed = w * 32 + 31 - __clz((int)rem[w]);
-            if (seed < 0) break;
-            int sp = 0;
-            stack[sp++] = (uint8_t)seed;
-            rem[seed >> 5] &= ~(1u << (seed & 31));
-            while (sp > 0) {
-                const int b = stack[--sp];
-                label[b] = (uint32_t)seed;
-                for (int t = head[b]; t != HUGE_NONE;) {
-                    const uint32_t ew = H.ew[t];
-                    const int ta = ew & 0xff, tb = (ew >> 8) & 0xff;
-                    const int nx = (ta == b) ? H.na[t] : H.nb[t];
-                    if (!(ew & HUGE_TAKEN)) {
-                        H.ew[t] = ew | HUGE_TAKEN;
-                        const int l = 1 + max((int)lastlvl[ta], (int)lastlvl[tb]);
-                        H.ord[nord++] = (uint32_t)t | ((uint32_t)l << 16);
-                        lastlvl[ta] = (uint16_t)l; lastlvl[tb] = (uint16_t)l;
-                        L = max(L, l);
-                        const int other = (ta == b) ? tb : ta;
-                        const uint32_t ob = 1u << (other & 31);
-                        if (rem[other >> 5] & ob) { rem[other >> 5] &= ~ob; stack[sp++] = (uint8_t)other; }
-                    }
-                    t = nx;
-                }
-            }
-        }
-    }
-    L = g.shfl(L, 0);
-    g.sync();
-    // 3. warm start (it == -1) and the velocity iterations, level by level
-    const float mass_n = P.normal_mass, mass_t = P.normal_mass;
-    for (int it = -1; it < P.vel_iters; ++it) {
-        for (int lev = 1; lev <= L; ++lev) {
-            for (int k = g.gl; k < tc; k += G) {
-                const uint32_t ol = H.ord[k];
-                if ((int)(ol >> 16) != lev) continue;
-                const int t = ol & 0xffff;
-                const uint32_t ew = H.ew[t];
-                const int a = ew & 0xff, b = (ew >> 8) & 0xff;
-                const float2 n = H.n[t];
-                float2 im = H.imp[t];
-                float2 va = vel[a], vb = vel[b];
-                if (it < 0) warm_start(n.x, n.y, im.x, im.y, P.inv_mass, va, vb);
-                else solve_velocity(n.x, n.y, P.friction, mass_n, mass_t, P.inv_mass, im.x, im.y, va, vb);
-                vel[a] = va; vel[b] = vb;
-                H.imp[t] = im;
-            }
-            g.sync();
-        }
-    }
-    // StoreImpulses -> manifold (next step's warm start)
-    for (int t = g.gl; t < tc; t += G) c_imp[H.slot[t]] = H.imp[t];
-    if (g.gl == 0) S.misc()[3] = (uint32_t)tc;   // for solve_position_huge
-    g.sync();
-    return L | (g.ballot(overflow) ? (1 << 30) : 0);
-}
-
-template <int G, int APL>
-__device__ __noinline__ void solve_position_huge(const Grp<G>& g, const EnvS<G * APL>& S, const SimConst& P, int env, int L)
-{
-    float2* pos = S.pos();
-    const uint32_t* label = S.label();
-    uint8_t* isl_act = S.isl_act(); uint8_t* isl_bad = S.isl_bad();
-    const HugeStage H(P, env);
-    const int tc = (int)S.misc()[3];   // how many contacts the velocity part staged
-#pragma unroll
-    for (int s = 0; s < APL; ++s) { isl_act[g.gl + s * G] = 1; isl_bad[g.gl + s * G] = 0; }
-    g.sync();
-    for (int it = 0; it < P.pos_iters; ++it) {
-        for (int lev = 1; lev <= L; ++lev) {
-            for (int k = g.gl; k < tc; k += G) {
-                const uint32_t ol = H.ord[k];
-                if ((int)(ol >> 16) != lev) continue;
-                const uint32_t ew = H.ew[ol & 0xffff];
-                const int a = ew & 0xff, b = (ew >> 8) & 0xff;
-                const int isl = label[a];
-                if (!isl_act[isl]) continue;
-                float2 ca = pos[a], cb = pos[b];
-                const float sep = solve_position(P.radius, P.k_sum, P.inv_mass, ca, cb);
-                pos[a] = ca; pos[b] = cb;
-                if (!(b2min(0.0f, sep) >= -3.0f * B2_LINEAR_SLOP)) isl_bad[isl] = 1;
-            }
-            g.sync();
-        }
-        bool any_bad = false;
-#pragma unroll
-        for (int s = 0; s < APL; ++s) {
-            const int i = g.gl + s * G;
-            const uint8_t bad = isl_bad[i];
-            isl_act[i] = bad;
-            isl_bad[i] = 0;
-            any_bad |= bad != 0;
-        }
-        g.sync();
-        if (!g.ballot(any_bad)) break;
-    }
-#pragma unroll
-    for (int s = 0; s < APL; ++s) S.solved()[g.gl + s * G] = (P.pos_iters > 0) && !isl_act[g.gl + s * G];
-    g.sync();
-}
-#endif   // MACM_HUGE_BUILD
-
-// ------------------------------------------------------------------------------------------
-// Generic contact solver for environments with more touching contacts than lanes (tc > G):
-// every ordered contact goes through shared memory, level by level.  Rare (dense piles) and kept
-// out of line so that the common path stays small in the instruction cache.
-// ------------------------------------------------------------------------------------------
-template <int G, int APL>
-__device__ __noinline__ void solve_velocity_big(const Grp<G>& g, const EnvS<G * APL>& S, const SimConst& P, int tc,
-                                                int nlev, float ratio, float2* c_imp)
-{
-    using EWT = EW<G * APL>;
-    const float2* pos = S.pos(); float2* vel = S.vel();
-    float2* t_n = S.t_n(); float2* t_imp = S.t_imp();
-    const uint32_t* t_ew = S.t_ew();
-    const uint16_t* ordlvl = S.ordlvl();
-    const float mass_n = P.normal_mass, mass_t = P.normal_mass;
-    for (int t = g.gl; t < tc; t += G) {
-        const uint32_t ew = t_ew[t];
-        const float2 pa = pos[EWT::a(ew)], pb = pos[EWT::b(ew)];
-        float nx = 1.0f, ny = 0.0f;
-        const float dx = pb.x - pa.x, dy = pb.y - pa.y;
-        if ((dx * dx + dy * dy) > B2_EPSILON * B2_EPSILON) { nx = dx; ny = dy; b2normalize(nx, ny); }
-        float2 im = make_float2(0.0f, 0.0f);
-        if (P.warm_starting) { im = t_imp[t]; im.x = ratio * im.x; im.y = ratio * im.y; }
-        t_n[t] = make_float2(nx, ny);
-        t_imp[t] = im;
-    }
-    g.sync();
-    for (int it = -1; it < P.vel_iters; ++it) {   // it == -1: WarmStart
-        for (int lev = 1; lev <= nlev; ++lev) {
-            for (int k = g.gl; k < tc; k += G) {
-                const int ol = ordlvl[k];
-                if ((ol >> 8) != lev) continue;
-                const int t = ol & 0xff;
-                const uint32_t ew = t_ew[t];
-                const int a = EWT::a(ew), b = EWT::b(ew);
-                const float2 n = t_n[t];
-                float2 im = t_imp[t];
-                float2 va = vel[a], vb = vel[b];
-                if (it < 0) warm_start(n.x, n.y, im.x, im.y, P.inv_mass, va, vb);
-                else solve_velocity(n.x, n.y, P.friction, mass_n, mass_t, P.inv_mass, im.x, im.y, va, vb);
-                vel[a] = va; vel[b] = vb;
-                t_imp[t] = im;
-            }
-            g.sync();
-        }
-    }
-    const uint16_t* t_slot = S.t_slot();
-    for (int t = g.gl; t < tc; t += G) c_imp[t_slot[t]] = t_imp[t];
-}
-
-template <int G, int APL>
-__device__ __noinline__ void solve_position_big(const Grp<G>& g, const EnvS<G * APL>& S, const SimConst& P, int tc,
-                                                int nlev)
-{
-    using EWT = EW<G * APL>;
-    float2* pos = S.pos();
-    const uint32_t* label = S.label();
-    uint8_t* isl_act = S.isl_act(); uint8_t* isl_bad = S.isl_bad();
-    const uint32_t* t_ew = S.t_ew();
-    const uint16_t* ordlvl = S.ordlvl();
-#pragma unroll
-    for (int s = 0; s < APL; ++s) { isl_act[g.gl + s * G] = 1; isl_bad[g.gl + s * G] = 0; }
-    g.sync();
-    for (int it = 0; it < P.pos_iters; ++it) {
-        for (int lev = 1; lev <= nlev; ++lev) {
-            for (int k = g.gl; k < tc; k += G) {
-                const int ol = ordlvl[k];
-                if ((ol >> 8) != lev) continue;
-                const uint32_t ew = t_ew[ol & 0xff];
-                const int a = EWT::a(ew), b = EWT::b(ew);
-                const int isl = label[a];
-                if (!isl_act[isl]) continue;
-                float2 ca = pos[a], cb = pos[b];
-                const float sep = solve_position(P.radius, P.k_sum, P.inv_mass, ca, cb);
-                pos[a] = ca; pos[b] = cb;
-                if (!(b2min(0.0f, sep) >= -3.0f * B2_LINEAR_SLOP)) isl_bad[isl] = 1;
-            }
-            g.sync();
-        }
-        bool any_bad = false;
-#pragma unroll
-        for (int s = 0; s < APL; ++s) {
-            const int i = g.gl + s * G;
-            const uint8_t bad = isl_bad[i];
-            isl_act[i] = bad;
-            isl_bad[i] = 0;
-            any_bad |= bad != 0;
-        }
-        g.sync();
-        if (!g.ballot(any_bad)) break;
-    }
-#pragma unroll
-    for (int s = 0; s < APL; ++s) S.solved()[g.gl + s * G] = (P.pos_iters > 0) && !isl_act[g.gl + s * G];
-    g.sync();
-}
-
-// Islands of a dense pile (tc > G): Box2D's depth-first traversal replayed by one lane over
-// per-body edge lists (head-inserted in birth order, like b2ContactManager::AddPair builds them);
-// every contact gets its position in the island order and a level = 1 + max(level of the previous
-// contact of either body).  Contacts of one level share no body and run across lanes.
-template <int G, int APL>
-__device__ __noinline__ int islands_big(const Grp<G>& g, const EnvS<G * APL>& S, int tc)
-{
-    using EWT = EW<G * APL>;
-    uint32_t* t_ew = S.t_ew();
-    uint16_t* ordlvl = S.ordlvl();
-    uint32_t* label = S.label();
-#pragma unroll
-    for (int s = 0; s < APL; ++s) { S.lastlvl()[g.gl + s * G] = 0; S.head()[g.gl + s * G] = EW_NONE; }
-    g.sync();
-    int L = 1;
-    if (g.gl == 0) {
-        uint8_t* stack = S.stack(); uint8_t* head = S.head(); uint8_t* lastlvl = S.lastlvl();
-        constexpr int W = (G * APL + 31) / 32 < 2 ? 2 : (G * APL + 31) / 32;
+        constexpr int W = G * APL > 64 ? 4 : 2;
         uint32_t rem[W];   // bodies with a touching contact that are not in an island yet
 #pragma unroll
         for (int w = 0; w < W; ++w) rem[w] = 0u;
         for (int t = 0; t < tc; ++t) {
-            const uint32_t ew = t_ew[t];
-            const int a = EWT::a(ew), b = EWT::b(ew);
-            t_ew[t] = ew | ((uint32_t)head[a] << EWT::SH_NA) | ((uint32_t)head[b] << EWT::SH_NB);
-            head[a] = (uint8_t)t;
-            head[b] = (uint8_t)t;
+            const uint32_t w = st.edge(t);
+            const int a = St::a(w), b = St::b(w);
+            st.link(t, w, st.head[a], st.head[b]);
+            st.head[a] = t;
+            st.head[b] = t;
             rem[a >> 5] |= 1u << (a & 31);
             rem[b >> 5] |= 1u << (b & 31);
         }
@@ -1223,16 +998,16 @@ __device__ __noinline__ int islands_big(const Grp<G>& g, const EnvS<G * APL>& S,
             while (sp > 0) {
                 const int b = stack[--sp];
                 label[b] = (uint32_t)seed;
-                for (int t = head[b]; t != EW_NONE;) {
-                    const uint32_t ew = t_ew[t];
-                    const int ta = EWT::a(ew), tb = EWT::b(ew);
-                    const int nx = (ta == b) ? EWT::na(ew) : EWT::nb(ew);
-                    if (!(ew & EWT::TAKEN)) {
-                        t_ew[t] = ew | EWT::TAKEN;
-                        const int l = 1 + max((int)lastlvl[ta], (int)lastlvl[tb]);
-                        ordlvl[nord++] = (uint16_t)(t | (l << 8));
-                        lastlvl[ta] = (uint8_t)l;
-                        lastlvl[tb] = (uint8_t)l;
+                for (int t = st.head[b]; t != St::NONE;) {
+                    const uint32_t w = st.edge(t);
+                    const int ta = St::a(w), tb = St::b(w);
+                    const int nx = st.next(w, t, b);
+                    if (!St::taken(w)) {
+                        st.take(t, w);
+                        const int l = 1 + max((int)st.lastlvl[ta], (int)st.lastlvl[tb]);
+                        st.set_ord(nord++, t, l);
+                        st.lastlvl[ta] = l;
+                        st.lastlvl[tb] = l;
                         L = max(L, l);
                         const int other = (ta == b) ? tb : ta;
                         const uint32_t ob = 1u << (other & 31);
@@ -1248,38 +1023,160 @@ __device__ __noinline__ int islands_big(const Grp<G>& g, const EnvS<G * APL>& S,
     return L;
 }
 
-#if MACM_HUGE_BUILD
-// The dense-pile solver of the kernels built WITH the global-memory stage (translation unit macm_kernels_huge.cu, launched for
-// sims that bound macm_buffers.touch_scratch; the default kernels are compiled without any of this -- their register
-// allocation is not to be disturbed by a path for overlapping spawn piles, and ptxas allocates per translation unit).  A full shared-memory stage may be a truncated one:
-// then solve_velocity_huge takes the env from its contact list and leaves its level count (and the env index) in the
-// env's MISC words for the position solver.  Returns 1 when even the global stage was too small.
-template <int G, int APL>
-__device__ __noinline__ int solve_velocity_dense_h(const Grp<G>& g, const EnvS<G * APL>& S, const SimConst& P, int env, int cnt,
-                                                   int tc, float ratio, const uint32_t* c_ab, float2* c_imp)
+// b2ContactSolver ctor + InitializeVelocityConstraints (world normals at the pre-integration positions, impulses scaled
+// by dtRatio), WarmStart and the velocity iterations level by level, then StoreImpulses to the HBM list.
+template <int G, int APL, class St>
+__device__ __forceinline__ void dense_solve_velocity(const Grp<G>& g, const EnvS<G * APL>& S, const St& st, const SimConst& P,
+                                                     int tc, int nlev, float ratio, float2* c_imp)
 {
-    if (g.gl == 0) S.misc()[0] = 0u;
-    if (tc == P.TC) {
-        const int r = solve_velocity_huge<G, APL>(g, S, P, env, cnt, c_ab, c_imp, ratio);
-        if (r & 0xffff) {
-            if (g.gl == 0) { S.misc()[0] = (uint32_t)(r & 0xffff); S.misc()[1] = (uint32_t)env; }
-            g.sync();
-            return r >> 30;
-        }
+    const float2* pos = S.pos(); float2* vel = S.vel();
+    const float mass_n = P.normal_mass, mass_t = P.normal_mass;
+    for (int t = g.gl; t < tc; t += G) {
+        const uint32_t w = st.edge(t);
+        const float2 pa = pos[St::a(w)], pb = pos[St::b(w)];
+        float nx = 1.0f, ny = 0.0f;
+        const float dx = pb.x - pa.x, dy = pb.y - pa.y;
+        if ((dx * dx + dy * dy) > B2_EPSILON * B2_EPSILON) { nx = dx; ny = dy; b2normalize(nx, ny); }
+        float2 im = make_float2(0.0f, 0.0f);
+        if (P.warm_starting) { im = st.imp[t]; im.x = ratio * im.x; im.y = ratio * im.y; }
+        st.n[t] = make_float2(nx, ny);
+        st.imp[t] = im;
     }
     g.sync();
-    const int nlev = islands_big<G, APL>(g, S, tc);
-    if (g.gl == 0) S.misc()[2] = (uint32_t)nlev;
-    solve_velocity_big<G, APL>(g, S, P, tc, nlev, ratio, c_imp);
-    return 0;
+    for (int it = -1; it < P.vel_iters; ++it) {   // it == -1: WarmStart
+        for (int lev = 1; lev <= nlev; ++lev) {
+            for (int k = g.gl; k < tc; k += G) {
+                const int2 o = st.ord(k);
+                if (o.y != lev) continue;
+                const int t = o.x;
+                const uint32_t w = st.edge(t);
+                const int a = St::a(w), b = St::b(w);
+                const float2 n = st.n[t];
+                float2 im = st.imp[t];
+                float2 va = vel[a], vb = vel[b];
+                if (it < 0) warm_start(n.x, n.y, im.x, im.y, P.inv_mass, va, vb);
+                else solve_velocity(n.x, n.y, P.friction, mass_n, mass_t, P.inv_mass, im.x, im.y, va, vb);
+                vel[a] = va; vel[b] = vb;
+                st.imp[t] = im;
+            }
+            g.sync();
+        }
+    }
+    for (int t = g.gl; t < tc; t += G) c_imp[st.slot[t]] = st.imp[t];
+}
+
+// The position iterations level by level; an island stops as soon as it is solved.  Leaves solved[] for the sleep pass.
+template <int G, int APL, class St>
+__device__ __forceinline__ void dense_solve_position(const Grp<G>& g, const EnvS<G * APL>& S, const St& st, const SimConst& P,
+                                                     int tc, int nlev)
+{
+    float2* pos = S.pos();
+    const uint32_t* label = S.label();
+    uint8_t* isl_act = S.isl_act(); uint8_t* isl_bad = S.isl_bad();
+#pragma unroll
+    for (int s = 0; s < APL; ++s) { isl_act[g.gl + s * G] = 1; isl_bad[g.gl + s * G] = 0; }
+    g.sync();
+    for (int it = 0; it < P.pos_iters; ++it) {
+        for (int lev = 1; lev <= nlev; ++lev) {
+            for (int k = g.gl; k < tc; k += G) {
+                const int2 o = st.ord(k);
+                if (o.y != lev) continue;
+                const uint32_t w = st.edge(o.x);
+                const int a = St::a(w), b = St::b(w);
+                const int isl = label[a];
+                if (!isl_act[isl]) continue;
+                float2 ca = pos[a], cb = pos[b];
+                const float sep = solve_position(P.radius, P.k_sum, P.inv_mass, ca, cb);
+                pos[a] = ca; pos[b] = cb;
+                if (!(b2min(0.0f, sep) >= -3.0f * B2_LINEAR_SLOP)) isl_bad[isl] = 1;
+            }
+            g.sync();
+        }
+        bool any_bad = false;
+#pragma unroll
+        for (int s = 0; s < APL; ++s) {
+            const int i = g.gl + s * G;
+            const uint8_t bad = isl_bad[i];
+            isl_act[i] = bad;
+            isl_bad[i] = 0;
+            any_bad |= bad != 0;
+        }
+        g.sync();
+        if (!g.ballot(any_bad)) break;
+    }
+#pragma unroll
+    for (int s = 0; s < APL; ++s) S.solved()[g.gl + s * G] = (P.pos_iters > 0) && !isl_act[g.gl + s * G];
+    g.sync();
+}
+
+// The default kernels' entry points (shared-memory stage only): phase 5 calls the first two, phase 7 the third.
+template <int G, int APL>
+__device__ __noinline__ int dense_islands_smem(const Grp<G>& g, const EnvS<G * APL>& S, int tc)
+{
+    return dense_islands<G, APL>(g, S, SmemStage<G * APL>(S), tc);
 }
 template <int G, int APL>
-__device__ __noinline__ void solve_position_dense_h(const Grp<G>& g, const EnvS<G * APL>& S, const SimConst& P, int tc)
+__device__ __noinline__ void dense_solve_velocity_smem(const Grp<G>& g, const EnvS<G * APL>& S, const SimConst& P, int tc,
+                                                       int nlev, float ratio, float2* c_imp)
 {
-    g.sync();
-    const int Lh = (int)S.misc()[0];   // (uniform over the group)
-    if (Lh) solve_position_huge<G, APL>(g, S, P, (int)S.misc()[1], Lh);
-    else solve_position_big<G, APL>(g, S, P, tc, (int)S.misc()[2]);
+    dense_solve_velocity<G, APL>(g, S, SmemStage<G * APL>(S), P, tc, nlev, ratio, c_imp);
+}
+template <int G, int APL>
+__device__ __noinline__ void dense_solve_position_smem(const Grp<G>& g, const EnvS<G * APL>& S, const SimConst& P, int tc,
+                                                       int nlev)
+{
+    dense_solve_position<G, APL>(g, S, SmemStage<G * APL>(S), P, tc, nlev);
+}
+
+#if MACM_HUGE_BUILD
+// Phases 5 and 7 of the kernels built with the global-memory stage.  A full shared-memory stage (tc == TC) may be a
+// truncated one: then every touching contact of the env's HBM list is staged in global memory, in birth order, and the
+// env is solved from there.  Returns the number of levels, with bit 30 set when even the global stage was too small
+// (the contacts beyond it are left out); MISC word 0 tells the position part which stage holds the env.  (The
+// shared-memory stage is inlined here rather than called: fewer spills in this unit's step kernels, measured with ptxas.)
+template <int G, int APL>
+__device__ __noinline__ int dense_solve_velocity_huge(const Grp<G>& g, const EnvS<G * APL>& S, const SimConst& P, int env, int cnt,
+                                                      int tc, float ratio, const uint32_t* c_ab, float2* c_imp)
+{
+    const GmemStage H(S, P, env);
+    int ht = 0;
+    bool overflow = false;
+    if (tc == P.TC) {
+        for (int base = 0; base < cnt; base += G) {
+            const int k = base + g.gl;
+            const uint32_t ab = k < cnt ? c_ab[k] : 0u;
+            const bool touch = (ab >> 16) & 1u;
+            const unsigned tm = g.ballot(touch);
+            const int t = ht + __popc(tm & g.below());
+            if (touch && t < P.TCH) {
+                H.ew[t] = ab & 0xffffu;   // a | b<<8
+                H.slot[t] = (uint16_t)k;
+                // the first TC impulses were staged in shared memory by phase 2, the rest kept theirs in the HBM list
+                H.imp[t] = t < P.TC ? S.t_imp()[t] : c_imp[k];
+            }
+            overflow |= touch && t >= P.TCH;
+            ht += __popc(tm);
+        }
+    }
+    const int gtc = ht <= P.TC ? 0 : min(ht, P.TCH);   // (uniform) 0: the shared-memory stage holds every touching contact
+    if (g.gl == 0) S.misc()[0] = (uint32_t)gtc;
+    if (!gtc) {
+        const SmemStage<G * APL> st(S);
+        const int nlev = dense_islands<G, APL>(g, S, st, tc);
+        dense_solve_velocity<G, APL>(g, S, st, P, tc, nlev, ratio, c_imp);
+        return nlev;
+    }
+    const int nlev = dense_islands<G, APL>(g, S, H, gtc);
+    dense_solve_velocity<G, APL>(g, S, H, P, gtc, nlev, ratio, c_imp);
+    return nlev | (g.ballot(overflow) ? (1 << 30) : 0);
+}
+template <int G, int APL>
+__device__ __noinline__ void dense_solve_position_huge(const Grp<G>& g, const EnvS<G * APL>& S, const SimConst& P, int env, int tc,
+                                                       int nlev)
+{
+    const int gtc = (int)S.misc()[0];
+    if (gtc) dense_solve_position<G, APL>(g, S, GmemStage(S, P, env), P, gtc, nlev);
+    else dense_solve_position<G, APL>(g, S, SmemStage<G * APL>(S), P, tc, nlev);
 }
 #endif   // MACM_HUGE_BUILD
 
@@ -1890,7 +1787,7 @@ __global__ void __launch_bounds__(shape_max_threads(G, APL), 1) macm_step_kernel
     //     the k-th seed goes to lane k, which runs the DFS over the bodies' touching-contact sets
     //     (bit t = staged contact t, highest = newest) and threads the contacts into a list;
     //   * dense piles (tc > G): one lane replays the DFS for the whole world and the contacts are
-    //     level-scheduled across lanes (islands_big / solve_*_big, out of line).
+    //     level-scheduled across lanes (dense_* above, out of line).
     const bool big = tc > G;
     const bool has = !big && g.gl < tc;
     nlev = 0;
@@ -1899,14 +1796,19 @@ __global__ void __launch_bounds__(shape_max_threads(G, APL), 1) macm_step_kernel
     int ohead = EW_NONE, oseed = 0;     // multi: first contact of this lane's island, its seed body
     // inv_dt0 == 0 on a world's first step -> dtRatio 0
     const float ratio = (step_cnt == 0) ? 0.0f : P.dt_ratio;
+#if MACM_HUGE_BUILD
+    // a dense pile's level count, phase 5 to 7 (nlev stays 0 in this unit: live for the whole step it costs spills)
+    int hlev = 0;
+#endif
 
     // ---- phase 5: contact solver, velocity part -------------------------------------------------
     if (big) {
 #if MACM_HUGE_BUILD
-        if (solve_velocity_dense_h<G, APL>(g, S, P, env, cnt, tc, ratio, c_ab, c_imp)) overflow_t = true;
+        hlev = dense_solve_velocity_huge<G, APL>(g, S, P, env, cnt, tc, ratio, c_ab, c_imp);
+        if (hlev >> 30) { overflow_t = true; hlev &= 0xffff; }
 #else
-        nlev = islands_big<G, APL>(g, S, tc);
-        solve_velocity_big<G, APL>(g, S, P, tc, nlev, ratio, c_imp);
+        nlev = dense_islands_smem<G, APL>(g, S, tc);
+        dense_solve_velocity_smem<G, APL>(g, S, P, tc, nlev, ratio, c_imp);
 #endif
     } else if (tc > 0) {
         const float mass_n = P.normal_mass, mass_t = P.normal_mass;
@@ -2071,9 +1973,9 @@ __global__ void __launch_bounds__(shape_max_threads(G, APL), 1) macm_step_kernel
     // ---- phase 7: contact solver, position part (each island stops as soon as it is solved) -------
     if (big) {
 #if MACM_HUGE_BUILD
-        solve_position_dense_h<G, APL>(g, S, P, tc);
+        dense_solve_position_huge<G, APL>(g, S, P, env, tc, hlev);
 #else
-        solve_position_big<G, APL>(g, S, P, tc, nlev);
+        dense_solve_position_smem<G, APL>(g, S, P, tc, nlev);
 #endif
 #pragma unroll
         for (int s = 0; s < APL; ++s) c[s] = pos[g.gl + s * G];
