@@ -27,6 +27,7 @@ struct macm_sim {
     double2* d_sincos;
     int* d_scratch;            // two counters (macm_overflow_count)
     uint64_t auto_seed;        // seed of the resets appended under MACM_FLAG_AUTO_RESET
+    Finals fin;                // macm_bind_final: where every reset copies the env's rows first
     // Ordering between the caller's streams and the handle's own host-path stream: the last stream an entry point
     // enqueued device work on, whether that work is still unordered against hstream, and the reverse.  Events are
     // recorded lazily, at the moment the other side is used -- nothing is inserted between two step launches
@@ -98,11 +99,12 @@ static SampleConst sample_const(const macm_sim* sim, uint64_t seed)
     return sc;
 }
 
-// MACM_FLAG_AUTO_RESET: the launch that follows every step / rollout launch
-static int auto_reset(macm_sim* sim, cudaStream_t s)
+// MACM_FLAG_AUTO_RESET: the launch that follows every step / rollout launch.  `row`: the last row of a rollout's
+// final_* arrays, which receives the terminal rows of the envs this launch restarts
+static int auto_reset(macm_sim* sim, cudaStream_t s, const Finals& row = Finals{})
 {
     if (!(sim->params.flags & MACM_FLAG_AUTO_RESET)) return MACM_OK;
-    CU(macm_launch_reset_masked(sim->K, sim->cfg, nullptr, sample_const(sim, sim->auto_seed), s));
+    CU(macm_launch_reset_masked(sim->K, sim->cfg, nullptr, sample_const(sim, sim->auto_seed), sim->fin, row, s));
     sim->launches += 1;
     return MACM_OK;
 }
@@ -390,6 +392,27 @@ extern "C" int macm_bind(macm_sim* sim, const macm_buffers* b)
     return MACM_OK;
 }
 
+// the final arrays of `f` fit this sim's env kind and the alignment of the bound buffers of the same names
+static int check_final(const macm_sim* sim, const float* obs, const int32_t* nn_idx, const float* tdm_state,
+                       const int32_t* env_state)
+{
+    const bool flock = sim->K.kind == MACM_ENV_FLOCK;
+    if ((nn_idx && !flock) || (tdm_state && flock)) return MACM_E_INVALID;
+    if ((obs && !aligned(obs, 16)) || (nn_idx && !aligned(nn_idx, 4)) || (tdm_state && !aligned(tdm_state, 16)) ||
+        (env_state && !aligned(env_state, 16)))
+        return MACM_E_ALIGN;
+    return MACM_OK;
+}
+
+extern "C" int macm_bind_final(macm_sim* sim, const macm_final_out* f)
+{
+    if (!sim) return MACM_E_INVALID;
+    if (!f) { sim->fin = Finals{}; return MACM_OK; }
+    if (int rc = check_final(sim, f->obs, f->nn_idx, f->tdm_state, f->env_state)) return rc;
+    sim->fin = Finals{f->obs, f->nn_idx, (float4*)f->tdm_state, (int4*)f->env_state};
+    return MACM_OK;
+}
+
 extern "C" int macm_reset(macm_sim* sim, void* stream)
 {
     if (!sim) return MACM_E_INVALID;
@@ -420,7 +443,7 @@ extern "C" int macm_reset_masked(macm_sim* sim, const uint8_t* mask, uint64_t se
     if (!sim->bound) return MACM_E_UNBOUND;
     GUARD();
     if (int rc = order_after_host(sim, (cudaStream_t)stream)) return rc;
-    CU(macm_launch_reset_masked(sim->K, sim->cfg, mask, sample_const(sim, seed), (cudaStream_t)stream));
+    CU(macm_launch_reset_masked(sim->K, sim->cfg, mask, sample_const(sim, seed), sim->fin, Finals{}, (cudaStream_t)stream));
     sim->launches += 1;
     note_device_work(sim, (cudaStream_t)stream);
     return MACM_OK;
@@ -507,13 +530,24 @@ extern "C" int macm_rollout(macm_sim* sim, const void* actions, int32_t n_steps,
             (out->nn_idx && !aligned(out->nn_idx, 4)))
             return MACM_E_ALIGN;
         R.obs = out->obs; R.nn_idx = out->nn_idx; R.rewards = out->rewards; R.collided = out->collided; R.done = out->done;
+        if (int rc = check_final(sim, out->final_obs, out->final_nn_idx, out->final_tdm_state, out->final_env_state))
+            return rc;
+        R.fin_k = Finals{out->final_obs, out->final_nn_idx, (float4*)out->final_tdm_state, (int4*)out->final_env_state};
     }
+    R.fin = sim->fin;
+    R.finals = R.fin.obs || R.fin.nn_idx || R.fin.tdm || R.fin.es || R.fin_k.obs || R.fin_k.nn_idx || R.fin_k.tdm ||
+               R.fin_k.es;
+    // the launch's last step: the appended reset copies its terminal rows to row n_steps - 1 of the final_* arrays
+    const SimConst& K = sim->K;
+    const size_t last = (size_t)(n_steps - 1) * K.E, EN = last * K.N;
+    const Finals row = {R.fin_k.obs ? R.fin_k.obs + EN * K.obs_dim : nullptr, R.fin_k.nn_idx ? R.fin_k.nn_idx + EN : nullptr,
+                        R.fin_k.tdm ? R.fin_k.tdm + EN : nullptr, R.fin_k.es ? R.fin_k.es + last : nullptr};
     GUARD();
     if (int rc = order_after_host(sim, (cudaStream_t)stream)) return rc;
     CU(macm_launch_step(sim->K, sim->cfg, actions, R, (cudaStream_t)stream));
     sim->launches += 1;
     note_device_work(sim, (cudaStream_t)stream);
-    return auto_reset(sim, (cudaStream_t)stream);
+    return auto_reset(sim, (cudaStream_t)stream, row);
 }
 
 extern "C" int macm_observe(macm_sim* sim, void* stream)

@@ -2146,11 +2146,50 @@ __global__ void __launch_bounds__(shape_max_threads(G, APL), 1) macm_step_kernel
     }
 
     PHASE_STAMP(11);
-    // ---- auto-reset inside a rollout (MACM_FLAG_AUTO_RESET): an env that is done starts its next episode before the
+    // Between two steps of a rollout the velocities, fat AABBs and sleep timers wait in shared memory (the
+    // velocity array and the touching-contact stage, both idle until the next step's phase 2), so that the
+    // nearest-agent search of phase 13 -- the register-hungriest phase -- does not have to carry them.
+    float4* fat_park = reinterpret_cast<float4*>(S.t_n());
+    float* slp_park = reinterpret_cast<float*>(fat_park + NC);
+    if (ROLL && !last) {
+        g.sync();
+#pragma unroll
+        for (int s = 0; s < APL; ++s) {
+            const int i = g.gl + s * G;
+            vel[i] = v[s];
+            fat_park[i] = fatr[s];
+            slp_park[i] = slp[s];
+        }
+    }
+    // Auto-reset inside a rollout (MACM_FLAG_AUTO_RESET): an env that is done starts its next episode before the
     // step's observation is written -- the draws, the body creation and the order of events of macm_reset_masked
     // (the launch the flag appends to a single step), so K steps in one launch stay bit-identical to K single
     // steps.  The launch's last step leaves the reset to that appended launch: its state is already written back.
-    if (ROLL && !last && (P.flags & MACM_FLAG_AUTO_RESET) && done) {
+    // With final destinations given (R.finals), phase 13 first runs on the finished episode (pass 0) and stores its
+    // terminal observation and state there, as macm_reset_masked copies them; then the reset and pass 1.  One copy
+    // of the observation code serves both passes: code size is what limits a rollout (DESIGN, instruction supply).
+    const bool restart = ROLL && !last && (P.flags & MACM_FLAG_AUTO_RESET) && done;
+#pragma unroll 1
+    for (int pass = (restart && R_.finals) ? 0 : 1;; ++pass) {
+    if (ROLL && pass == 0) {   // terminal TDM state and env state, as phase 12 and the env-state store above write them
+        if (TDM) {
+#pragma unroll
+            for (int s = 0; s < APL; ++s) {
+                if (!valid[s]) continue;
+                const size_t gi = (size_t)env * N + g.gl + s * G;
+                const float4 td = make_float4(health[s], __int_as_float(cd_atk[s]), __int_as_float(cd_mov[s]),
+                                              __int_as_float((now_alive[s] ? 1 : 0) | (hits[s] << 8)));
+                if (R_.fin.tdm) R_.fin.tdm[gi] = td;
+                if (R_.fin_k.tdm) R_.fin_k.tdm[(size_t)ks * EN + gi] = td;
+            }
+        }
+        if (g.gl == 0) {
+            const int4 es = make_int4(step_cnt, eflags, tc, winner);
+            if (R_.fin.es) R_.fin.es[env] = es;
+            if (R_.fin_k.es) R_.fin_k.es[(size_t)ks * P.E + env] = es;
+        }
+    }
+    if (restart && pass == 1) {
         const uint32_t episode = ((uint32_t)eflags >> MACM_ENV_EPISODE_SHIFT) + 1u;
         g.sync();
 #pragma unroll
@@ -2160,9 +2199,11 @@ __global__ void __launch_bounds__(shape_max_threads(G, APL), 1) macm_step_kernel
                 float x, y, a;
                 sample_agent(P, R_.sc, (uint64_t)env * N + i + (uint64_t)P.env_base * N, i, episode, x, y, a);
                 const float r = P.radius;
-                c[s] = make_float2(x, y); v[s] = make_float2(0.0f, 0.0f); ang[s] = a; slp[s] = 0.0f;
-                fatr[s] = make_float4((x - r) - B2_AABB_EXTENSION, (y - r) - B2_AABB_EXTENSION,
-                                      (x + r) + B2_AABB_EXTENSION, (y + r) + B2_AABB_EXTENSION);
+                c[s] = make_float2(x, y); ang[s] = a;
+                vel[i] = make_float2(0.0f, 0.0f);
+                fat_park[i] = make_float4((x - r) - B2_AABB_EXTENSION, (y - r) - B2_AABB_EXTENSION,
+                                          (x + r) + B2_AABB_EXTENSION, (y + r) + B2_AABB_EXTENSION);
+                slp_park[i] = 0.0f;
                 pos[i] = c[s];
                 if (TDM) { health[s] = P.init_health; cd_atk[s] = 0; cd_mov[s] = 0; hits[s] = 0; S.ang()[i] = a; }
                 else S.tgt()[i] = sample_target(R_.sc, (uint64_t)(env + P.env_base) * P.T + (P.T == 1 ? 0 : (int)P.target_idx[i]), episode);
@@ -2182,32 +2223,35 @@ __global__ void __launch_bounds__(shape_max_threads(G, APL), 1) macm_step_kernel
         g.sync();
     }
     // ---- phase 13: observations (mvmnt.py:181-222 / combat.py:206-227) ----------------------------
-    // Between two steps of a rollout the velocities, fat AABBs and sleep timers wait in shared memory (the
-    // velocity array and the touching-contact stage, both idle until the next step's phase 2), so that the
-    // nearest-agent search -- the register-hungriest phase -- does not have to carry them.
-    if (ROLL && !last) {
-        g.sync();
-#pragma unroll
-        for (int s = 0; s < APL; ++s) {
-            const int i = g.gl + s * G;
-            vel[i] = v[s];
-            reinterpret_cast<float4*>(S.t_n())[i] = fatr[s];
-            reinterpret_cast<float*>(reinterpret_cast<float4*>(S.t_n()) + NC)[i] = slp[s];
-        }
-    }
     // (a rollout without per-step observation arrays only observes after its last step)
-    if (last || R.obs() || R.policy() == MACM_BOT_FLOCK) {
+    // (pass 0 only observes when the terminal observation has somewhere to go)
+    const bool obs0 = ROLL && pass == 0 &&
+                      (R_.fin.obs || R_.fin_k.obs || (!TDM && (R_.fin.nn_idx || R_.fin_k.nn_idx)));
+    if (((last || R.obs() || R.policy() == MACM_BOT_FLOCK) && !(ROLL && pass == 0)) || obs0) {
         float* ob_k = R.obs() ? R.obs() + (size_t)ks * EN * P.obs_dim : nullptr;
+        int* nn_k = R.nn_idx() ? R.nn_idx() + (size_t)ks * EN : nullptr;
+        float* ob1 = last ? P.obs : ob_k;
+        float* ob2 = last ? ob_k : nullptr;
+        int* nn1 = last ? P.nn_idx : nn_k;
+        int* nn2 = last ? nn_k : nullptr;
+        // the flock actor steers by the new episode's first observation, as macm_bot_actions after the reset does
+        float2* tgo = (R.policy() == MACM_BOT_FLOCK && !last) ? reinterpret_cast<float2*>(S.nw()) : nullptr;
+        if (ROLL && pass == 0) {
+            ob1 = R_.fin.obs;
+            ob2 = R_.fin_k.obs ? R_.fin_k.obs + (size_t)ks * EN * P.obs_dim : nullptr;
+            nn1 = R_.fin.nn_idx;
+            nn2 = R_.fin_k.nn_idx ? R_.fin_k.nn_idx + (size_t)ks * EN : nullptr;
+            tgo = nullptr;
+        }
         if (TDM) {
             g.sync();
-            tdm_observe<G, APL>(g, S, P, env, alive, last ? P.obs : ob_k, last ? ob_k : nullptr);
+            tdm_observe<G, APL>(g, S, P, env, alive, ob1, ob2);
         } else {
-            int* nn_k = R.nn_idx() ? R.nn_idx() + (size_t)ks * EN : nullptr;
-            float2* tgo = (R.policy() == MACM_BOT_FLOCK && !last) ? reinterpret_cast<float2*>(S.nw()) : nullptr;
-            flock_observe<G, APL>(g, S, P, env, ang, last ? P.obs : ob_k, last ? P.nn_idx : nn_k, last ? ob_k : nullptr,
-                                  last ? nn_k : nullptr, tgo);
+            flock_observe<G, APL>(g, S, P, env, ang, ob1, nn1, ob2, nn2, tgo);
         }
     }
+    if (!ROLL || pass == 1) break;
+    }   // for pass
     PHASE_STAMP(12);
     }   // for ks
 #ifndef MACM_PHASE_TRACE
@@ -2225,12 +2269,44 @@ __global__ void __launch_bounds__(shape_max_threads(G, APL), 1) macm_step_kernel
 #endif
 }
 
+// The group copies row `row` (n 32-bit words) of an array to the same row of up to two arrays of its layout: 16-byte
+// vectors when n is a multiple of 4 and all three arrays start 16-byte aligned (every row then does too), single words
+// otherwise (cartesian observations of an odd N; nn_idx arrays, which need only 4-byte alignment).
+template <int G>
+__device__ __forceinline__ void copy_row(const Grp<G>& g, const void* src, void* d1, void* d2, size_t row, int n)
+{
+    const bool vec = (n & 3) == 0 && (((uintptr_t)src | (uintptr_t)d1 | (uintptr_t)d2) & 15) == 0;   // warp-uniform
+    if (vec) {
+        const int n4 = n >> 2;
+        const uint4* s = reinterpret_cast<const uint4*>(src) + row * n4;
+        uint4* a = d1 ? reinterpret_cast<uint4*>(d1) + row * n4 : nullptr;
+        uint4* b = d2 ? reinterpret_cast<uint4*>(d2) + row * n4 : nullptr;
+        for (int k = g.gl; k < n4; k += G) {
+            const uint4 v = s[k];
+            if (a) a[k] = v;
+            if (b) b[k] = v;
+        }
+    } else {
+        const uint32_t* s = reinterpret_cast<const uint32_t*>(src) + row * n;
+        uint32_t* a = d1 ? reinterpret_cast<uint32_t*>(d1) + row * n : nullptr;
+        uint32_t* b = d2 ? reinterpret_cast<uint32_t*>(d2) + row * n : nullptr;
+        for (int k = g.gl; k < n; k += G) {
+            const uint32_t v = s[k];
+            if (a) a[k] = v;
+            if (b) b[k] = v;
+        }
+    }
+}
+
 // get_obs() alone; with RESET, first a new episode for the envs selected by `mask` (null: the bound `done`
 // buffer) and nothing at all for the others -- macm_reset_masked: the reference's env.reset() (mvmnt.py:224-233,
-// combat.py:229-239) for the envs that are done (mvmnt.py:134-136, combat.py:171-182).
+// combat.py:229-239) for the envs that are done (mvmnt.py:134-136, combat.py:171-182).  Before anything of a
+// selected env is overwritten, its rows of obs / nn_idx / tdm_state / env_state go to `fin` (the bound final slots)
+// and `fin2` (row K-1 of a rollout's final_* arrays); both are unused without RESET.
 template <int G, int APL, int KIND, bool RESET>
 __global__ void __launch_bounds__(128) macm_observe_kernel(const __grid_constant__ SimConst P, const uint8_t* __restrict__ mask,
-                                                           const __grid_constant__ SampleConst sc)
+                                                           const __grid_constant__ SampleConst sc,
+                                                           const __grid_constant__ Finals fin, const __grid_constant__ Finals fin2)
 {
     constexpr int NC = G * APL;
     constexpr int GPW = 32 / G;
@@ -2244,6 +2320,13 @@ __global__ void __launch_bounds__(128) macm_observe_kernel(const __grid_constant
     S.base = smem_raw + (size_t)slot_in_block * Lay<NC>::bytes(P.TC);
     if (RESET) {
         if (!(mask ? mask[env] : P.done[env])) return;   // the whole group leaves together
+        if (fin.obs || fin.nn_idx || fin.tdm || fin.es || fin2.obs || fin2.nn_idx || fin2.tdm || fin2.es) {
+            if (fin.obs || fin2.obs) copy_row<G>(g, P.obs, fin.obs, fin2.obs, env, P.N * P.obs_dim);
+            if (KIND != MACM_ENV_TDM && (fin.nn_idx || fin2.nn_idx)) copy_row<G>(g, P.nn_idx, fin.nn_idx, fin2.nn_idx, env, P.N);
+            if (KIND == MACM_ENV_TDM && (fin.tdm || fin2.tdm)) copy_row<G>(g, P.tdm, fin.tdm, fin2.tdm, env, P.N * 4);
+            if (fin.es || fin2.es) copy_row<G>(g, P.env_state, fin.es, fin2.es, env, 4);
+            g.sync();   // every lane's loads are done before any of the rows is overwritten below
+        }
         // episode counter of the env: bits 8.. of its flag word; keys the draws so that episodes differ
         const uint32_t episode = ((uint32_t)P.env_state[env].y >> MACM_ENV_EPISODE_SHIFT) + 1u;
         const float r = P.radius;
@@ -2334,7 +2417,8 @@ cudaError_t launch_one(const SimConst& P, const LaunchCfg& cfg, const void* acti
 {
 #if !MACM_HUGE_BUILD
     if (observe_only) {
-        macm_observe_kernel<G, APL, KIND, false><<<cfg.obs_blocks, 128, cfg.obs_smem_bytes, s>>>(P, nullptr, SampleConst{});
+        macm_observe_kernel<G, APL, KIND, false><<<cfg.obs_blocks, 128, cfg.obs_smem_bytes, s>>>(P, nullptr, SampleConst{},
+                                                                                                 Finals{}, Finals{});
         return cudaGetLastError();
     }
 #endif
@@ -2367,9 +2451,10 @@ cudaError_t launch_one(const SimConst& P, const LaunchCfg& cfg, const void* acti
 
 #if !MACM_HUGE_BUILD
 template <int G, int APL, int KIND>
-cudaError_t reset_masked_one(const SimConst& P, const LaunchCfg& cfg, const uint8_t* mask, const SampleConst& sc, cudaStream_t s)
+cudaError_t reset_masked_one(const SimConst& P, const LaunchCfg& cfg, const uint8_t* mask, const SampleConst& sc,
+                             const Finals& fin, const Finals& fin2, cudaStream_t s)
 {
-    macm_observe_kernel<G, APL, KIND, true><<<cfg.obs_blocks, 128, cfg.obs_smem_bytes, s>>>(P, mask, sc);
+    macm_observe_kernel<G, APL, KIND, true><<<cfg.obs_blocks, 128, cfg.obs_smem_bytes, s>>>(P, mask, sc, fin, fin2);
     return cudaGetLastError();
 }
 #endif
@@ -2513,9 +2598,9 @@ cudaError_t macm_launch_observe(const SimConst& P, const LaunchCfg& cfg, cudaStr
 }
 
 cudaError_t macm_launch_reset_masked(const SimConst& P, const LaunchCfg& cfg, const uint8_t* mask, const SampleConst& sc,
-                                     cudaStream_t s)
+                                     const Finals& fin, const Finals& fin2, cudaStream_t s)
 {
-#define CALL(G_, A_, K_) reset_masked_one<G_, A_, K_>(P, cfg, mask, sc, s)
+#define CALL(G_, A_, K_) reset_masked_one<G_, A_, K_>(P, cfg, mask, sc, fin, fin2, s)
     DISPATCH_SHAPE(CALL)
 #undef CALL
 }

@@ -65,9 +65,17 @@ struct SampleConst {
     double spread, sx, sy, tmin, tmax, width, height;
 };
 
+// Where a reset copies an env's rows of obs / nn_idx / tdm_state / env_state before it overwrites them: the terminal
+// observation and state of the finished episode (macm_bind_final, macm_rollout_out.final_*).  Each array has the
+// layout of the bound buffer of the same name; any pointer may be null.
+struct Finals {
+    float* obs; int* nn_idx; float4* tdm; int4* es;
+};
+
 // Arguments of a multi-step launch (macm_rollout): K consecutive steps of every env inside one kernel, the env's
 // state staying on chip between them.  Per-step outputs go to the caller's [K, ...] arrays (any of them may be
 // null); the sim's bound output buffers receive the last step's values, exactly as after K calls of macm_step.
+// (Members are only ever appended: the single-step kernels read the leading ones at fixed parameter offsets.)
 struct Rollout {
     SampleConst sc;     // distributions and seed of the in-launch resets (MACM_FLAG_AUTO_RESET)
     int K;              // steps in this launch (macm_step: 1)
@@ -75,6 +83,10 @@ struct Rollout {
     int policy;         // MACM_BOT_* when `actions` is null (the actions=None mode of mvmnt.py:86-92), else -1
     unsigned long long seed;
     float* obs; int* nn_idx; float* rewards; uint8_t* collided; uint8_t* done;
+    // terminal rows of the envs an in-launch reset restarts after step k < K - 1 (the reset the launch appends
+    // covers step K - 1): the bound final slots [E, ...] and the caller's per-step final arrays [K, E, ...]
+    Finals fin, fin_k;
+    int finals;         // some pointer of fin / fin_k is set
 };
 
 struct LaunchCfg {
@@ -145,8 +157,9 @@ cudaError_t macm_launch_observe(const SimConst& P, const LaunchCfg& cfg, cudaStr
 cudaError_t macm_prepare_kernels_huge(const SimConst& P, const LaunchCfg& cfg);
 cudaError_t macm_launch_step_huge(const SimConst& P, const LaunchCfg& cfg, const void* actions, const Rollout& R, cudaStream_t s);
 cudaError_t macm_launch_reset(const SimConst& P, cudaStream_t s);
+// fin / fin2: where each reset env's rows go first (bound final slots; row K-1 of a rollout's final_* arrays)
 cudaError_t macm_launch_reset_masked(const SimConst& P, const LaunchCfg& cfg, const uint8_t* mask, const SampleConst& sc,
-                                     cudaStream_t s);
+                                     const Finals& fin, const Finals& fin2, cudaStream_t s);
 cudaError_t macm_launch_sample(const SimConst& P, const SampleConst& sc, cudaStream_t s);
 cudaError_t macm_launch_overflow_count(const SimConst& P, int* d_out2, cudaStream_t s);
 cudaError_t macm_launch_pack_actions(const void* src, int elem_bytes, int width, uint64_t n_agents, void* out, cudaStream_t s);

@@ -16,7 +16,7 @@ ENV_FRESH, ENV_CONTACT_OVERFLOW, ENV_TOUCH_OVERFLOW = 1, 2, 4
 BOTS = {"idle": 0, "forward": 1, "rotate": 2, "diag": 3, "flock": 4, "random": 5, "combat": 6, "circle": 7}
 FLAG_REPAIR_MOV_COOLDOWN, FLAG_AUTO_RESET = 1, 2
 ENV_EPISODE_SHIFT = 8
-ABI_VERSION = 4
+ABI_VERSION = 5
 
 i32, f64, u64 = C.c_int32, C.c_double, C.c_uint64
 
@@ -58,13 +58,22 @@ class MacmLaunchInfo(C.Structure):
                [(n, C.c_float) for n in ("dt", "dt_ratio", "inv_mass", "damping_factor", "binary_d2_threshold")]
 
 
+# the arrays a reset copies an env's rows to before overwriting them (macm_final_out)
+FINAL_NAMES = ("obs", "nn_idx", "tdm_state", "env_state")
+
+
+class MacmFinalOut(C.Structure):
+    _fields_ = [(n, C.c_void_p) for n in FINAL_NAMES]
+
+
 class MacmRolloutOut(C.Structure):
-    _fields_ = [(n, C.c_void_p) for n in ("obs", "nn_idx", "rewards", "collided", "done")]
+    _fields_ = [(n, C.c_void_p) for n in ("obs", "nn_idx", "rewards", "collided", "done")] + \
+               [("final_" + n, C.c_void_p) for n in FINAL_NAMES]
 
 
 EXPORTS = ("macm_abi_version", "macm_strerror", "macm_last_cuda_error", "macm_params_default", "macm_create",
            "macm_destroy", "macm_get_buffer_sizes", "macm_get_launch_info", "macm_bind", "macm_reset",
-           "macm_sample_reset", "macm_reset_masked", "macm_set_auto_reset_seed", "macm_overflow_count", "macm_pack_actions",
+           "macm_sample_reset", "macm_reset_masked", "macm_bind_final", "macm_set_auto_reset_seed", "macm_overflow_count", "macm_pack_actions",
            "macm_step", "macm_rollout", "macm_observe", "macm_bot_actions", "macm_step_host", "macm_step_host_async", "macm_host_sync",
            "macm_host_alloc",
            "macm_host_free", "macm_launch_count", "macm_set_trace", "macm_enable_peer_access", "macm_ipc_open",
@@ -101,6 +110,7 @@ def lib():
         L.macm_reset.argtypes = [vp, vp]
         L.macm_sample_reset.argtypes = [vp, u64, vp]
         L.macm_reset_masked.argtypes = [vp, vp, u64, vp]
+        L.macm_bind_final.argtypes = [vp, C.POINTER(MacmFinalOut)]
         L.macm_set_auto_reset_seed.argtypes = [vp, u64]
         L.macm_overflow_count.argtypes = [vp, C.POINTER(i32), C.POINTER(i32), vp]
         L.macm_pack_actions.argtypes = [vp, vp, i32, i32, vp, vp]

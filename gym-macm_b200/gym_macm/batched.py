@@ -155,6 +155,20 @@ class Engine(object):
         _lib.check(L.macm_bind(h, C.byref(bufs)), h)
         self.E, self.N, self.T, self.C, self.obs_dim = E, N, T, Cc, D
         self.action_bytes = self.sizes.action_bytes
+        self.final = None
+
+    def bind_final(self):
+        """Allocate and bind (macm_bind_final) the final arrays: obs, env_state and nn_idx (Flock) / tdm_state (TDM),
+        shaped like the bound buffers of the same names.  Every reset copies the env's rows there first, so after a
+        reset `final` holds the finished episode's terminal observation and outcome; rows of envs that were never
+        reset keep their zeros."""
+        torch = _torch()
+        self.final = {n: torch.zeros_like(self.t[n]) for n in _lib.FINAL_NAMES if n in self.t}
+        f = _lib.MacmFinalOut()
+        for n, ten in self.final.items():
+            setattr(f, n, ten.data_ptr())
+        _lib.check(_lib.lib().macm_bind_final(self._h, C.byref(f)), self._h)
+        return self.final
 
     def close(self):
         h, self._h = self._h, None
@@ -219,7 +233,8 @@ class Engine(object):
     def rollout(self, actions, n_steps, policy=None, seed=0, out=None, stream=None):
         """macm_rollout: `n_steps` steps in one launch.  `actions` is a device tensor with a leading step
         axis, or None with `policy` = a _lib.BOTS code (the actions=None mode).  `out` maps any of
-        obs / nn_idx / rewards / collided / done to a device tensor with a leading step axis."""
+        obs / nn_idx / rewards / collided / done / final_obs / final_nn_idx / final_tdm_state / final_env_state to a
+        device tensor with a leading step axis (final_*: only rows of envs reset after that step are written)."""
         ro = _lib.MacmRolloutOut()
         for name, ten in (out or {}).items():
             setattr(ro, name, ten.data_ptr())
@@ -228,10 +243,14 @@ class Engine(object):
                                            C.c_uint64(int(seed) & (2 ** 64 - 1)), C.byref(ro), self._stream(stream)), self._h)
 
     def rollout_buffers(self, n_steps, want=("obs", "nn_idx", "rewards", "collided", "done")):
-        """Device tensors for the per-step outputs of rollout(): the bound output buffers with a leading step axis."""
+        """Device tensors for the per-step outputs of rollout(): the bound output buffers with a leading step axis.
+        final_obs / final_nn_idx / final_tdm_state / final_env_state have the shapes of obs / nn_idx / tdm_state /
+        env_state; row [k][e] is only defined where env e was reset after step k (auto_reset and done[k][e])."""
         torch = _torch()
-        return {n: torch.empty((int(n_steps),) + tuple(self.t[n].shape), dtype=self.t[n].dtype, device=self.device)
-                for n in want if n in self.t}
+        base = lambda n: n[len("final_"):] if n.startswith("final_") else n
+        return {n: torch.empty((int(n_steps),) + tuple(self.t[base(n)].shape), dtype=self.t[base(n)].dtype,
+                               device=self.device)
+                for n in want if base(n) in self.t and (n == base(n) or base(n) in _lib.FINAL_NAMES)}
 
     def observe(self):
         _lib.check(_lib.lib().macm_observe(self._h, self._stream()), self._h)
@@ -304,6 +323,24 @@ class _BatchedCommon(object):
                 raise _lib.MacmError("contact capacity overflow: %d envs dropped contacts (max_contacts=%d), %d envs "
                                      "exceeded the solver stage (max_touching=%d, limit 240); results of those envs "
                                      "differ from the reference's" % (c, self.engine.C, t, self.engine.sizes.max_touching))
+
+    def _final(self):
+        if self.engine.final is None:
+            raise _lib.MacmError("final_obs / final_info need keep_final=True")
+        return self.engine.final
+
+    @property
+    def final_info(self):
+        """The outcome of each env's last finished episode, from the env state a reset copies before it overwrites it
+        (keep_final=True): step_count, episode and overflowed, plus winner for TDM, each [E].  A row is valid where
+        `done` is set after an auto-reset step, or where a reset_done mask was set; other rows hold an earlier
+        episode's values (zeros before the first reset)."""
+        es = self._final()["env_state"]
+        info = {"step_count": es[:, 0], "episode": es[:, 1] >> _lib.ENV_EPISODE_SHIFT,
+                "overflowed": (es[:, 1] & (_lib.ENV_CONTACT_OVERFLOW | _lib.ENV_TOUCH_OVERFLOW)) != 0}
+        if self.engine.params.env_kind == _lib.TDM:
+            info["winner"] = es[:, 3]
+        return info
 
     def reset_done(self, mask=None, seed=0):
         """The reference's env.reset() (mvmnt.py:224-233, combat.py:229-239) for SOME envs of the batch: those
@@ -399,6 +436,8 @@ class BatchedFlock(_BatchedCommon):
             raise ValueError("targets must use the indices 0..T-1")
         self.actors, self.colors = actors, colors
         self.engine = Engine(flock_params(self.settings, self.n_envs, N, self.n_targets), device)
+        if self.settings.keep_final:
+            self.engine.bind_final()
         # Independent batches given a stream each overlap on the device (one batch's last envs finish while the
         # next batch starts); with stream=None every call goes to torch's current stream.
         self.engine.stream = stream
@@ -466,6 +505,14 @@ class BatchedFlock(_BatchedCommon):
                           {"type": 1, "id": self.engine.N, "position": o[..., D:2 * D]}]}
 
     @property
+    def final_obs(self):
+        """The terminal observation of each env's last finished episode (keep_final=True), laid out as `obs`: what
+        `obs` held when the env was last reset (valid rows: see final_info)."""
+        f, D = self._final(), self.engine.obs_dim // 2
+        return {"nodes": [{"type": 0, "id": f["nn_idx"], "position": f["obs"][..., 0:D]},
+                          {"type": 1, "id": self.engine.N, "position": f["obs"][..., D:2 * D]}]}
+
+    @property
     def rewards(self):
         return self.engine.t["rewards"]
 
@@ -508,7 +555,10 @@ class BatchedFlock(_BatchedCommon):
         reference's actions=None mode (mvmnt.py:86-92) with every agent driven by the scripted actor `policy`
         (test_scripts/bots.py).  Returns a dict of per-step tensors (leading axis K) for the names in `want`;
         with "obs" left out the observation pass only runs after the last step (action repeat).  The usual
-        attributes (obs, rewards, done, state) hold the last step's values afterwards."""
+        attributes (obs, rewards, done, state) hold the last step's values afterwards.  With auto_reset, `want` may
+        also name final_obs / final_nn_idx (Flock) / final_tdm_state (TDM) / final_env_state: the terminal rows of the
+        envs reset after each step; only rows [k][e] with done[k][e] set are defined, the others are left as
+        allocated (torch.empty)."""
         torch = _torch()
         E, N = self.engine.E, self.engine.N
         if actions is not None:
@@ -591,6 +641,8 @@ class BatchedTDM(_BatchedCommon):
             raise ValueError("at most 8 teams")
         self.actors, self.colors = actors, colors
         self.engine = Engine(tdm_params(self.settings, self.n_envs, N), device)
+        if self.settings.keep_final:
+            self.engine.bind_final()
         self.engine.stream = stream
         torch = _torch()
         self.engine.t["team"].copy_(torch.tensor(self.teams, dtype=torch.uint8))
@@ -654,6 +706,16 @@ class BatchedTDM(_BatchedCommon):
     def obs(self):
         o = self.engine.t["obs"].view(self.engine.E, self.engine.N, self.engine.N, 4)
         return {"myHealth": self.health, "myTeam": self.engine.t["team"], "alive": self.alive,
+                "agents": {"type": o[..., 3], "position": o[..., 0:3]}}
+
+    @property
+    def final_obs(self):
+        """The terminal observation of each env's last finished match (keep_final=True), laid out as `obs`, with
+        myHealth / alive from the final TDM state (valid rows: see final_info)."""
+        f = self._final()
+        o = f["obs"].view(self.engine.E, self.engine.N, self.engine.N, 4)
+        ts = f["tdm_state"]
+        return {"myHealth": ts[..., 0], "myTeam": self.engine.t["team"], "alive": (ts[..., 3].view(_torch().int32) & 1).bool(),
                 "agents": {"type": o[..., 3], "position": o[..., 0:3]}}
 
     @property

@@ -70,6 +70,7 @@ class _EnvSettings(fwSettings):
         self.env_index_base = 0            # global index of this batch's env 0 (gym_macm.dist shards)
         # batched hosts only (the reference has one world and a broken reset(), SURVEY App. B3):
         self.auto_reset = False            # an env whose `done` flag is set starts a new episode right after the step
+        self.keep_final = False            # keep each reset env's terminal observation and outcome (final_obs, final_info)
         self.check_overflow = False        # debug: step() raises when an env ran out of contact capacity
 
 

@@ -31,7 +31,7 @@
 extern "C" {
 #endif
 
-#define MACM_ABI_VERSION 4
+#define MACM_ABI_VERSION 5
 #define MACM_MAX_AGENTS 128  /* per environment (the reference has no cap, mvmnt.py:61); up to 64: two agents per lane,
                                 beyond: four, with 128-bit contact adjacency rows */
 #define MACM_MAX_TARGETS 16
@@ -59,7 +59,9 @@ enum {
     MACM_FLAG_AUTO_RESET = 2           /* every macm_step / macm_rollout launch is followed by macm_reset_masked(NULL):
                                           envs whose `done` flag is set start a new episode (see macm_reset_masked);
                                           inside a macm_rollout launch the same reset happens after every step, so the
-                                          per-step outputs are those of n_steps single steps with the flag set */
+                                          per-step outputs are those of n_steps single steps with the flag set; the
+                                          finished episode's terminal rows go to the final destinations first
+                                          (macm_bind_final, macm_rollout_out.final_*) */
 };
 /* env_state[e][1]: bits 0-2 flags, bits 8-31 the env's episode counter (incremented by macm_reset_masked) */
 enum {
@@ -215,6 +217,20 @@ int macm_sample_reset(macm_sim* sim, uint64_t seed, void* stream);
  * values of the env's last step (the learner reads the terminal reward next to the new episode's first observation;
  * the next step overwrites them).  One launch, no host synchronisation. */
 int macm_reset_masked(macm_sim* sim, const uint8_t* mask, uint64_t seed, void* stream);
+/* Final destinations: whenever the library resets an env -- macm_reset_masked, the launch MACM_FLAG_AUTO_RESET appends to
+ * a step or rollout, a rollout's in-launch reset -- it first copies that env's rows of obs, nn_idx (Flock), tdm_state
+ * (TDM) and env_state, as they stand at that moment, to the bound final arrays: the finished episode's terminal
+ * observation (a time-limit end is a truncation: a learner bootstraps from it) and its outcome (step count, overflow
+ * bits, TDM winner; TDM health / alive).  Rows of envs that are not reset are left untouched.  Any member may be NULL. */
+typedef struct macm_final_out {
+    float* obs;        /* [E,N,obs_dim]  16-byte aligned */
+    int32_t* nn_idx;   /* [E,N]          Flock only */
+    float* tdm_state;  /* [E,N,4]        TDM only, 16-byte aligned */
+    int32_t* env_state;/* [E,4]          16-byte aligned */
+} macm_final_out;
+/* Binds (the addresses are kept; caller-owned device memory) or, with f == NULL, unbinds the final arrays.
+ * MACM_E_ALIGN: a misaligned member; MACM_E_INVALID: nn_idx on TDM or tdm_state on Flock.  Nothing bound: no copies. */
+int macm_bind_final(macm_sim* sim, const macm_final_out* f);
 /* Seed of the resets that MACM_FLAG_AUTO_RESET appends to every step (default 0). */
 int macm_set_auto_reset_seed(macm_sim* sim, uint64_t seed);
 /* Device-side overflow summary: *contact_envs / *touching_envs receive how many envs currently carry
@@ -237,6 +253,12 @@ typedef struct macm_rollout_out {
     float* rewards;    /* [K,E,N] */
     uint8_t* collided; /* [K,E,N] */
     uint8_t* done;     /* [K,E] */
+    /* Terminal rows of the envs reset after step k (MACM_FLAG_AUTO_RESET on and done[k][e] set), as macm_bind_final
+     * describes; row [k][e] is written iff env e was reset after step k, every other row is left untouched. */
+    float* final_obs;        /* [K,E,N,obs_dim]  16-byte aligned */
+    int32_t* final_nn_idx;   /* [K,E,N]          Flock only */
+    float* final_tdm_state;  /* [K,E,N,4]        TDM only, 16-byte aligned */
+    int32_t* final_env_state;/* [K,E,4]          16-byte aligned */
 } macm_rollout_out;
 
 /* n_steps consecutive Flock.step / TDM.step calls for every env in ONE launch -- the reference's
@@ -244,7 +266,8 @@ typedef struct macm_rollout_out {
  * n_steps steps back to back with its bodies, fat AABBs and clocks held on chip; only the actions (in), the
  * per-step outputs (out) and the contact lists touch HBM between the steps.  Bit-identical to n_steps calls
  * of macm_step: the bound state and output buffers end up exactly as after the last of those calls, and
- * out->x[k] holds what buffer x held after call k.
+ * out->x[k] holds what buffer x held after call k.  The same holds for the bound final arrays (each holds the latest
+ * terminal row of its env) and out->final_x[k] holds what final array x received from the reset after call k.
  *   actions != NULL : [n_steps,E,N,4] uint8 (discrete) or [n_steps,E,N,2] float (continuous), device.
  *   actions == NULL : the actions=None mode (mvmnt.py:86-92): every agent's actor picks its action from
  *                     its own last observation, policy = MACM_BOT_* as in macm_bot_actions (MACM_BOT_FLOCK: Flock
