@@ -90,6 +90,13 @@ def make_pair(E, N, targets=None, seed=0, spread=20.0, max_contacts=0, max_touch
     env = gym_macm.BatchedFlock(E, n_agents=[N], targets=targets, device="cuda:0", seed=None,
                                 max_contacts=max_contacts, max_touching=max_touching, **kw)
     env.load_state(pos, ang, targets=tg)
+    ref = oracle.OracleBatch(E, n_agents=N, n_targets=T, **oracle_kwargs(kw))
+    ref.reset(pos, ang, targets=tg, target_idx=targets)
+    return env, ref, rng
+
+
+def oracle_kwargs(kw):
+    """BatchedFlock settings keywords -> the OracleBatch parameters they set."""
     okw = {}
     if "reward_mode" in kw: okw["reward_mode"] = {"binary": 0, "linear": 1}[kw["reward_mode"]]
     if "action_mode" in kw: okw["action_mode"] = {"discrete": 0, "continuous": 1}[kw["action_mode"]]
@@ -99,9 +106,7 @@ def make_pair(E, N, targets=None, seed=0, spread=20.0, max_contacts=0, max_touch
                    ("positionIterations", "position_iterations"), ("agent_force", "agent_force"),
                    ("_reward_radius", "reward_radius"), ("enableWarmStarting", "warm_starting")):
         if k_ in kw: okw[ok] = kw[k_]
-    ref = oracle.OracleBatch(E, n_agents=N, n_targets=T, **okw)
-    ref.reset(pos, ang, targets=tg, target_idx=targets)
-    return env, ref, rng
+    return okw
 
 
 def run_parity(E, N, steps, targets=None, seed=0, spread=20.0, policy="random", check_every=1, **kw):

@@ -49,6 +49,12 @@ def rollout_case(rng, N, E, kw):
     return K
 
 
+def capacity(rng, N):
+    """max_touching of a case: the library default (0), the shared-memory stage's 240, or full capacity N(N-1)/2,
+    which is more than 240 from 23 agents on and then runs the kernels of macm_kernels_huge.cu."""
+    return int(rng.choice([0, 240, N * (N - 1) // 2]))
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--seconds", type=float, default=180.0)
@@ -58,17 +64,22 @@ def main():
     rng = np.random.default_rng(args.seed)
     t0, cases, agent_steps, worst_tc, skipped = time.time(), 0, 0, 0, 0
     tdm_cases, deaths = 0, 0
+    # per build: the default kernels, or those of macm_kernels_huge.cu (max_touching above 240)
+    by_build = {"default": {"flock": 0, "tdm": 0}, "huge": {"flock": 0, "tdm": 0}}
     while time.time() - t0 < args.seconds:
         if rng.random() < args.tdm:
             n_teams = int(rng.integers(2, 5))
             teams = [int(rng.integers(1, (128 if rng.random() < 0.2 else 64) // n_teams + 1)) for _ in range(n_teams)]
             side = float(rng.choice([3.0, 6.0, 12.0, 30.0]))
-            desc = dict(kind="tdm", teams=teams, side=side)
+            N = sum(teams)
+            mt = capacity(rng, N)
+            desc = dict(kind="tdm", teams=teams, side=side, max_touching=mt)
             try:
                 steps = int(rng.integers(100, 500))
                 E = int(rng.choice([4, 24]))
                 deaths += run_tdm(E, teams, steps, seed=int(rng.integers(0, 1 << 30)), width=side, height=side,
-                                  attack_p=float(rng.choice([0.2, 0.5, 0.9])), check_every=int(rng.choice([1, 7])))
+                                  attack_p=float(rng.choice([0.2, 0.5, 0.9])), check_every=int(rng.choice([1, 7])),
+                                  max_touching=mt)
             except AssertionError as ex:
                 if "overflow" in str(ex):
                     skipped += 1
@@ -76,6 +87,7 @@ def main():
                 print("MISMATCH", json.dumps(desc), str(ex)[:300], flush=True)
                 sys.exit(1)
             tdm_cases += 1
+            by_build["huge" if mt > 240 else "default"]["tdm"] += 1
             agent_steps += E * sum(teams) * steps
             continue
         N = int(rng.choice([2, 3, 4, 5, 6, 7, 8, 9, 12, 16, 17, 24, 31, 32, 33, 40, 45, 48, 63, 64, 65, 80, 100, 128]))
@@ -97,12 +109,13 @@ def main():
         policy = "random"
         if kw["action_mode"] == "discrete" and kw["coord"] == "polar" and rng.random() < 0.25:
             policy = str(rng.choice(["flock", "idle"]))
-        desc = dict(N=N, E=E, spread=round(spread, 2), steps=steps, policy=policy, targets=targets, **kw)
+        mt = capacity(rng, N)
+        desc = dict(N=N, E=E, spread=round(spread, 2), steps=steps, policy=policy, targets=targets, max_touching=mt, **kw)
         try:
             st = run_parity(E, N, steps, targets=targets, seed=int(rng.integers(0, 1 << 30)), spread=spread, policy=policy,
-                            max_contacts=N * (N - 1) // 2, max_touching=N * (N - 1) // 2, **kw)
+                            max_contacts=N * (N - 1) // 2, max_touching=mt, **kw)
             if cases % 4 == 0:
-                rollout_case(rng, N, E, {k: v for k, v in kw.items()})
+                rollout_case(rng, N, E, dict(kw, max_contacts=N * (N - 1) // 2, max_touching=mt))
         except AssertionError as ex:
             if "capacity overflow" in str(ex):
                 # more than 240 touching contacts at once (an unphysical spawn pile: bodies that do not overlap cannot
@@ -114,9 +127,11 @@ def main():
             print("MISMATCH", json.dumps(desc), str(ex)[:300], flush=True)
             sys.exit(1)
         cases += 1
+        by_build["huge" if mt > 240 else "default"]["flock"] += 1
         agent_steps += E * N * steps
         worst_tc = max(worst_tc, st["max_touching"])
     print(json.dumps({"cases": cases, "tdm_cases": tdm_cases, "tdm_deaths_at_case_end": deaths, "agent_steps_checked": agent_steps, "max_touching_seen": worst_tc, "overflow_reported_by_device": skipped,
+                      "cases_by_build": by_build,
                       "seconds": round(time.time() - t0, 1), "seed": args.seed}))
 
 
