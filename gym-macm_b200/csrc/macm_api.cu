@@ -384,10 +384,6 @@ extern "C" int macm_bind(macm_sim* sim, const macm_buffers* b)
     K.obs = b->obs; K.nn_idx = b->nn_idx; K.rewards = b->rewards; K.collided = b->collided; K.done = b->done;
     if (K.TCH > 0 && (!b->touch_scratch || !aligned(b->touch_scratch, 16))) return b->touch_scratch ? MACM_E_ALIGN : MACM_E_UNBOUND;
     K.scratch = K.TCH > 0 ? b->touch_scratch : nullptr;
-    K.bulk = flock && K.action_mode == MACM_ACTION_DISCRETE && sim->cfg.G == 32 && (K.N & 3) == 0 && K.C >= 32 &&
-             28 * K.N + 384 <= 24 * K.TC && aligned(b->angsleep, 16) && aligned(b->contact_ab, 16) &&
-             aligned(b->contact_imp, 16) && ((K.C * 4) & 15) == 0;
-    if (getenv("MACM_NO_BULK")) K.bulk = 0;   // experiments
     sim->bound = 1;
     return MACM_OK;
 }

@@ -41,9 +41,6 @@
 // block sets the kernel time; warps of one block are served evenly.)
 #define MACM_WIDE_THREADS 896
 #define MACM_TABLE_BYTES (418 * 16)   // sin/cos(k/128) as double2, staged per block in the wide launch
-#ifndef MACM_SMALL_BLOCKS
-#define MACM_SMALL_BLOCKS 7   // several envs per warp (N <= 16): 128-thread blocks; 8 or 9 blocks (64 / 56 registers) measured no faster
-#endif
 
 // Phase stamps for profiles/phase_trace.py (a separate build with -DMACM_PHASE_TRACE; the trace
 // buffer then holds 16 words per env: SM clock at the end of each phase, relative to the start).
@@ -55,16 +52,81 @@
 
 namespace {
 
-// Agent sets: one bit per agent of an env.  Up to 64 agents: a uint2 (word = agent >> 5); 65..128 agents (four agents per
-// lane): four words.  Everything that existed before the wide shape keeps its uint2 code verbatim.
-struct Set4 { uint32_t w[4]; };
-template <int NC> struct SetOf { typedef uint2 type; };
-template <> struct SetOf<128> { typedef Set4 type; };
-template <typename T> __device__ __forceinline__ T empty_set();
-template <> __device__ __forceinline__ uint2 empty_set<uint2>() { return make_uint2(0u, 0u); }
-template <> __device__ __forceinline__ Set4 empty_set<Set4>() { Set4 r; r.w[0] = r.w[1] = r.w[2] = r.w[3] = 0u; return r; }
-__device__ __forceinline__ bool set_nonzero(uint2 m) { return (m.x | m.y) != 0u; }
-__device__ __forceinline__ bool set_nonzero(const Set4& m) { return (m.w[0] | m.w[1] | m.w[2] | m.w[3]) != 0u; }
+// Agent sets: one bit per agent of an env, agent i in bit i & 31 of word i >> 5 (slot s of a 32-lane group is word s).
+// Two words for envs of up to 64 agents, four beyond; a set is aligned to its size, so that a row of a set array in
+// shared memory is one vector access.  A set in registers is only ever indexed by a word number known at compile time,
+// or through compares on the agent (word_of, add_bit, drop_bit): a subscript known only at run time would put the set in
+// local memory.
+template <int W>
+struct __align__(4 * W) Bits { uint32_t w[W]; };
+template <int NC> using AgentSet = Bits<(NC > 64) ? 4 : 2>;
+
+// agent i falls in word k of a W-word set (the last word takes every i >= 32 * (W - 1))
+template <int W>
+__device__ __forceinline__ bool in_word(int i, int k) { return (k == 0 || i >= 32 * k) && (k == W - 1 || i < 32 * k + 32); }
+template <int W>
+__device__ __forceinline__ uint32_t word_of(const Bits<W>& m, int i)   // the word that holds agent i
+{
+    uint32_t r = m.w[W - 1];
+#pragma unroll
+    for (int k = W - 2; k >= 0; --k) r = i < 32 * k + 32 ? m.w[k] : r;
+    return r;
+}
+template <int W>
+__device__ __forceinline__ bool bit_of(const Bits<W>& m, int i) { return (word_of(m, i) >> (i & 31)) & 1u; }
+template <int W>
+__device__ __forceinline__ void add_bit(Bits<W>& m, int i)
+{
+#pragma unroll
+    for (int k = 0; k < W; ++k)
+        if (in_word<W>(i, k)) m.w[k] |= 1u << (i & 31);
+}
+template <int W>
+__device__ __forceinline__ void drop_bit(Bits<W>& m, int i)
+{
+#pragma unroll
+    for (int k = 0; k < W; ++k)
+        if (in_word<W>(i, k)) m.w[k] &= ~(1u << (i & 31));
+}
+// atomically adds agent `bit` to row r of a set array in shared memory (the word address: a compare for two words, a
+// shift for four -- what ptxas turns into the fewer instructions at each width)
+template <int W>
+__device__ __forceinline__ void or_bit(Bits<W>* row, int r, int bit)
+{
+    atomicOr(W == 2 ? (bit < 32 ? &row[r].w[0] : &row[r].w[1]) : &row[r].w[bit >> 5], 1u << (bit & 31));
+}
+// the ballot of slot s (agents s*G .. s*G + G - 1) into a set that starts out empty: the first slot of a word assigns it
+template <int G, int W>
+__device__ __forceinline__ void put_slot(Bits<W>& m, int s, unsigned bm)
+{
+    const int k = (s * G) >> 5, sh = (s * G) & 31;
+    m.w[k] = (sh ? m.w[k] : 0u) | (bm << sh);
+}
+template <int W>
+__device__ __forceinline__ bool set_nonzero(const Bits<W>& m)
+{
+    uint32_t r = 0u;
+#pragma unroll
+    for (int k = 0; k < W; ++k) r |= m.w[k];
+    return r != 0u;
+}
+template <int W>
+__device__ __forceinline__ int set_count(const Bits<W>& m)
+{
+    int r = 0;
+#pragma unroll
+    for (int k = 0; k < W; ++k) r += __popc(m.w[k]);
+    return r;
+}
+template <int W>
+__device__ __forceinline__ int highest_of(const Bits<W>& m)   // the highest agent of the set, -1 if it is empty
+{
+    int r = -1;
+#pragma unroll
+    for (int k = W - 1; k >= 0; --k)
+        if (r < 0 && m.w[k]) r = k * 32 + 31 - __clz((int)m.w[k]);
+    return r;
+}
 
 // ------------------------------------------------------------------------------------------
 // shared-memory layout of one environment
@@ -74,12 +136,12 @@ struct Lay {
     static constexpr int POS = 0;                 // float2 [NC]  centre
     static constexpr int VEL = POS + 8 * NC;      // float2 [NC]  linear velocity
     static constexpr int FAT = VEL + 8 * NC;      // float4 [NC]  fat AABB lo.xy hi.xy
-    static constexpr int ROWB = NC > 64 ? 16 : 8; // bytes of one agent-set row: 64 agents in a uint2, 128 in four words
+    static constexpr int ROWB = sizeof(AgentSet<NC>);   // bytes of one agent-set row
     static constexpr int ADJ = FAT + 16 * NC;     // set    [NC]  contact adjacency row (agents 0-31, 32-63, ...)
-    // One 8-byte-per-agent scratch region, used by phases that never overlap in time:
+    // One agent-set row per agent of scratch, used by phases that never overlap in time:
     //   phase 1b  float2 [NC]  far end of an attacker's ray (TDM)
     //   phase 8   u32    [NC]  min sleep time of the island seeded here            (first half)
-    //   phase 2a/10  uint2 [NC]  new-pair row being assembled (re-zeroed on entry)
+    //   phase 2a/10  set [NC]  new-pair row being assembled (re-zeroed on entry)
     //   phase 12-13  float [NC]  body angle for the TDM observation pass           (second half)
     static constexpr int NEW = ADJ + ROWB * NC;
     static constexpr int ISLMIN = NEW;
@@ -93,10 +155,8 @@ struct Lay {
     // dense piles only (more touching contacts than lanes, dense_* below):
     static constexpr int LASTLVL = SOLVED + NC, ISLACT = LASTLVL + NC, ISLBAD = ISLACT + NC;
     static constexpr int HEAD = ISLBAD + NC;      // u8     [NC]  newest touching contact of a body
-    // 4 x u32, used by phases that never overlap in time:
-    //   phase 0 (MACM_BULK_STAGE build)  two mbarriers of the bulk state copies
-    //   phases 5-7 (macm_kernels_huge.cu)  word 0: contacts of a dense pile in the global-memory stage (0: the env is in
-    //                                      the shared-memory stage), from the velocity to the position part
+    // 4 x u32; word 0, phases 5-7 of macm_kernels_huge.cu: contacts of a dense pile in the global-memory stage (0: the
+    // env is in the shared-memory stage), from the velocity to the position part
     static constexpr int MISC = (HEAD + NC + 15) / 16 * 16;
     static constexpr int FIXED = MISC + 16;
     // per touching contact (capacity TC, a multiple of 16):
@@ -125,9 +185,8 @@ struct EnvS {
     __device__ float2* pos() const { return (float2*)(base + Lay<NC>::POS); }
     __device__ float2* vel() const { return (float2*)(base + Lay<NC>::VEL); }
     __device__ float4* fat() const { return (float4*)(base + Lay<NC>::FAT); }
-    typedef typename SetOf<NC>::type SetT;
-    __device__ SetT* adj() const { return (SetT*)(base + Lay<NC>::ADJ); }
-    __device__ SetT* nw() const { return (SetT*)(base + Lay<NC>::NEW); }
+    __device__ AgentSet<NC>* adj() const { return (AgentSet<NC>*)(base + Lay<NC>::ADJ); }
+    __device__ AgentSet<NC>* nw() const { return (AgentSet<NC>*)(base + Lay<NC>::NEW); }
     __device__ uint32_t* isl_min() const { return (uint32_t*)(base + Lay<NC>::ISLMIN); }
     __device__ float* ang() const { return (float*)(base + Lay<NC>::ANG); }
     __device__ float2* tgt() const { return (float2*)(base + Lay<NC>::TGT); }
@@ -179,20 +238,6 @@ struct Grp {
     }
 };
 
-// 64-bit agent sets as two words: agent i -> word i >> 5, bit i & 31 (slot s of a 32-lane group is word s)
-__device__ __forceinline__ bool bit_of(uint2 m, int i) { return (((i < 32) ? m.x : m.y) >> (i & 31)) & 1u; }
-__device__ __forceinline__ void or_bit(uint2* row, int r, int bit)
-{
-    atomicOr(bit < 32 ? &row[r].x : &row[r].y, 1u << (bit & 31));
-}
-__device__ __forceinline__ bool bit_of(const Set4& m, int i) { return (m.w[i >> 5] >> (i & 31)) & 1u; }
-__device__ __forceinline__ void or_bit(Set4* row, int r, int bit) { atomicOr(&row[r].w[bit >> 5], 1u << (bit & 31)); }
-// the ballot of slot s (agents s*G .. s*G + G - 1) into an agent set that starts out empty
-template <int G>
-__device__ __forceinline__ void put_slot(uint2& m, int s, unsigned bm) { if (s == 0) m.x = bm; else m.y = bm; }
-template <int G>
-__device__ __forceinline__ void put_slot(Set4& m, int s, unsigned bm) { m.w[(s * G) >> 5] |= bm << ((s * G) & 31); }
-
 // Packed fp32x2 arithmetic of sm_100 (FADD2 / FMUL2): two IEEE round-to-nearest operations per
 // instruction, bit-identical to the scalar ones.  (A packed multiply feeding a packed add would be
 // contracted into FFMA2 by ptxas even with .rn, so sums of products are finished with scalar adds.)
@@ -208,35 +253,6 @@ __device__ __forceinline__ void prefetch_l2(int gl, const void* p, int bytes)
 {
     for (int off = gl * 128; off < bytes; off += G * 128)
         asm volatile("prefetch.global.L2 [%0];" ::"l"((const char*)p + off));
-}
-
-// 1-D bulk asynchronous copies global -> shared memory, completion counted in bytes on an mbarrier (TMA unit, no
-// tensor map): the step kernel fetches an env's contiguous state rows with a handful of instructions on one lane.
-__device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ __attribute__((unused)) void mbar_init(uint32_t bar, int count)
-{
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(bar), "r"(count));
-}
-__device__ __forceinline__ void mbar_expect_tx(uint32_t bar, int bytes)
-{
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void bulk_g2s(uint32_t dst, const void* src, int bytes, uint32_t bar)
-{
-    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-                 ::"r"(dst), "l"(src), "r"(bytes), "r"(bar) : "memory");
-}
-__device__ __forceinline__ void mbar_wait(uint32_t bar, int parity)
-{
-    asm volatile(
-        "{\n"
-        ".reg .pred p;\n"
-        "WAIT_%=:\n"
-        "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1;\n"
-        "@p bra DONE_%=;\n"
-        "bra WAIT_%=;\n"
-        "DONE_%=:\n"
-        "}" ::"r"(bar), "r"(parity) : "memory");
 }
 
 // b2TestOverlap(b2AABB, b2AABB): d1 = b.lo - a.hi, d2 = a.lo - b.hi; overlap iff no component > 0.
@@ -383,114 +399,29 @@ __device__ __forceinline__ float solve_position(float radius, float k_sum, float
 // Appends to the HBM contact list at `cnt`; returns the new count (uniform over the group).
 // ------------------------------------------------------------------------------------------
 template <int G, int APL>
-__device__ int find_new_contacts(const Grp<G>& g, const EnvS<G * APL>& S, const SimConst& P, uint2 moved, uint2 alive,
-                                 int cnt, uint32_t* c_ab, float2* c_imp, bool& overflow)
+__device__ int find_new_contacts(const Grp<G>& g, const EnvS<G * APL>& S, const SimConst& P, const AgentSet<G * APL>& moved,
+                                 const AgentSet<G * APL>& alive, int cnt, uint32_t* c_ab, float2* c_imp, bool& overflow)
 {
+    typedef AgentSet<G * APL> Set;
+    constexpr int W = sizeof(Set) / 4, NW = (G * APL + 31) / 32;   // words of a set, words that can hold an agent
     const float4* fat = S.fat();
-    uint2* adj = S.adj();
-    uint2* nw = S.nw();
+    Set* adj = S.adj();
+    Set* nw = S.nw();
 
-    uint2 hit[APL];
+    Set hit[APL];
     float4 own[APL];
 #pragma unroll
     for (int s = 0; s < APL; ++s) {
         const int i = g.gl + s * G;
-        hit[s] = make_uint2(0u, 0u);
+        hit[s] = Set{};
         own[s] = fat[i];
         // dead / padding agents have no proxy: park their box where nothing overlaps it
         if (!bit_of(alive, i)) own[s] = make_float4(3.0e38f, 3.0e38f, -3.0e38f, -3.0e38f);
-        nw[i] = make_uint2(0u, 0u);
+        nw[i] = Set{};
     }
     g.sync();
 #pragma unroll
-    for (int w = 0; w < (G * APL + 31) / 32; ++w) {
-        for (unsigned mm = w ? moved.y : moved.x; mm; mm &= mm - 1) {
-            const int m = w * 32 + __ffs((int)mm) - 1;
-            const float4 mb = fat[m];
-            const unsigned bit = 1u << (m & 31);
-#pragma unroll
-            for (int s = 0; s < APL; ++s) {
-                const bool h = (g.gl + s * G != m) && aabb_overlap(mb, own[s]);
-                if (w == 0) hit[s].x |= h ? bit : 0u; else hit[s].y |= h ? bit : 0u;
-            }
-        }
-    }
-    // pair (m, i) with m < i belongs to row m: the owner of m finds it itself iff i moved too;
-    // otherwise the owner of i posts it
-#pragma unroll
-    for (int s = 0; s < APL; ++s) {
-        const int i = g.gl + s * G;
-        if (!bit_of(moved, i)) {
-            unsigned lo = hit[s].x, hi = hit[s].y;
-            if (i < 32) { lo &= (1u << i) - 1u; hi = 0u; } else { hi &= (1u << (i - 32)) - 1u; }
-            for (; lo; lo &= lo - 1) or_bit(nw, __ffs((int)lo) - 1, i);
-            for (; hi; hi &= hi - 1) or_bit(nw, 32 + __ffs((int)hi) - 1, i);
-        }
-    }
-    g.sync();
-    uint2 fresh[APL];
-    bool any = false;
-#pragma unroll
-    for (int s = 0; s < APL; ++s) {
-        const int i = g.gl + s * G;
-        uint2 row = hit[s];
-        // keep partners j > i only
-        if (i < 32) row.x &= ~((2u << i) - 1u); else { row.x = 0u; row.y &= ~((2u << (i - 32)) - 1u); }
-        const uint2 posted = nw[i], have = adj[i];
-        fresh[s] = make_uint2((row.x | posted.x) & ~have.x, (row.y | posted.y) & ~have.y);
-        any |= (fresh[s].x | fresh[s].y) != 0u;
-    }
-    if (!g.ballot(any)) return cnt;
-    int base = cnt;
-#pragma unroll
-    for (int s = 0; s < APL; ++s) {
-        const int i = g.gl + s * G;
-        const int c = __popc(fresh[s].x) + __popc(fresh[s].y);
-        const int incl = g.scan_incl(c);
-        const int total = g.shfl(incl, G - 1);
-        int pos = base + incl - c;
-#pragma unroll
-        for (int w = 0; w < 2; ++w) {
-            for (unsigned f = w ? fresh[s].y : fresh[s].x; f; f &= f - 1) {
-                const int j = w * 32 + __ffs((int)f) - 1;
-                if (pos < P.C) {
-                    c_ab[pos] = (uint32_t)i | ((uint32_t)j << 8);
-                    c_imp[pos] = make_float2(0.0f, 0.0f);
-                    or_bit(adj, i, j);
-                    or_bit(adj, j, i);
-                } else {
-                    overflow = true;
-                }
-                ++pos;
-            }
-        }
-        base += total;
-    }
-    g.sync();
-    return base < P.C ? base : P.C;
-}
-
-// The same for envs of 65..128 agents (four words per set): rows and bit scans run over the words.
-template <int G, int APL>
-__device__ int find_new_contacts(const Grp<G>& g, const EnvS<G * APL>& S, const SimConst& P, const Set4& moved, const Set4& alive,
-                                 int cnt, uint32_t* c_ab, float2* c_imp, bool& overflow)
-{
-    const float4* fat = S.fat();
-    Set4* adj = S.adj();
-    Set4* nw = S.nw();
-    Set4 hit[APL];
-    float4 own[APL];
-#pragma unroll
-    for (int s = 0; s < APL; ++s) {
-        const int i = g.gl + s * G;
-        hit[s] = empty_set<Set4>();
-        own[s] = fat[i];
-        if (!bit_of(alive, i)) own[s] = make_float4(3.0e38f, 3.0e38f, -3.0e38f, -3.0e38f);
-        nw[i] = empty_set<Set4>();
-    }
-    g.sync();
-#pragma unroll
-    for (int w = 0; w < 4; ++w) {
+    for (int w = 0; w < NW; ++w) {
         for (unsigned mm = moved.w[w]; mm; mm &= mm - 1) {
             const int m = w * 32 + __ffs((int)mm) - 1;
             const float4 mb = fat[m];
@@ -502,31 +433,34 @@ __device__ int find_new_contacts(const Grp<G>& g, const EnvS<G * APL>& S, const 
             }
         }
     }
+    // pair (m, i) with m < i belongs to row m: the owner of m finds it itself iff i moved too;
+    // otherwise the owner of i posts it
 #pragma unroll
     for (int s = 0; s < APL; ++s) {
         const int i = g.gl + s * G;
         if (!bit_of(moved, i)) {
 #pragma unroll
-            for (int w = 0; w < 4; ++w) {
+            for (int w = 0; w < NW; ++w) {
                 unsigned lo = hit[s].w[w];
-                if (w == (i >> 5)) lo &= (1u << (i & 31)) - 1u;      // partners m < i only
-                if (w > (i >> 5)) lo = 0u;
+                if (in_word<W>(i, w)) lo &= (1u << (i & 31)) - 1u;   // partners m < i only
+                if (w > 0 && i < 32 * w) lo = 0u;
                 for (; lo; lo &= lo - 1) or_bit(nw, w * 32 + __ffs((int)lo) - 1, i);
             }
         }
     }
     g.sync();
-    Set4 fresh[APL];
+    Set fresh[APL];
     bool any = false;
 #pragma unroll
     for (int s = 0; s < APL; ++s) {
         const int i = g.gl + s * G;
-        const Set4 posted = nw[i], have = adj[i];
+        const Set posted = nw[i], have = adj[i];
+        fresh[s] = Set{};
 #pragma unroll
-        for (int w = 0; w < 4; ++w) {
+        for (int w = 0; w < NW; ++w) {
             unsigned row = hit[s].w[w];
-            if (w == (i >> 5)) row &= ~((2u << (i & 31)) - 1u);      // keep partners j > i only
-            if (w < (i >> 5)) row = 0u;
+            if (in_word<W>(i, w)) row &= ~((2u << (i & 31)) - 1u);   // keep partners j > i only
+            if (w < W - 1 && i >= 32 * w + 32) row = 0u;
             fresh[s].w[w] = (row | posted.w[w]) & ~have.w[w];
         }
         any |= set_nonzero(fresh[s]);
@@ -536,12 +470,12 @@ __device__ int find_new_contacts(const Grp<G>& g, const EnvS<G * APL>& S, const 
 #pragma unroll
     for (int s = 0; s < APL; ++s) {
         const int i = g.gl + s * G;
-        const int c = __popc(fresh[s].w[0]) + __popc(fresh[s].w[1]) + __popc(fresh[s].w[2]) + __popc(fresh[s].w[3]);
+        const int c = set_count(fresh[s]);
         const int incl = g.scan_incl(c);
         const int total = g.shfl(incl, G - 1);
         int pos = base + incl - c;
 #pragma unroll
-        for (int w = 0; w < 4; ++w) {
+        for (int w = 0; w < NW; ++w) {
             for (unsigned f = fresh[s].w[w]; f; f &= f - 1) {
                 const int j = w * 32 + __ffs((int)f) - 1;
                 if (pos < P.C) {
@@ -855,7 +789,7 @@ __device__ void flock_observe(const Grp<G>& g, const EnvS<G * APL>& S, const Sim
 // an entry is selected, not jumped around), row pointers advanced instead of recomputed.
 template <int G, int APL>
 __device__ void tdm_observe(const Grp<G>& g, const EnvS<G * APL>& S, const SimConst& P, int env,
-                            const typename SetOf<G * APL>::type& alive, float* ob1, float* ob2)
+                            const AgentSet<G * APL>& alive, float* ob1, float* ob2)
 {
     const float2* pos = S.pos();
     const float* angs = S.ang();
@@ -972,29 +906,23 @@ __device__ __forceinline__ int dense_islands(const Grp<G>& g, const EnvS<G * APL
     int L = 1;
     if (g.gl == 0) {
         uint8_t* stack = S.stack();
-        constexpr int W = G * APL > 64 ? 4 : 2;
-        uint32_t rem[W];   // bodies with a touching contact that are not in an island yet
-#pragma unroll
-        for (int w = 0; w < W; ++w) rem[w] = 0u;
+        AgentSet<G * APL> rem = {};   // bodies with a touching contact that are not in an island yet
         for (int t = 0; t < tc; ++t) {
             const uint32_t w = st.edge(t);
             const int a = St::a(w), b = St::b(w);
             st.link(t, w, st.head[a], st.head[b]);
             st.head[a] = t;
             st.head[b] = t;
-            rem[a >> 5] |= 1u << (a & 31);
-            rem[b >> 5] |= 1u << (b & 31);
+            add_bit(rem, a);
+            add_bit(rem, b);
         }
         int nord = 0;
         for (;;) {
-            int seed = -1;   // the highest body left: Box2D walks its body list from the last-created body
-#pragma unroll
-            for (int w = W - 1; w >= 0; --w)
-                if (seed < 0 && rem[w]) seed = w * 32 + 31 - __clz((int)rem[w]);
+            const int seed = highest_of(rem);   // the highest body left: Box2D walks its body list from the last-created body
             if (seed < 0) break;
             int sp = 0;
             stack[sp++] = (uint8_t)seed;
-            rem[seed >> 5] &= ~(1u << (seed & 31));
+            drop_bit(rem, seed);
             while (sp > 0) {
                 const int b = stack[--sp];
                 label[b] = (uint32_t)seed;
@@ -1010,8 +938,7 @@ __device__ __forceinline__ int dense_islands(const Grp<G>& g, const EnvS<G * APL
                         st.lastlvl[tb] = l;
                         L = max(L, l);
                         const int other = (ta == b) ? tb : ta;
-                        const uint32_t ob = 1u << (other & 31);
-                        if (rem[other >> 5] & ob) { rem[other >> 5] &= ~ob; stack[sp++] = (uint8_t)other; }
+                        if (bit_of(rem, other)) { drop_bit(rem, other); stack[sp++] = (uint8_t)other; }
                     }
                     t = nx;
                 }
@@ -1184,11 +1111,10 @@ __device__ __noinline__ void dense_solve_position_huge(const Grp<G>& g, const En
 // the first step after a reset only; out of line.
 template <int G, int APL>
 __device__ __noinline__ int fresh_world_contacts(const Grp<G>& g, const EnvS<G * APL>& S, const SimConst& P,
-                                                 typename SetOf<G * APL>::type alive, int cnt, uint32_t* c_ab, float2* c_imp,
+                                                 AgentSet<G * APL> alive, int cnt, uint32_t* c_ab, float2* c_imp,
                                                  bool& overflow)
 {
-    typedef typename SetOf<G * APL>::type SetT;
-    SetT* adj = S.adj();
+    AgentSet<G * APL>* adj = S.adj();
     for (int base = 0; base < cnt; base += G) {
         const int k = base + g.gl;
         if (k < cnt) {
@@ -1200,7 +1126,7 @@ __device__ __noinline__ int fresh_world_contacts(const Grp<G>& g, const EnvS<G *
     g.sync();
     cnt = find_new_contacts<G, APL>(g, S, P, alive, alive, cnt, c_ab, c_imp, overflow);
 #pragma unroll
-    for (int s = 0; s < APL; ++s) adj[g.gl + s * G] = empty_set<SetT>();
+    for (int s = 0; s < APL; ++s) adj[g.gl + s * G] = AgentSet<G * APL>{};
     g.sync();
     return cnt;
 }
@@ -1245,9 +1171,9 @@ __device__ __noinline__ uint32_t bot_action(const SimConst& P, const Rollout& R,
 // from the staged positions and angles with the arithmetic of tdm_observe, so the choice is the one
 // macm_bot_kernel makes from the `obs` buffer: nearest enemy (lowest index among equal r), turn towards it,
 // walk when it is within +-36 degrees, strike inside 3 m.
-template <typename SetT>
+template <int W>
 __device__ __noinline__ uint32_t combat_action(const float2* pos, const float* angs, const uint8_t* team, int N,
-                                               SetT alive, int i)
+                                               Bits<W> alive, int i)
 {
     uint32_t a0 = 1, a2 = 1, a3 = 0;
     if (i < N && bit_of(alive, i)) {
@@ -1330,7 +1256,7 @@ __global__ void __launch_bounds__(shape_max_threads(G, APL), 1) macm_step_kernel
     S.base = smem_raw + (size_t)slot_in_block * Lay<NC>::bytes(P.TC);
 
     float2* pos = S.pos(); float2* vel = S.vel(); float4* fat = S.fat();
-    typedef typename SetOf<NC>::type ASet;
+    typedef AgentSet<NC> ASet;
     ASet* adj = S.adj();
     uint32_t* label = S.label();
     uint32_t* tmask = S.tmask();
@@ -1371,14 +1297,6 @@ __global__ void __launch_bounds__(shape_max_threads(G, APL), 1) macm_step_kernel
             prefetch_l2<G>(g.gl, P.angsleep + a0, P.N * 8);
         }
     }
-#ifdef MACM_BULK_STAGE
-    if (!TDM && G == 32 && P.bulk && g.gl == 0) {   // the two mbarriers of the bulk state copies (phase 0)
-        mbar_init(smem_u32(S.misc()), 1);
-        mbar_init(smem_u32(S.misc()) + 8, 1);
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
-    __syncwarp();
-#endif
     asm volatile("griddepcontrol.wait;" ::: "memory");
     asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
     if (P.trace) { asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(tr_t0)); tr_c0 = clock64(); }
@@ -1398,30 +1316,7 @@ __global__ void __launch_bounds__(shape_max_threads(G, APL), 1) macm_step_kernel
     // first chunk of the contact list, fetched together with the state (one HBM round trip less)
     uint32_t pre_ab = 0u;
     float2 pre_imp = make_float2(0.0f, 0.0f);
-    // Bulk path (P.bulk, macm_sim.h): lane 0 issues six cp.async.bulk copies -- angle/sleep + actions on one
-    // mbarrier (all phase 1 needs), positions/velocities + fat AABBs + the head of the contact list on a second one
-    // that is only waited for after the float64 action decode -- into the still idle touching-contact stage (the
-    // fat AABBs land where they live).  Otherwise every lane loads its own agents' rows.
-#ifdef MACM_BULK_STAGE   // measured (profiles/README.md, r2 finding 3): no faster than per-lane loads; an experiment build
-    const bool bulk = !TDM && G == 32 && P.bulk && actions != nullptr && (reinterpret_cast<uintptr_t>(actions) & 15) == 0;
-#else
-    constexpr bool bulk = false;
-#endif
-    unsigned char* stg = S.base + Lay<NC>::FIXED;
-    const uint32_t bar = smem_u32(S.misc());
-    if (bulk) {
-        if (g.gl == 0) {
-            const size_t a0 = (size_t)env * N;
-            mbar_expect_tx(bar, N * 12);
-            bulk_g2s(smem_u32(stg + N * 16), P.angsleep + a0, N * 8, bar);
-            bulk_g2s(smem_u32(stg + N * 24), reinterpret_cast<const uint32_t*>(actions) + a0, N * 4, bar);
-            mbar_expect_tx(bar + 8, N * 32 + 384);
-            bulk_g2s(smem_u32(stg), P.posvel + a0, N * 16, bar + 8);
-            bulk_g2s(smem_u32(fat), P.fat + a0, N * 16, bar + 8);
-            bulk_g2s(smem_u32(stg + N * 28), c_ab, 128, bar + 8);
-            bulk_g2s(smem_u32(stg + N * 28 + 128), c_imp, 256, bar + 8);
-        }
-    } else if (g.gl < P.C) { pre_ab = c_ab[g.gl]; pre_imp = c_imp[g.gl]; }
+    if (g.gl < P.C) { pre_ab = c_ab[g.gl]; pre_imp = c_imp[g.gl]; }
     // TDM per-agent host state (combat.Agent): health, cool-downs (steps left), alive, hits taken
     float health[APL];
     int cd_atk[APL], cd_mov[APL], hits[APL];
@@ -1434,12 +1329,10 @@ __global__ void __launch_bounds__(shape_max_threads(G, APL), 1) macm_step_kernel
         valid[s] = i < N;
         team[s] = (TDM && valid[s]) ? P.team[i] : 0;
         const size_t gi = (size_t)env * N + (valid[s] ? i : 0);
-        if (!bulk) {
-            const float4 pv = P.posvel[gi];
-            const float2 as = P.angsleep[gi];
-            fatr[s] = P.fat[gi];
-            c[s] = make_float2(pv.x, pv.y); v[s] = make_float2(pv.z, pv.w); ang[s] = as.x; slp[s] = as.y;
-        }
+        const float4 pv = P.posvel[gi];
+        const float2 as = P.angsleep[gi];
+        fatr[s] = P.fat[gi];
+        c[s] = make_float2(pv.x, pv.y); v[s] = make_float2(pv.z, pv.w); ang[s] = as.x; slp[s] = as.y;
         was_alive[s] = valid[s];
         if (TDM) {
             const float4 td = P.tdm[gi];
@@ -1461,14 +1354,6 @@ __global__ void __launch_bounds__(shape_max_threads(G, APL), 1) macm_step_kernel
             reinterpret_cast<float2*>(S.nw())[i] = make_float2(o4.z, o4.w);
         }
     }
-    if (bulk) {   // angles, sleep timers and (below) the action words have landed
-        mbar_wait(bar, 0);
-#pragma unroll
-        for (int s = 0; s < APL; ++s) {
-            const float2 as = reinterpret_cast<const float2*>(stg + N * 16)[valid[s] ? g.gl + s * G : 0];
-            ang[s] = as.x; slp[s] = as.y;
-        }
-    }
     const bool discrete = TDM || P.action_mode == MACM_ACTION_DISCRETE;
     const size_t EN = (size_t)P.E * N;
     int tc = 0, nlev = 0;
@@ -1478,14 +1363,14 @@ __global__ void __launch_bounds__(shape_max_threads(G, APL), 1) macm_step_kernel
 #pragma unroll 1
     for (int ks = 0; ks < R.K(); ++ks) {
     const bool last = ks == R.K() - 1;
-    ASet alive = empty_set<ASet>();   // bodies that are active (have a proxy) during this step
+    ASet alive = {};   // bodies that are active (have a proxy) during this step
     // The block's warps start every R.sync()-th step together.  Measured (profiles/README.md, finding 8): the hot
     // path is ~48 KB of straight-line code; warps that drift apart each stream it from the GPC-level instruction
     // cache on their own, which saturates (gcc requests 83 % of peak, "no instruction" the top stall) -- in step
     // they share every fetched line.
     if (R.sync() > 0 && ks > 0 && (ks % R.sync()) == 0) __syncthreads();
     g.sync();   // the previous step's observation pass has finished reading the staging arrays
-    ASet alive0 = empty_set<ASet>();   // (combat actor) who is in the observation the actors decide on
+    ASet alive0 = {};   // (combat actor) who is in the observation the actors decide on
     if (ROLL && TDM && R.policy() == MACM_BOT_COMBAT) {
         if (ks == 0) {   // later steps: positions and angles are staged since the previous step's phases 7 and 11
 #pragma unroll
@@ -1512,8 +1397,7 @@ __global__ void __launch_bounds__(shape_max_threads(G, APL), 1) macm_step_kernel
         if (discrete && valid[s]) {
             if (!ROLL || actions) {
                 const uint32_t* aw = reinterpret_cast<const uint32_t*>(actions) + (size_t)ks * EN + gi;
-                if (bulk && ks == 0) act_raw[s] = reinterpret_cast<const uint32_t*>(stg + N * 24)[i];
-                else act_raw[s] = *aw;
+                act_raw[s] = *aw;
                 if (!last) asm volatile("prefetch.global.L2 [%0];" ::"l"(aw + EN));
             } else if (TDM && R.policy() == MACM_BOT_COMBAT) {
                 act_raw[s] = combat_action(pos, S.ang(), P.team, N, alive0, i);
@@ -1590,29 +1474,12 @@ __global__ void __launch_bounds__(shape_max_threads(G, APL), 1) macm_step_kernel
     // The bodies reach shared memory only now: phase 1 needs nothing but the angle and the action word, so the
     // rest of the state (positions, fat AABBs, contact list head, target) is still arriving from L2 while the
     // float64 action decode runs -- the whole batch loads its state at the same moment and the L2 is the queue.
-    if (bulk && ks == 0) {   // positions, velocities, fat AABBs and the head of the contact list have landed
-        mbar_wait(bar + 8, 0);
-#pragma unroll
-        for (int s = 0; s < APL; ++s) {
-            const int i = g.gl + s * G;
-            const float4 pv = reinterpret_cast<const float4*>(stg)[valid[s] ? i : 0];
-            c[s] = make_float2(pv.x, pv.y); v[s] = make_float2(pv.z, pv.w);
-            fatr[s] = fat[valid[s] ? i : 0];
-            if (!valid[s]) {  // padding agents: parked far away
-                c[s] = make_float2(3.0e30f, 3.0e30f); v[s] = make_float2(0.0f, 0.0f);
-                fatr[s] = make_float4(3.0e30f, 3.0e30f, 3.0e30f, 3.0e30f);
-            }
-        }
-        pre_ab = reinterpret_cast<const uint32_t*>(stg + N * 28)[g.gl];
-        pre_imp = reinterpret_cast<const float2*>(stg + N * 28 + 128)[g.gl];
-        g.sync();   // every lane has read its rows before a padding slot's fat AABB is overwritten below
-    }
 #pragma unroll
     for (int s = 0; s < APL; ++s) {
         const int i = g.gl + s * G;
         pos[i] = c[s];
         fat[i] = fatr[s];
-        adj[i] = empty_set<ASet>();
+        adj[i] = ASet{};
         S.tmask()[i] = 0u;
         if (!TDM && !ROLL) S.tgt()[i] = tg0[s];
     }
@@ -1879,13 +1746,12 @@ __global__ void __launch_bounds__(shape_max_threads(G, APL), 1) macm_step_kernel
             if (has && (__ffs((int)cset) - 1) == g.gl) {
                 oseed = seed;
                 uint8_t* nxt = S.stack();
-                uint32_t taken = 0u, vis_lo = 0u, vis_hi = 0u;
-                uint32_t vis_w2 = 0u, vis_w3 = 0u;   // (agents 64..127 of the wide shape)
+                uint32_t taken = 0u;
+                ASet vis = {};   // bodies pushed so far
                 int top = oseed, otail = EW_NONE;
                 uint32_t otail_ew = 0u;
                 nxt[oseed] = EW_NONE;
-                if (NC <= 64 || oseed < 64) { if (oseed < 32) vis_lo = 1u << oseed; else vis_hi = 1u << (oseed - 32); }
-                else if (oseed < 96) vis_w2 = 1u << (oseed - 64); else vis_w3 = 1u << (oseed - 96);
+                add_bit(vis, oseed);
                 while (top != EW_NONE) {
                     const int b = top;
                     top = nxt[b];
@@ -1897,12 +1763,8 @@ __global__ void __launch_bounds__(shape_max_threads(G, APL), 1) macm_step_kernel
                         if (otail == EW_NONE) ohead = t; else t_ew[otail] = otail_ew | ((uint32_t)t << EWT::SH_NA);
                         otail = t; otail_ew = ew;
                         const int other = (EWT::a(ew) == b) ? EWT::b(ew) : EWT::a(ew);
-                        const uint32_t ob = 1u << (other & 31);
-                        bool seen = ((other < 32 ? vis_lo : vis_hi) & ob) != 0u;
-                        if (NC > 64 && other >= 64) seen = ((other < 96 ? vis_w2 : vis_w3) & ob) != 0u;
-                        if (!seen) {
-                            if (NC <= 64 || other < 64) { if (other < 32) vis_lo |= ob; else vis_hi |= ob; }
-                            else if (other < 96) vis_w2 |= ob; else vis_w3 |= ob;
+                        if (!bit_of(vis, other)) {
+                            add_bit(vis, other);
                             nxt[other] = (uint8_t)top;
                             top = other;
                         }
@@ -2054,7 +1916,7 @@ __global__ void __launch_bounds__(shape_max_threads(G, APL), 1) macm_step_kernel
 
     PHASE_STAMP(8);
     // ---- phase 9: SynchronizeFixtures -> b2DynamicTree::MoveProxy -----------------------------------
-    ASet moved = empty_set<ASet>();
+    ASet moved = {};
 #pragma unroll
     for (int s = 0; s < APL; ++s) {
         const int i = g.gl + s * G;
@@ -2214,7 +2076,7 @@ __global__ void __launch_bounds__(shape_max_threads(G, APL), 1) macm_step_kernel
             for (int t = g.gl; t < P.T; t += G)
                 const_cast<float2*>(P.targets)[(size_t)env * P.T + t] = sample_target(R_.sc, (uint64_t)(env + P.env_base) * P.T + t, episode);
         if (TDM) {
-            alive = empty_set<ASet>();
+            alive = ASet{};
 #pragma unroll
             for (int s = 0; s < APL; ++s) { put_slot<G>(alive, s, g.ballot(valid[s])); was_alive[s] = valid[s]; }
         }
@@ -2359,7 +2221,7 @@ __global__ void __launch_bounds__(128) macm_observe_kernel(const __grid_constant
         g.sync();   // the group's stores (targets) are visible to its lanes below
     }
     float ang[APL];
-    typename SetOf<NC>::type alive = empty_set<typename SetOf<NC>::type>();
+    AgentSet<NC> alive = {};
 #pragma unroll
     for (int s = 0; s < APL; ++s) {
         const int i = g.gl + s * G;

@@ -54,9 +54,6 @@ struct SimConst {
     // blocks of the step kernel that are resident at once (SMs x blocks per SM): only those can overlap their L2
     // prefetch with the predecessor's tail; a block of a later wave starts when its loads can be issued anyway
     int first_wave;
-    // the env's state rows can travel to shared memory as 1-D bulk async copies (cp.async.bulk + mbarrier): one env
-    // per warp, Flock, discrete actions, N a multiple of 4, 16-byte aligned rows, room in the staging area
-    int bulk;
 };
 
 // Initial-state distributions (mvmnt.py:48-52,62-64; combat.py:84-86) and the key of the counter-based draws.
