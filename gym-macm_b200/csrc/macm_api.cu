@@ -200,6 +200,13 @@ static int derive_constants(macm_sim* sim)
     }
     int TCH = 0;             // beyond the shared-memory stage: a global-memory one of the requested capacity
     if (TC > 240) { TCH = (TC + 7) / 8 * 8; TC = 240; }  // (shared-memory stage: levels and list links are bytes)
+    // envs of 65..128 agents by default: a gathered flock (the bots.flock actor at the target) reaches up to ~1.8N
+    // touching contacts, more than the 192 of the shared stage from about 116 agents on, so a global-memory stage of
+    // 3N takes what the shared one cannot hold
+    if (p.max_touching <= 0 && p.n_agents > 64) {
+        const int h = C < 3 * p.n_agents ? C : 3 * p.n_agents;
+        if (h > TC) TCH = (h + 7) / 8 * 8;
+    }
     K.C = C; K.TC = TC; K.TCH = TCH;
     K.kind = p.env_kind; K.reward_mode = p.reward_mode; K.action_mode = p.action_mode; K.coord = p.coord;
     K.vel_iters = p.velocity_iterations; K.pos_iters = p.position_iterations;

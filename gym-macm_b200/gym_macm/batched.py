@@ -309,7 +309,8 @@ class _BatchedCommon(object):
         """bool [E]: the env ran out of contact capacity (`max_contacts`: newest pairs dropped; `max_touching`: the
         solver skipped the excess) at some step since its last reset -- from that step on its results differ from the
         reference's.  Sticky until the env is reset.  `max_touching` up to 240 is a shared-memory stage; a larger value
-        (up to `max_contacts`) adds a global-memory stage that takes the rare denser env exactly (spawn piles)."""
+        (up to `max_contacts`), and the default beyond 64 agents, add a global-memory stage that takes the denser env
+        exactly (gathered flocks, spawn piles)."""
         return (self.engine.t["env_state"][:, 1] & (_lib.ENV_CONTACT_OVERFLOW | _lib.ENV_TOUCH_OVERFLOW)) != 0
 
     def overflow_count(self):
@@ -321,7 +322,7 @@ class _BatchedCommon(object):
             c, t = self.engine.overflow_count()
             if c or t:
                 raise _lib.MacmError("contact capacity overflow: %d envs dropped contacts (max_contacts=%d), %d envs "
-                                     "exceeded the solver stage (max_touching=%d, limit 240); results of those envs "
+                                     "exceeded the solver stage (max_touching=%d); results of those envs "
                                      "differ from the reference's" % (c, self.engine.C, t, self.engine.sizes.max_touching))
 
     def _final(self):

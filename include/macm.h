@@ -86,10 +86,13 @@ typedef struct macm_params {
     int32_t n_agents;             /* sum(n_agents) of the ctor (mvmnt.py:61), 2..MACM_MAX_AGENTS */
     int32_t n_targets;            /* len(unique(targets)) (mvmnt.py:42), 1..MACM_MAX_TARGETS; TDM: 0 */
     int32_t max_contacts;         /* contact capacity per env; 0 = min(N(N-1)/2, 8N) */
-    int32_t max_touching;         /* touching-contact capacity per env; 0 = min(max_contacts, 2N), 192 beyond 64 agents.  Up to 240 the
-                                     solver's stage lives in shared memory; a larger value adds a global-memory stage
-                                     (macm_buffers.touch_scratch, 32 bytes per contact and env) that takes the rare env
-                                     with more touching contacts than that -- exact, slow, for dense spawn piles */
+    int32_t max_touching;         /* touching-contact capacity per env; 0 = min(max_contacts, 2N) up to 64 agents, and beyond 64 a
+                                     shared stage of min(2N, 192) with a global-memory one of min(max_contacts, 3N) behind
+                                     it (a flock gathered at its target reaches ~1.8N).  Up to 240 the solver's stage lives
+                                     in shared memory; a larger value adds a global-memory stage (macm_buffers.touch_scratch,
+                                     32 bytes per contact and env) that takes the env with more touching contacts than the
+                                     shared stage holds -- exact, slow, for gathered flocks and dense spawn piles.
+                                     macm_buffer_sizes.max_touching reports the effective capacity */
     double hz;                    /* settings.py:30   60.0 */
     int32_t velocity_iterations;  /* settings.py:31   8 */
     int32_t position_iterations;  /* settings.py:32   3 */
@@ -147,7 +150,7 @@ typedef struct macm_buffers {
     float* rewards;           /* [E,N] */
     uint8_t* collided;        /* [E,N] agent appears in some world contact (mvmnt.py:162-164) */
     uint8_t* done;            /* [E] */
-    /* ---- scratch (only when max_touching > 240 was asked for; see macm_buffer_sizes.touch_scratch) ---- */
+    /* ---- scratch (max_touching > 240, or the default beyond 64 agents; see macm_buffer_sizes.touch_scratch) ---- */
     uint8_t* touch_scratch;   /* the solver's stage of an env with more touching contacts than shared memory holds  16-byte aligned */
 } macm_buffers;
 

@@ -118,6 +118,8 @@ typedef struct {
     float radius, mass, inv_mass, friction, linear_damping;
     /* statistics of the last step */
     int last_touching, last_islands_multi;
+    int last_peak_contacts;   /* most contacts the world held at once during the last step (after the prologue's
+                                 FindNewContacts of a world with new fixtures, or at the end of the step) */
 } OWorld;
 
 static void ow_init(OWorld* w, int max_bodies, double radius, double density, double friction, double linear_damping,
@@ -616,6 +618,7 @@ static void ow_solve(OWorld* w, float h, float dt_ratio, int vel_iters, int pos_
 static void ow_step(OWorld* w, float dt, int vel_iters, int pos_iters)
 {
     if (w->new_fixture) { ow_find_new_contacts(w); w->new_fixture = 0; }
+    int peak = w->contact_count;
     float inv_dt = dt > 0.0f ? 1.0f / dt : 0.0f;
     float dt_ratio = w->inv_dt0 * dt;
     ow_collide(w);
@@ -625,6 +628,7 @@ static void ow_step(OWorld* w, float dt, int vel_iters, int pos_iters)
     if (dt > 0.0f) ow_solve(w, dt, dt_ratio, vel_iters, pos_iters);
     /* SolveTOI: every contact is skipped (two non-bullet dynamic bodies) */
     if (dt > 0.0f) w->inv_dt0 = inv_dt;
+    w->last_peak_contacts = peak > w->contact_count ? peak : w->contact_count;
     for (int i = 0; i < w->n; ++i) w->b[i].f = v2(0.0f, 0.0f);
 }
 
@@ -1126,11 +1130,11 @@ void oracle_get_tdm(const OBatch* B, double* st)
         }
 }
 
-void oracle_get_env_info(const OBatch* B, int ei, double* out /*[6]*/)
+void oracle_get_env_info(const OBatch* B, int ei, double* out /*[7]*/)
 {
     const OEnv* e = &B->e[ei];
     out[0] = e->time_passed; out[1] = e->done; out[2] = e->step_count; out[3] = e->w.inv_dt0;
-    out[4] = e->w.last_touching; out[5] = e->w.contact_count;
+    out[4] = e->w.last_touching; out[5] = e->w.contact_count; out[6] = e->w.last_peak_contacts;
 }
 
 /* ---- thin body-level API: lets tests drive ONE world the way pybox2d is driven, so that the

@@ -176,10 +176,12 @@ class OracleBatch:
         lib().oracle_set_targets(self._h, ei, _p(t))
 
     def env_info(self, ei):
-        out = np.zeros(6, np.float64)
+        """touching: touching contacts after the last step's Collide; contacts: contacts at its end; peak_contacts:
+        the most the world held at once during it (a fresh world's prologue can list pairs Collide then destroys)."""
+        out = np.zeros(7, np.float64)
         lib().oracle_get_env_info(self._h, ei, _p(out))
         return dict(time_passed=out[0], done=int(out[1]), step_count=int(out[2]), inv_dt0=np.float32(out[3]),
-                    touching=int(out[4]), contacts=int(out[5]))
+                    touching=int(out[4]), contacts=int(out[5]), peak_contacts=int(out[6]))
 
     def tdm_state(self):
         out = np.zeros((self.E, self.N, 4), np.float64)

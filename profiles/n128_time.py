@@ -1,6 +1,7 @@
 #!/usr/bin/env python
 """us per step of 128-agent flock envs (four agents per lane): 2048 envs x 128 agents = the headline's 262,144 agents.
-Arguments: N, E, and `tdm` for two-team deathmatch envs of N agents instead (random moves and attacks)."""
+Arguments: N, E, `tdm` for two-team deathmatch envs of N agents instead (random moves and attacks) or `flock`, and
+max_touching (default 0: the library default)."""
 import os
 import sys
 
@@ -13,14 +14,15 @@ dev = torch.device("cuda", 0)
 N = int(sys.argv[1]) if len(sys.argv) > 1 else 128
 E = int(sys.argv[2]) if len(sys.argv) > 2 else 2048
 TDM = len(sys.argv) > 3 and sys.argv[3] == "tdm"
+MT = int(sys.argv[4]) if len(sys.argv) > 4 else 0
 R, K = 8, 400
 g = torch.Generator(device=dev)
 g.manual_seed(9)
 if TDM:
-    sims = [gym_macm.BatchedTDM(E, n_agents=[N // 2, N - N // 2], device=dev, seed=70 + r) for r in range(R)]
+    sims = [gym_macm.BatchedTDM(E, n_agents=[N // 2, N - N // 2], device=dev, seed=70 + r, max_touching=MT) for r in range(R)]
 else:
     sims = [gym_macm.BatchedFlock(E, n_agents=[N], reward_mode="linear", device=dev, seed=70 + r,
-                                  start_spread=20.0 * (N / 64.0) ** 0.5) for r in range(R)]
+                                  start_spread=20.0 * (N / 64.0) ** 0.5, max_touching=MT) for r in range(R)]
 acts = torch.zeros((31, E, N, 4), dtype=torch.uint8, device=dev)
 acts[..., :3] = torch.randint(0, 3, (31, E, N, 3), generator=g, device=dev, dtype=torch.uint8)
 if TDM:
@@ -40,6 +42,6 @@ for rep in range(2):
     e1.record()
     torch.cuda.synchronize()
 info = sims[0].engine.info
-print("%s N=%d E=%d: %.2f us per step, %.3g agent-steps/s; %d threads x %d blocks, %d B smem; overflow %s" % (
-    "tdm" if TDM else "flock", N, E, 1e3 * e0.elapsed_time(e1) / K, E * N * K / (e0.elapsed_time(e1) * 1e-3),
+print("%s N=%d E=%d max_touching=%d: %.2f us per step, %.3g agent-steps/s; %d threads x %d blocks, %d B smem; overflow %s" % (
+    "tdm" if TDM else "flock", N, E, sims[0].engine.sizes.max_touching, 1e3 * e0.elapsed_time(e1) / K, E * N * K / (e0.elapsed_time(e1) * 1e-3),
     info.threads_per_block, info.blocks, info.smem_bytes_per_block, sims[0].overflow_count()))

@@ -33,32 +33,38 @@ def ang_diff(a, b):
     return np.minimum(d, 2 * np.pi - d)
 
 
-def compare_step(env, ref, o, k, coord="polar", reward_mode="binary", check_contacts_envs=None):
+def compare_step(env, ref, o, k, coord="polar", reward_mode="binary", check_contacts_envs=None, envs=None):
+    """Hold a BatchedFlock to the oracle after step k (o: that step's flock_step outputs).  envs: bool [E], the envs
+    held (None: all); the others, e.g. envs that ran out of contact capacity, are left out."""
     import torch
     torch.cuda.synchronize()
     E, N = ref.E, ref.N
+    m = np.ones(E, bool) if envs is None else np.asarray(envs, bool)
     st = env.state
-    assert not (st["env_state"][:, 1].cpu().numpy() & 6).any(), "step %d: contact capacity overflow" % k
-    gb, rb = gpu_bodies(env), ref.bodies()
+    assert not (st["env_state"][:, 1].cpu().numpy()[m] & 6).any(), "step %d: contact capacity overflow" % k
+    if not m.any():
+        return
+    gb, rb = gpu_bodies(env)[m], ref.bodies()[m]
     names = ["x", "y", "vx", "vy", "angle", "sleep", "fat_lx", "fat_ly", "fat_hx", "fat_hy"]
     for c, nm in enumerate(names):
         bad = np.argwhere(gb[..., c] != rb[..., c])
-        assert len(bad) == 0, "step %d: %s differs at %d agents, first (env,agent)=%s gpu=%r oracle=%r" % (
+        assert len(bad) == 0, "step %d: %s differs at %d agents, first (held env,agent)=%s gpu=%r oracle=%r" % (
             k, nm, len(bad), bad[0], gb[tuple(bad[0])][c], rb[tuple(bad[0])][c])
     st = env.state
-    assert np.array_equal(st["collided"].cpu().numpy(), o["collided"]), "step %d: collision flags" % k
-    assert np.array_equal(st["nn_idx"].cpu().numpy(), o["nn_idx"]), "step %d: nearest-agent ids" % k
-    assert np.array_equal(st["done"].cpu().numpy(), o["done"]), "step %d: done" % k
-    rew = st["rewards"].cpu().numpy().astype(np.float64)
+    assert np.array_equal(st["collided"].cpu().numpy()[m], o["collided"][m]), "step %d: collision flags" % k
+    assert np.array_equal(st["nn_idx"].cpu().numpy()[m], o["nn_idx"][m]), "step %d: nearest-agent ids" % k
+    assert np.array_equal(st["done"].cpu().numpy()[m], o["done"][m]), "step %d: done" % k
+    rew, orew = st["rewards"].cpu().numpy().astype(np.float64)[m], o["rewards"][m]
     if reward_mode == "binary":
-        assert np.array_equal(rew, o["rewards"]), "step %d: binary rewards" % k
+        assert np.array_equal(rew, orew), "step %d: binary rewards" % k
     else:
-        assert np.array_equal(rew == -1, o["rewards"] == -1)
-        assert np.allclose(rew, o["rewards"], rtol=0, atol=LIN_REWARD_ATOL), "step %d: linear rewards" % k
+        assert np.array_equal(rew == -1, orew == -1)
+        assert np.allclose(rew, orew, rtol=0, atol=LIN_REWARD_ATOL), "step %d: linear rewards" % k
     # contact lists: same pairs in the same (birth) order, same touching flags, same impulses
     cnt = st["contact_count"].cpu().numpy()
-    envs = range(E) if check_contacts_envs is None else check_contacts_envs
-    for e in envs:
+    for e in range(E) if check_contacts_envs is None else check_contacts_envs:
+        if not m[e]:
+            continue
         ab, fl, imp = env.contacts(e)
         rab, rfl, rimp = ref.contacts(e)
         assert cnt[e] == len(rab), "step %d env %d: %d contacts vs oracle %d" % (k, e, cnt[e], len(rab))
@@ -66,7 +72,35 @@ def compare_step(env, ref, o, k, coord="polar", reward_mode="binary", check_cont
         assert np.array_equal(fl, rfl), "step %d env %d: touching flags" % (k, e)
         t = rfl.astype(bool)
         assert np.array_equal(imp[t], rimp[t]), "step %d env %d: warm-start impulses" % (k, e)
-    compare_obs(st["obs"].cpu().numpy(), o, coord, k)
+    compare_obs(st["obs"].cpu().numpy()[m], {n: o[n][m] for n in ("nn_pos", "tg_pos")}, coord, k)
+
+
+def overflow_bits(env, ref, prev, ever, k):
+    """Overflow bits of every env after step k against the oracle's counts.  ever: int [E], updated in place with the
+    bits the oracle's envs have earned so far (2: peak live contacts above max_contacts, 4: touching contacts at Collide
+    above the effective max_touching); prev: the device's bits after step k - 1.  An env unflagged before the step must
+    carry exactly the oracle's bits, a set bit stays set, a flagged env still lists at most max_contacts pairs a < b < N.
+    (On a fresh world's first step the pairs dropped by the prologue's FindNewContacts are missing at Collide already:
+    an env whose contact bit is set there may miss the touching bit the oracle earns in the same step.)
+    Returns the device's bits."""
+    import torch
+    C, T, N = env.engine.sizes.max_contacts, env.engine.sizes.max_touching, ref.N
+    for e in range(ref.E):
+        i = ref.env_info(e)
+        ever[e] |= (2 if i["peak_contacts"] > C else 0) | (4 if i["touching"] > T else 0)
+    torch.cuda.synchronize()
+    bits = env.state["env_state"][:, 1].cpu().numpy() & 6
+    fresh = prev == 0
+    assert np.array_equal(bits[fresh] & 2, ever[fresh] & 2), "step %d: contact-overflow bits" % k
+    first = env.state["env_state"][:, 0].cpu().numpy() == 1
+    t = fresh & ~(first & (bits & 2 != 0))
+    assert np.array_equal(bits[t] & 4, ever[t] & 4), "step %d: touch-overflow bits" % k
+    assert ((bits & prev) == prev).all(), "step %d: an overflow bit was cleared" % k
+    assert (env.state["contact_count"].cpu().numpy() <= C).all(), "step %d: more than max_contacts listed" % k
+    for e in np.flatnonzero(bits):
+        ab = env.contacts(e)[0]
+        assert ((ab[:, 0] < ab[:, 1]) & (ab[:, 1] < N)).all(), "step %d env %d: pair out of range" % (k, e)
+    return bits
 
 
 def compare_obs(obs, o, coord, k=0):

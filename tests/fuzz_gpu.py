@@ -18,7 +18,7 @@ for p in (ROOT, os.path.join(ROOT, "gym-macm_b200"), os.path.join(ROOT, "tests")
     if p not in sys.path:
         sys.path.insert(0, p)
 
-from _parity import run_parity  # noqa: E402
+from _parity import compare_step, make_pair, overflow_bits, run_parity  # noqa: E402
 from test_gpu_tdm import run_tdm  # noqa: E402
 
 
@@ -55,6 +55,31 @@ def capacity(rng, N):
     return int(rng.choice([0, 240, N * (N - 1) // 2]))
 
 
+def capped_case(rng, N, E, steps, spread, kw):
+    """Capacities below full: every step, the overflow bits against the oracle's counts and every unflagged env held to
+    the oracle (_parity.overflow_bits, compare_step's env mask).  Returns the number of envs flagged at the end."""
+    import torch
+    pairs = N * (N - 1) // 2
+    C = int(rng.integers(max(1, pairs // 8), pairs + 1))
+    mt = int(rng.choice([0, 16 * int(rng.integers(1, 16))]))
+    env, ref, r2 = make_pair(E, N, None, int(rng.integers(0, 1 << 30)), spread, max_contacts=C, max_touching=mt, **kw)
+    coord, rmode = kw.get("coord", "polar"), kw.get("reward_mode", "binary")
+    cont = kw.get("action_mode", "discrete") == "continuous"
+    ever, bits = np.zeros(E, int), np.zeros(E, int)
+    for k in range(steps):
+        if cont:
+            act = r2.uniform(-1.2, 1.2, (E, N, 2)).astype(np.float32).astype(np.float64)
+            env.step(torch.as_tensor(act, dtype=torch.float32, device="cuda:0"))
+        else:
+            act = r2.integers(0, 3, (E, N, 3))
+            env.step(torch.as_tensor(act, device="cuda:0"))
+        o = ref.flock_step(act)
+        bits = overflow_bits(env, ref, bits, ever, k)
+        compare_step(env, ref, o, k, coord, rmode, envs=bits == 0)
+    env.close()
+    return int((bits != 0).sum()), dict(max_contacts=C, max_touching=mt)
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--seconds", type=float, default=180.0)
@@ -63,7 +88,7 @@ def main():
     args = ap.parse_args()
     rng = np.random.default_rng(args.seed)
     t0, cases, agent_steps, worst_tc, skipped = time.time(), 0, 0, 0, 0
-    tdm_cases, deaths = 0, 0
+    tdm_cases, deaths, capped, flagged = 0, 0, 0, 0
     # per build: the default kernels, or those of macm_kernels_huge.cu (max_touching above 240)
     by_build = {"default": {"flock": 0, "tdm": 0}, "huge": {"flock": 0, "tdm": 0}}
     while time.time() - t0 < args.seconds:
@@ -109,6 +134,17 @@ def main():
         policy = "random"
         if kw["action_mode"] == "discrete" and kw["coord"] == "polar" and rng.random() < 0.25:
             policy = str(rng.choice(["flock", "idle"]))
+        if rng.random() < 0.25:   # capacities below full: the overflow flags and the isolation of the other envs
+            desc = dict(N=N, E=E, spread=round(spread, 2), steps=steps, capped=True, **kw)
+            try:
+                f, caps = capped_case(rng, N, E, steps, spread, kw)
+            except AssertionError as ex:
+                print("MISMATCH", json.dumps(desc), str(ex)[:300], flush=True)
+                sys.exit(1)
+            capped += 1
+            flagged += f
+            agent_steps += E * N * steps
+            continue
         mt = capacity(rng, N)
         desc = dict(N=N, E=E, spread=round(spread, 2), steps=steps, policy=policy, targets=targets, max_touching=mt, **kw)
         try:
@@ -131,6 +167,7 @@ def main():
         agent_steps += E * N * steps
         worst_tc = max(worst_tc, st["max_touching"])
     print(json.dumps({"cases": cases, "tdm_cases": tdm_cases, "tdm_deaths_at_case_end": deaths, "agent_steps_checked": agent_steps, "max_touching_seen": worst_tc, "overflow_reported_by_device": skipped,
+                      "capped_cases": capped, "capped_envs_flagged": flagged,
                       "cases_by_build": by_build,
                       "seconds": round(time.time() - t0, 1), "seed": args.seed}))
 

@@ -52,18 +52,20 @@ def run_tdm(E, teams, steps, seed, width=30.0, height=30.0, attack_p=0.5, check_
     return deaths
 
 
-def compare_tdm_step(env, ref, o, k, contact_envs=8):
+def compare_tdm_step(env, ref, o, k, contact_envs=8, envs=None):
     """Hold a BatchedTDM to the oracle after step k (o: that step's tdm_step outputs); returns the oracle's alive
-    mask [E,N].  Contact lists are compared for the first `contact_envs` envs (None: all)."""
+    mask [E,N].  Contact lists are compared for the first `contact_envs` envs (None: all).  envs: bool [E], the envs
+    held (None: all); the others, e.g. envs that ran out of contact capacity, are left out."""
     import torch
     E, N = ref.E, ref.N
+    m = np.ones(E, bool) if envs is None else np.asarray(envs, bool)
     torch.cuda.synchronize()
     st = env.state
-    assert not (st["env_state"][:, 1].cpu().numpy() & 6).any(), "overflow"
-    gb, rb = gpu_bodies(env), ref.bodies()
-    assert np.array_equal(gb, rb), "step %d: body state differs at %s" % (k, np.argwhere(gb != rb)[:3])
-    ts = ref.tdm_state()
-    tg = st["tdm_state"].cpu()
+    assert not (st["env_state"][:, 1].cpu().numpy()[m] & 6).any(), "overflow"
+    gb, rb = gpu_bodies(env)[m], ref.bodies()[m]
+    assert np.array_equal(gb, rb), "step %d: body state differs at (held env, agent, field) %s" % (k, np.argwhere(gb != rb)[:3])
+    ts = ref.tdm_state()[m]
+    tg = st["tdm_state"].cpu()[torch.as_tensor(m)]
     ti = tg.view(torch.int32).numpy()
     assert np.array_equal(tg[..., 0].numpy().astype(np.float64), ts[..., 0]), "step %d: health" % k
     assert np.array_equal((ti[..., 3] & 1), ts[..., 3].astype(np.int32)), "step %d: alive" % k
@@ -72,22 +74,25 @@ def compare_tdm_step(env, ref, o, k, contact_envs=8):
     alive = ts[..., 3] > 0
     assert np.array_equal(ti[..., 1][alive], want_atk[alive]), "step %d: attack cool-down" % k
     assert np.array_equal(ti[..., 2][alive], want_mov[alive]), "step %d: movement cool-down" % k
-    assert np.array_equal(st["collided"].cpu().numpy(), o["collided"]), "step %d: collision flags" % k
-    assert np.array_equal(st["rewards"].cpu().numpy().astype(np.float64), o["rewards"]), "step %d: rewards" % k
-    assert np.array_equal(st["done"].cpu().numpy(), o["done"]), "step %d: done" % k
-    assert np.array_equal(st["env_state"][:, 3].cpu().numpy(), o["winner"]), "step %d: winner" % k
-    obs = st["obs"].cpu().numpy().reshape(E, N, N, 4)
-    assert np.array_equal(obs[..., 3].astype(np.int8), o["type"]), "step %d: ally/enemy/none flags" % k
-    m = o["type"] >= 0
-    assert np.allclose(obs[..., 0][m], o["obs"][..., 0][m], rtol=OBS_RTOL, atol=OBS_ATOL)
-    assert ang_diff(obs[..., 1][m].astype(np.float64), o["obs"][..., 1][m]).max() <= 3e-6
-    assert ang_diff(obs[..., 2][m].astype(np.float64), o["obs"][..., 2][m]).max() <= 3e-6
+    assert np.array_equal(st["collided"].cpu().numpy()[m], o["collided"][m]), "step %d: collision flags" % k
+    assert np.array_equal(st["rewards"].cpu().numpy().astype(np.float64)[m], o["rewards"][m]), "step %d: rewards" % k
+    assert np.array_equal(st["done"].cpu().numpy()[m], o["done"][m]), "step %d: done" % k
+    assert np.array_equal(st["env_state"][:, 3].cpu().numpy()[m], o["winner"][m]), "step %d: winner" % k
+    obs = st["obs"].cpu().numpy().reshape(E, N, N, 4)[m]
+    assert np.array_equal(obs[..., 3].astype(np.int8), o["type"][m]), "step %d: ally/enemy/none flags" % k
+    t = o["type"][m] >= 0
+    oo = o["obs"][m]
+    assert np.allclose(obs[..., 0][t], oo[..., 0][t], rtol=OBS_RTOL, atol=OBS_ATOL)
+    assert ang_diff(obs[..., 1][t].astype(np.float64), oo[..., 1][t]).max(initial=0) <= 3e-6
+    assert ang_diff(obs[..., 2][t].astype(np.float64), oo[..., 2][t]).max(initial=0) <= 3e-6
     for e in range(E if contact_envs is None else min(E, contact_envs)):
+        if not m[e]:
+            continue
         ab, fl, imp = env.contacts(e)
         rab, rfl, rimp = ref.contacts(e)
         assert np.array_equal(ab, rab) and np.array_equal(fl, rfl), "step %d env %d: contacts" % (k, e)
         assert np.array_equal(imp[rfl.astype(bool)], rimp[rfl.astype(bool)])
-    return alive
+    return ref.tdm_state()[..., 3] > 0
 
 
 def test_tdm_duel_small():
