@@ -212,6 +212,8 @@ static int derive_constants(macm_sim* sim)
     K.vel_iters = p.velocity_iterations; K.pos_iters = p.position_iterations;
     K.warm_starting = p.warm_starting; K.flags = p.flags;
     K.obs_dim = p.env_kind == MACM_ENV_TDM ? 4 * p.n_agents : (p.coord == MACM_COORD_POLAR ? 4 : 6);
+    K.obs_dtype = p.obs_dtype;
+    K.obs_words = p.obs_dtype == MACM_OBS_F32 ? K.obs_dim : K.obs_dim / 2;   // obs_dim is even
 
     // cm_framework.py:182,222: timeStep = 1.0/hz is a Python float, rounded to float32 by SWIG
     K.h = (float)(1.0 / p.hz);
@@ -279,6 +281,7 @@ extern "C" int macm_create(macm_sim** out, const macm_params* p, int device)
     if (p->reward_mode < 0 || p->reward_mode > 1 || p->action_mode < 0 || p->action_mode > 1 || p->coord < 0 ||
         p->coord > 1 || p->damping_model < 0 || p->damping_model > 1)
         return MACM_E_INVALID;
+    if (p->obs_dtype != MACM_OBS_F32 && p->obs_dtype != MACM_OBS_F16 && p->obs_dtype != MACM_OBS_BF16) return MACM_E_INVALID;
 
     macm_sim* sim = new (std::nothrow) macm_sim;
     if (!sim) return MACM_E_NOMEM;
@@ -347,7 +350,7 @@ extern "C" int macm_get_buffer_sizes(const macm_sim* sim, macm_buffer_sizes* o)
     o->contact_count = (uint64_t)K.E * 4; o->env_state = (uint64_t)K.E * 16;
     o->targets = (uint64_t)K.E * K.T * 8; o->target_idx = K.kind == MACM_ENV_FLOCK ? (uint64_t)K.N : 0;
     o->tdm_state = K.kind == MACM_ENV_TDM ? EN * 16 : 0; o->team = K.kind == MACM_ENV_TDM ? (uint64_t)K.N : 0;
-    o->obs = EN * 4 * (uint64_t)K.obs_dim; o->nn_idx = K.kind == MACM_ENV_FLOCK ? EN * 4 : 0;
+    o->obs = EN * 4 * (uint64_t)K.obs_words; o->nn_idx = K.kind == MACM_ENV_FLOCK ? EN * 4 : 0;
     o->rewards = EN * 4; o->collided = EN; o->done = (uint64_t)K.E;
     o->touch_scratch = (uint64_t)K.E * K.TCH * 32;
     o->obs_dim = K.obs_dim;
@@ -369,6 +372,14 @@ extern "C" int macm_get_launch_info(const macm_sim* sim, macm_launch_info* o)
 
 static bool aligned(const void* p, size_t a) { return ((uintptr_t)p % a) == 0; }
 
+// alignment of an observation array: the vector width of its record stores -- float4 in fp32, one 8-byte record of
+// four 16-bit values (Flock polar, TDM), or three 32-bit words (Flock cartesian, 12-byte records)
+static size_t obs_align(const SimConst& K)
+{
+    if (K.obs_dtype == MACM_OBS_F32) return 16;
+    return (K.kind == MACM_ENV_FLOCK && K.coord == MACM_COORD_CARTESIAN) ? 4 : 8;
+}
+
 extern "C" int macm_bind(macm_sim* sim, const macm_buffers* b)
 {
     if (!sim || !b) return MACM_E_INVALID;
@@ -380,7 +391,7 @@ extern "C" int macm_bind(macm_sim* sim, const macm_buffers* b)
     if (flock && (!b->targets || !b->target_idx || !b->nn_idx)) return MACM_E_UNBOUND;
     if (!flock && (!b->tdm_state || !b->team)) return MACM_E_UNBOUND;
     if (!aligned(b->posvel, 16) || !aligned(b->fat, 16) || !aligned(b->angsleep, 8) || !aligned(b->contact_imp, 8) ||
-        !aligned(b->contact_ab, 4) || !aligned(b->env_state, 16) || !aligned(b->obs, 16) || !aligned(b->rewards, 4) ||
+        !aligned(b->contact_ab, 4) || !aligned(b->env_state, 16) || !aligned(b->obs, obs_align(K)) || !aligned(b->rewards, 4) ||
         (b->targets && !aligned(b->targets, 8)) || (b->tdm_state && !aligned(b->tdm_state, 16)) ||
         (b->nn_idx && !aligned(b->nn_idx, 4)))
         return MACM_E_ALIGN;
@@ -401,7 +412,7 @@ static int check_final(const macm_sim* sim, const float* obs, const int32_t* nn_
 {
     const bool flock = sim->K.kind == MACM_ENV_FLOCK;
     if ((nn_idx && !flock) || (tdm_state && flock)) return MACM_E_INVALID;
-    if ((obs && !aligned(obs, 16)) || (nn_idx && !aligned(nn_idx, 4)) || (tdm_state && !aligned(tdm_state, 16)) ||
+    if ((obs && !aligned(obs, obs_align(sim->K))) || (nn_idx && !aligned(nn_idx, 4)) || (tdm_state && !aligned(tdm_state, 16)) ||
         (env_state && !aligned(env_state, 16)))
         return MACM_E_ALIGN;
     return MACM_OK;
@@ -525,11 +536,13 @@ extern "C" int macm_rollout(macm_sim* sim, const void* actions, int32_t n_steps,
         if (!discrete) return MACM_E_UNSUPPORTED;
         if (policy == MACM_BOT_FLOCK && (sim->K.kind != MACM_ENV_FLOCK || sim->params.coord != MACM_COORD_POLAR))
             return MACM_E_UNSUPPORTED;
+        // the flock actor's first step reads the stored observation: a rounded one would change its decisions
+        if (policy == MACM_BOT_FLOCK && sim->K.obs_dtype != MACM_OBS_F32) return MACM_E_UNSUPPORTED;
         if (policy == MACM_BOT_COMBAT && sim->K.kind != MACM_ENV_TDM) return MACM_E_UNSUPPORTED;
         R.policy = policy;
     }
     if (out) {
-        if ((out->obs && !aligned(out->obs, 16)) || (out->rewards && !aligned(out->rewards, 4)) ||
+        if ((out->obs && !aligned(out->obs, obs_align(sim->K))) || (out->rewards && !aligned(out->rewards, 4)) ||
             (out->nn_idx && !aligned(out->nn_idx, 4)))
             return MACM_E_ALIGN;
         R.obs = out->obs; R.nn_idx = out->nn_idx; R.rewards = out->rewards; R.collided = out->collided; R.done = out->done;
@@ -543,7 +556,7 @@ extern "C" int macm_rollout(macm_sim* sim, const void* actions, int32_t n_steps,
     // the launch's last step: the appended reset copies its terminal rows to row n_steps - 1 of the final_* arrays
     const SimConst& K = sim->K;
     const size_t last = (size_t)(n_steps - 1) * K.E, EN = last * K.N;
-    const Finals row = {R.fin_k.obs ? R.fin_k.obs + EN * K.obs_dim : nullptr, R.fin_k.nn_idx ? R.fin_k.nn_idx + EN : nullptr,
+    const Finals row = {R.fin_k.obs ? R.fin_k.obs + EN * K.obs_words : nullptr, R.fin_k.nn_idx ? R.fin_k.nn_idx + EN : nullptr,
                         R.fin_k.tdm ? R.fin_k.tdm + EN : nullptr, R.fin_k.es ? R.fin_k.es + last : nullptr};
     GUARD();
     if (int rc = order_after_host(sim, (cudaStream_t)stream)) return rc;
@@ -573,6 +586,9 @@ extern "C" int macm_bot_actions(macm_sim* sim, int policy, uint64_t seed, void* 
     if (sim->params.action_mode != MACM_ACTION_DISCRETE) return MACM_E_UNSUPPORTED;
     if (policy == MACM_BOT_COMBAT && sim->K.kind != MACM_ENV_TDM) return MACM_E_UNSUPPORTED;
     if (policy == MACM_BOT_FLOCK && sim->K.kind != MACM_ENV_FLOCK) return MACM_E_UNSUPPORTED;
+    // these two actors decide from the stored observation: a rounded one would change their decisions
+    if ((policy == MACM_BOT_FLOCK || policy == MACM_BOT_COMBAT) && sim->K.obs_dtype != MACM_OBS_F32)
+        return MACM_E_UNSUPPORTED;
     GUARD();
     if (int rc = order_after_host(sim, (cudaStream_t)stream)) return rc;
     CU(macm_launch_bot(sim->K, policy, seed, actions_out, (cudaStream_t)stream));

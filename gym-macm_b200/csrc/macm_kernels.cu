@@ -281,6 +281,24 @@ __device__ __forceinline__ void b2normalize(float& x, float& y)
 // Engine state never goes through it (b2normalize, the translation clamp and the ray cast keep IEEE sqrtf).
 __device__ __forceinline__ float out_sqrtf(float x) { float r; asm("sqrt.approx.f32 %0, %1;" : "=f"(r) : "f"(x)); return r; }
 
+// Two fp32 observation values -> one word of two 16-bit ones (MACM_OBS_F16 / MACM_OBS_BF16), `lo` at the lower
+// address; rounded to nearest even, with subnormals kept (no .ftz), as torch's .to(float16 / bfloat16) rounds.
+// The PTX form puts its FIRST source in the upper half.
+__device__ __forceinline__ uint32_t obs_pack2(float lo, float hi, bool bf16)
+{
+    uint32_t r;
+    if (bf16) asm("cvt.rn.bf16x2.f32 %0, %1, %2;" : "=r"(r) : "f"(hi), "f"(lo));
+    else asm("cvt.rn.f16x2.f32 %0, %1, %2;" : "=r"(r) : "f"(hi), "f"(lo));
+    return r;
+}
+// one 4-value observation record at the element type of `Rec`: float4 (fp32) or uint2 (four 16-bit values)
+template <typename Rec> __device__ __forceinline__ Rec obs_record(float4 v, bool bf16);
+template <> __device__ __forceinline__ float4 obs_record<float4>(float4 v, bool) { return v; }
+template <> __device__ __forceinline__ uint2 obs_record<uint2>(float4 v, bool bf16)
+{
+    return make_uint2(obs_pack2(v.x, v.y, bf16), obs_pack2(v.z, v.w, bf16));
+}
+
 // t - sign(t)*2*pi if |t| > pi else t (mvmnt.py:199), in fp32 for the observation outputs
 __device__ __forceinline__ float wrap_pi_f(float t)
 {
@@ -695,16 +713,26 @@ __device__ __forceinline__ void nn_search_128(const Grp<G>& g, const EnvS<4 * G>
 // ------------------------------------------------------------------------------------------
 // observation pass for the agents a lane owns (Flock.get_obs, mvmnt.py:181-222)
 // ------------------------------------------------------------------------------------------
-// cartesian variant of the observation record (coord == "cartesian", mvmnt.py:202-203,215-216); cold
-__device__ __noinline__ void store_cartesian(float* obs, size_t gi, float nn_d, float nn_t, float tg_r, float tg_t)
+// cartesian variant of the observation record (coord == "cartesian", mvmnt.py:202-203,215-216); cold.
+// 24 bytes per agent in fp32, 12 (three words) at a 16-bit obs_dtype.
+__device__ __noinline__ void store_cartesian(float* obs, size_t gi, float nn_d, float nn_t, float tg_r, float tg_t,
+                                             int dtype)
 {
     float sn, cn, st, ct;
     sincosf(nn_t, &sn, &cn);
     sincosf(tg_t, &st, &ct);
-    float2* ob = reinterpret_cast<float2*>(obs) + gi * 3;
-    ob[0] = make_float2(nn_d, cn);
-    ob[1] = make_float2(sn, tg_r);
-    ob[2] = make_float2(ct, st);
+    if (dtype == MACM_OBS_F32) {
+        float2* ob = reinterpret_cast<float2*>(obs) + gi * 3;
+        ob[0] = make_float2(nn_d, cn);
+        ob[1] = make_float2(sn, tg_r);
+        ob[2] = make_float2(ct, st);
+    } else {
+        const bool bf16 = dtype == MACM_OBS_BF16;
+        uint32_t* ob = reinterpret_cast<uint32_t*>(obs) + gi * 3;
+        ob[0] = obs_pack2(nn_d, cn, bf16);
+        ob[1] = obs_pack2(sn, tg_r, bf16);
+        ob[2] = obs_pack2(ct, st, bf16);
+    }
 }
 
 // Destinations: (ob1, nn1) and (ob2, nn2), each pointer may be null (a rollout writes a step's observation to
@@ -771,18 +799,53 @@ __device__ void flock_observe(const Grp<G>& g, const EnvS<G * APL>& S, const Sim
         if (nn2) nn2[gi] = bi[s];
         if (P.coord == MACM_COORD_POLAR) {
             const float4 o4 = make_float4(nn_d, nn_t, tg_r, tg_t);
-            if (ob1) reinterpret_cast<float4*>(ob1)[gi] = o4;
-            if (ob2) reinterpret_cast<float4*>(ob2)[gi] = o4;
+            if (P.obs_dtype == MACM_OBS_F32) {
+                if (ob1) reinterpret_cast<float4*>(ob1)[gi] = o4;
+                if (ob2) reinterpret_cast<float4*>(ob2)[gi] = o4;
+            } else {
+                const uint2 w = obs_record<uint2>(o4, P.obs_dtype == MACM_OBS_BF16);
+                if (ob1) reinterpret_cast<uint2*>(ob1)[gi] = w;
+                if (ob2) reinterpret_cast<uint2*>(ob2)[gi] = w;
+            }
         } else {
-            if (ob1) store_cartesian(ob1, gi, nn_d, nn_t, tg_r, tg_t);
-            if (ob2) store_cartesian(ob2, gi, nn_d, nn_t, tg_r, tg_t);
+            if (ob1) store_cartesian(ob1, gi, nn_d, nn_t, tg_r, tg_t, P.obs_dtype);
+            if (ob2) store_cartesian(ob2, gi, nn_d, nn_t, tg_r, tg_t, P.obs_dtype);
         }
+    }
+}
+
+// The N x N records of one env, walked in MEMORY order, G at a time (record r = i * N + j -> lane r % G): every store
+// of the group is one contiguous run of records whatever N is, and no lane idles on a ragged row end (N = 45 on 32
+// lanes: 64 rounds instead of 90).  i and j advance without a division.  Rec is the record as stored: float4, or
+// uint2 for four 16-bit values -- chosen once per call, so that the fp32 loop carries no conversion.
+template <int G, typename Rec>
+__device__ __forceinline__ void tdm_rows(const Grp<G>& g, const float4* hdr, int N, Rec* out, Rec* out2, bool bf16)
+{
+    const int total = N * N;
+    int i = g.gl / N, j = g.gl - i * N;          // G may exceed N (small teams on a wide group)
+    const int di = G / N, dj = G - di * N;       // one round further: G records
+#pragma unroll 1
+    for (int r = g.gl; r < total; r += G) {
+        const float4 h = hdr[i];   // observer: x, y, heading, team (-1: dead, observes nothing)
+        const float4 q = hdr[j];   // observed
+        const float dx = q.x - h.x, dy = q.y - h.y;
+        const bool entry = h.w >= 0.0f && q.w >= 0.0f && j != i;
+        float4 v;
+        v.x = entry ? out_sqrtf(dx * dx + dy * dy) : 0.0f;
+        v.y = entry ? wrap_pi_f(fast_atan2f(dy, dx) - h.z) : 0.0f;
+        v.z = entry ? wrap_pi_f(q.z - h.z) : 0.0f;
+        v.w = entry ? ((q.w == h.w) ? 1.0f : 0.0f) : -1.0f;
+        const Rec rec = obs_record<Rec>(v, bf16);
+        if (out) out[r] = rec;
+        if (out2) out2[r] = rec;
+        j += dj; i += di;
+        if (j >= N) { j -= N; ++i; }
     }
 }
 
 // TDM.get_obs (combat.py:206-227): for every alive agent i, every other alive agent j:
 // [r, theta, phi] and the ally flag.  Row i of the [N,N,4] output is written by the whole group
-// (lane <-> j) so that the 16-byte stores of a row are contiguous.
+// (lane <-> j) so that the record stores of a row are contiguous.
 // The pass is the bulk of a TDM step (N^2 records of 16 bytes: 70 % of its instructions), so the row loop is kept
 // lean: one 16-byte header per agent (x, y, heading, team -- or -1 when it has no entry) staged where the fat AABBs
 // lived (dead by now, as in nn_search_64), one broadcast load per row, no branch inside the row (a record without
@@ -803,29 +866,13 @@ __device__ void tdm_observe(const Grp<G>& g, const EnvS<G * APL>& S, const SimCo
         hdr[j] = make_float4(q.x, q.y, angs[j], (j < N && bit_of(alive, j)) ? (float)P.team[j] : -1.0f);
     }
     g.sync();
-    // The N x N records are walked in MEMORY order, G at a time (record r = i * N + j -> lane r % G): every store of
-    // the group is one contiguous run of 16-byte records whatever N is, and no lane idles on a ragged row end
-    // (N = 45 on 32 lanes: 64 rounds instead of 90).  i and j advance without a division.
-    const int total = N * N;
-    float4* out = ob1 ? reinterpret_cast<float4*>(ob1) + (size_t)env * total : nullptr;
-    float4* out2 = ob2 ? reinterpret_cast<float4*>(ob2) + (size_t)env * total : nullptr;
-    int i = g.gl / N, j = g.gl - i * N;          // G may exceed N (small teams on a wide group)
-    const int di = G / N, dj = G - di * N;       // one round further: G records
-#pragma unroll 1
-    for (int r = g.gl; r < total; r += G) {
-        const float4 h = hdr[i];   // observer: x, y, heading, team (-1: dead, observes nothing)
-        const float4 q = hdr[j];   // observed
-        const float dx = q.x - h.x, dy = q.y - h.y;
-        const bool entry = h.w >= 0.0f && q.w >= 0.0f && j != i;
-        float4 v;
-        v.x = entry ? out_sqrtf(dx * dx + dy * dy) : 0.0f;
-        v.y = entry ? wrap_pi_f(fast_atan2f(dy, dx) - h.z) : 0.0f;
-        v.z = entry ? wrap_pi_f(q.z - h.z) : 0.0f;
-        v.w = entry ? ((q.w == h.w) ? 1.0f : 0.0f) : -1.0f;
-        if (out) out[r] = v;
-        if (out2) out2[r] = v;
-        j += dj; i += di;
-        if (j >= N) { j -= N; ++i; }
+    const size_t first = (size_t)env * N * N;   // the env's first record
+    if (P.obs_dtype == MACM_OBS_F32) {
+        tdm_rows<G>(g, hdr, N, ob1 ? reinterpret_cast<float4*>(ob1) + first : nullptr,
+                    ob2 ? reinterpret_cast<float4*>(ob2) + first : nullptr, false);
+    } else {
+        tdm_rows<G>(g, hdr, N, ob1 ? reinterpret_cast<uint2*>(ob1) + first : nullptr,
+                    ob2 ? reinterpret_cast<uint2*>(ob2) + first : nullptr, P.obs_dtype == MACM_OBS_BF16);
     }
 }
 
@@ -1350,7 +1397,7 @@ __global__ void __launch_bounds__(shape_max_threads(G, APL), 1) macm_step_kernel
         if (!TDM && ROLL) S.tgt()[i] = tg0[s];   // (a rollout stages it before its loop)
         // the flock actor steers by the target node of the last observation (bots.py:37-61)
         if (!TDM && R.policy() == MACM_BOT_FLOCK && valid[s]) {
-            const float4 o4 = reinterpret_cast<const float4*>(P.obs)[gi];   // polar only (macm_rollout checks)
+            const float4 o4 = reinterpret_cast<const float4*>(P.obs)[gi];   // fp32 polar only (macm_rollout checks)
             reinterpret_cast<float2*>(S.nw())[i] = make_float2(o4.z, o4.w);
         }
     }
@@ -2090,7 +2137,7 @@ __global__ void __launch_bounds__(shape_max_threads(G, APL), 1) macm_step_kernel
     const bool obs0 = ROLL && pass == 0 &&
                       (R_.fin.obs || R_.fin_k.obs || (!TDM && (R_.fin.nn_idx || R_.fin_k.nn_idx)));
     if (((last || R.obs() || R.policy() == MACM_BOT_FLOCK) && !(ROLL && pass == 0)) || obs0) {
-        float* ob_k = R.obs() ? R.obs() + (size_t)ks * EN * P.obs_dim : nullptr;
+        float* ob_k = R.obs() ? R.obs() + (size_t)ks * EN * P.obs_words : nullptr;
         int* nn_k = R.nn_idx() ? R.nn_idx() + (size_t)ks * EN : nullptr;
         float* ob1 = last ? P.obs : ob_k;
         float* ob2 = last ? ob_k : nullptr;
@@ -2100,7 +2147,7 @@ __global__ void __launch_bounds__(shape_max_threads(G, APL), 1) macm_step_kernel
         float2* tgo = (R.policy() == MACM_BOT_FLOCK && !last) ? reinterpret_cast<float2*>(S.nw()) : nullptr;
         if (ROLL && pass == 0) {
             ob1 = R_.fin.obs;
-            ob2 = R_.fin_k.obs ? R_.fin_k.obs + (size_t)ks * EN * P.obs_dim : nullptr;
+            ob2 = R_.fin_k.obs ? R_.fin_k.obs + (size_t)ks * EN * P.obs_words : nullptr;
             nn1 = R_.fin.nn_idx;
             nn2 = R_.fin_k.nn_idx ? R_.fin_k.nn_idx + (size_t)ks * EN : nullptr;
             tgo = nullptr;
@@ -2183,7 +2230,7 @@ __global__ void __launch_bounds__(128) macm_observe_kernel(const __grid_constant
     if (RESET) {
         if (!(mask ? mask[env] : P.done[env])) return;   // the whole group leaves together
         if (fin.obs || fin.nn_idx || fin.tdm || fin.es || fin2.obs || fin2.nn_idx || fin2.tdm || fin2.es) {
-            if (fin.obs || fin2.obs) copy_row<G>(g, P.obs, fin.obs, fin2.obs, env, P.N * P.obs_dim);
+            if (fin.obs || fin2.obs) copy_row<G>(g, P.obs, fin.obs, fin2.obs, env, P.N * P.obs_words);
             if (KIND != MACM_ENV_TDM && (fin.nn_idx || fin2.nn_idx)) copy_row<G>(g, P.nn_idx, fin.nn_idx, fin2.nn_idx, env, P.N);
             if (KIND == MACM_ENV_TDM && (fin.tdm || fin2.tdm)) copy_row<G>(g, P.tdm, fin.tdm, fin2.tdm, env, P.N * 4);
             if (fin.es || fin2.es) copy_row<G>(g, P.env_state, fin.es, fin2.es, env, 4);

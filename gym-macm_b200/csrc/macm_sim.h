@@ -34,7 +34,9 @@ struct SimConst {
     float k_sum, normal_mass;
     float binary_thr;   // fp32 d^2 threshold equivalent to sqrt64(d2) < reward_radius (mvmnt.py:177)
     float melee_dmg, init_health;
-    double rot_step;    // agent_rotation_speed * (1/hz)       (mvmnt.py:103-104)
+    int obs_dtype;      // MACM_OBS_*: element type of every observation store
+    int obs_words;      // 32-bit words per agent of an observation row: obs_dim (fp32) or obs_dim / 2 (16-bit)
+    double rot_step;   // agent_rotation_speed * (1/hz)       (mvmnt.py:103-104)
     double force;       // agent_force                           (mvmnt.py:113-116)
     double force_pen;   // agent_force * (1 - percent_mov_penalty) (combat.py:46-49)
     double diag;        // 1/np.sqrt(2)                          (mvmnt.py:112)

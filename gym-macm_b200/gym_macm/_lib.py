@@ -12,11 +12,13 @@ REWARD = {"binary": 0, "linear": 1}
 ACTION = {"discrete": 0, "continuous": 1}
 COORD = {"polar": 0, "cartesian": 1}
 DAMPING = {"taylor": 0, "pade": 1, "2.3.0": 0, "2.3.1": 1}
+OBS_F32, OBS_F16, OBS_BF16 = 0, 1, 2
+OBS_DTYPE = {"float32": OBS_F32, "float16": OBS_F16, "bfloat16": OBS_BF16}   # macm_params.obs_dtype; the torch dtype names
 ENV_FRESH, ENV_CONTACT_OVERFLOW, ENV_TOUCH_OVERFLOW = 1, 2, 4
 BOTS = {"idle": 0, "forward": 1, "rotate": 2, "diag": 3, "flock": 4, "random": 5, "combat": 6, "circle": 7}
 FLAG_REPAIR_MOV_COOLDOWN, FLAG_AUTO_RESET = 1, 2
 ENV_EPISODE_SHIFT = 8
-ABI_VERSION = 5
+ABI_VERSION = 6
 
 i32, f64, u64 = C.c_int32, C.c_double, C.c_uint64
 
@@ -35,7 +37,7 @@ class MacmParams(C.Structure):
         ("percent_mov_penalty", f64), ("init_health", f64),
         ("start_spread", f64), ("start_x", f64), ("start_y", f64), ("target_mindist", f64), ("target_maxdist", f64),
         ("world_width", f64), ("world_height", f64),
-        ("env_index_base", i32), ("reserved0", i32),
+        ("env_index_base", i32), ("obs_dtype", i32),
     ]
 
 

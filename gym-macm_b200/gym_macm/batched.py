@@ -26,6 +26,13 @@ def _as_list(n_agents):
     return [int(x) for x in n_agents]
 
 
+def obs_dtype_code(name):
+    """settings.obs_dtype -> MACM_OBS_*; ValueError for a name the library has no store for."""
+    if name not in _lib.OBS_DTYPE:
+        raise ValueError("obs_dtype must be one of %s, got %r" % (", ".join(_lib.OBS_DTYPE), name))
+    return _lib.OBS_DTYPE[name]
+
+
 def flock_params(settings, n_envs, n_agents, n_targets):
     """flockSettings -> macm_params (field-by-field; file:line in include/macm.h)."""
     p = _lib.default_params(_lib.FLOCK)
@@ -50,6 +57,7 @@ def flock_params(settings, n_envs, n_agents, n_targets):
     p.start_x, p.start_y = float(settings.start_point[0]), float(settings.start_point[1])
     p.target_mindist, p.target_maxdist = float(settings.target_mindist), float(settings.target_maxdist)
     p.env_index_base = int(settings.env_index_base)
+    p.obs_dtype = obs_dtype_code(settings.obs_dtype)
     if settings.auto_reset:
         p.flags |= _lib.FLAG_AUTO_RESET
     return p
@@ -78,6 +86,7 @@ def tdm_params(settings, n_envs, n_agents):
     p.percent_mov_penalty, p.init_health = float(settings.percent_mov_penalty), float(settings.init_health)
     p.world_width, p.world_height = float(settings.world_width), float(settings.world_height)
     p.env_index_base = int(settings.env_index_base)
+    p.obs_dtype = obs_dtype_code(settings.obs_dtype)
     return p
 
 
@@ -88,8 +97,8 @@ class Engine(object):
 
     _DTYPES = dict(posvel="float32", angsleep="float32", fat="float32", contact_ab="int32", contact_imp="float32",
                    contact_count="int32", env_state="int32", targets="float32", target_idx="uint8",
-                   tdm_state="float32", team="uint8", obs="float32", nn_idx="int32", rewards="float32",
-                   collided="uint8", done="uint8", touch_scratch="uint8")
+                   tdm_state="float32", team="uint8", nn_idx="int32", rewards="float32",
+                   collided="uint8", done="uint8", touch_scratch="uint8")   # obs: params.obs_dtype
 
     def __init__(self, params, device=None):
         torch = _torch()
@@ -125,6 +134,7 @@ class Engine(object):
                       contact_count=(E,), env_state=(E, 4), targets=(E, T, 2), target_idx=(N,), tdm_state=(E, N, 4),
                       team=(N,), obs=(E, N, D), nn_idx=(E, N), rewards=(E, N), collided=(E, N), done=(E,),
                       touch_scratch=(int(self.sizes.touch_scratch),))
+        dtypes = dict(self._DTYPES, obs={v: k for k, v in _lib.OBS_DTYPE.items()}[params.obs_dtype])
         self.t = {}
         bufs = _lib.MacmBuffers()
         # The per-step outputs live back to back in ONE device slab (each array 16-byte aligned), in the order
@@ -143,7 +153,7 @@ class Engine(object):
             nbytes = getattr(self.sizes, name)
             if nbytes == 0:
                 continue
-            dt = getattr(torch, self._DTYPES[name])
+            dt = getattr(torch, dtypes[name])
             if name in self._out_layout:
                 o = self._out_layout[name][0]
                 ten = slab[o:o + nbytes].view(dt).view(shapes[name])
@@ -415,6 +425,10 @@ class BatchedFlock(_BatchedCommon):
         obs["nodes"][0] = {"type": 0, "id": int32 [E,N],  "position": float32 [E,N,2|3]}   nearest agent
         obs["nodes"][1] = {"type": 1, "id": N,            "position": float32 [E,N,2|3]}   target
 
+    The "position" tensors (and `final_obs`, `rollout`'s obs / final_obs, `step_host`'s pinned obs) have the dtype of
+    the `obs_dtype` setting: float32 by default, or float16 / bfloat16 -- each fp32 value rounded once to nearest
+    even on the device.  Everything else (state, rewards, ids, done) is the same at every obs_dtype.
+
     `step(actions)` takes uint8 [E,N,4] (a0,a1,a2,pad) or any integer tensor [E,N,3] on the device
     (continuous mode: float32 [E,N,2]) and returns `(obs, rewards)` with rewards float32 [E,N].
     """
@@ -624,6 +638,9 @@ class BatchedTDM(_BatchedCommon):
         obs = {"myHealth": float32 [E,N], "myTeam": uint8 [N], "alive": bool [E,N],
                "agents": {"type": float32 [E,N,N] (1 ally, 0 enemy, -1 no entry),
                           "position": float32 [E,N,N,3] = r, theta, phi}}       (combat.py:211-226)
+
+    "type" and "position" (and `final_obs`, `rollout`'s obs / final_obs) have the dtype of the `obs_dtype` setting:
+    float32 by default, or float16 / bfloat16 -- each fp32 value rounded once to nearest even on the device.
 
     `step(actions)`: uint8 [E,N,4] = a0, a1, a2, attack (or any integer tensor of that shape);
     returns `(obs, rewards)`; rewards are -1 for an alive agent listed in a contact, else 0 (B12).

@@ -90,6 +90,10 @@ class TDM(_Base):
     def __init__(self, render="False", n_agents=[1, 1], actors=None, colors=None, device=None, **kwargs):
         if render is True:
             raise NotImplementedError("rendering stays with the reference's CPU backends")
+        if kwargs.get("obs_dtype", "float32") != "float32":
+            # the reference's dicts hold Python floats of the fp32 observation; a rounded one would not be it
+            raise ValueError("%s returns the reference's float observations: obs_dtype must be float32 "
+                             "(16-bit observations are for the batched classes)" % type(self).__name__)
         n_agents = _as_list(n_agents)
         nn = sum(n_agents)
         kwargs.setdefault("max_contacts", max(1, nn * (nn - 1) // 2))   # one world: full capacity (see mvmnt.Flock)

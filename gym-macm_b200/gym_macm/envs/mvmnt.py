@@ -109,6 +109,10 @@ class Flock(_Base):
     description = ("Flock")
 
     def __init__(self, n_agents=[10], actors=None, colors=None, targets=None, device=None, **kwargs):
+        if kwargs.get("obs_dtype", "float32") != "float32":
+            # the reference's dicts hold Python floats of the fp32 observation; a rounded one would not be it
+            raise ValueError("%s returns the reference's float observations: obs_dtype must be float32 "
+                             "(16-bit observations are for the batched classes)" % type(self).__name__)
         n_agents = _as_list(n_agents)
         # one world: room for every possible pair in the contact list and in the solver's stage, so that no pile
         # can run out of contact capacity (a batch trades that for shared memory, see BatchedFlock.overflowed)

@@ -31,7 +31,7 @@
 extern "C" {
 #endif
 
-#define MACM_ABI_VERSION 5
+#define MACM_ABI_VERSION 6
 #define MACM_MAX_AGENTS 128  /* per environment (the reference has no cap, mvmnt.py:61); up to 64: two agents per lane,
                                 beyond: four, with 128-bit contact adjacency rows */
 #define MACM_MAX_TARGETS 16
@@ -51,6 +51,10 @@ enum { MACM_ENV_FLOCK = 0, MACM_ENV_TDM = 1 };
 enum { MACM_REWARD_BINARY = 0, MACM_REWARD_LINEAR = 1 };
 enum { MACM_ACTION_DISCRETE = 0, MACM_ACTION_CONTINUOUS = 1 };
 enum { MACM_COORD_POLAR = 0, MACM_COORD_CARTESIAN = 1 };
+/* macm_params.obs_dtype: the element type of every observation the library stores.  The values are computed in fp32
+ * as always; a 16-bit type rounds each one once, to nearest even, at the store.  Nothing else changes: state,
+ * rewards, nn_idx, collided, done and the trajectory are those of MACM_OBS_F32. */
+enum { MACM_OBS_F32 = 0, MACM_OBS_F16 = 1, MACM_OBS_BF16 = 2 };
 /* Box2D <= 2.3.0: v *= clamp(1 - h*c, 0, 1);  Box2D >= 2.3.1: v *= 1 / (1 + h*c) */
 enum { MACM_DAMPING_TAYLOR = 0, MACM_DAMPING_PADE = 1 };
 /* macm_params.flags */
@@ -125,7 +129,7 @@ typedef struct macm_params {
     double world_width;           /* combat.py:76     30   TDM: x = U * (team + width/2), y = U * height */
     double world_height;          /* combat.py:77     30 */
     int32_t env_index_base;       /* global index of env 0 of this handle (shards of one batch); keys the samplers */
-    int32_t reserved0;
+    int32_t obs_dtype;            /* MACM_OBS_*: element type of `obs` and of every other observation destination */
 } macm_params;
 
 /* Caller-owned device buffers.  E = n_envs, N = n_agents, T = n_targets, C = max_contacts. */
@@ -145,7 +149,10 @@ typedef struct macm_buffers {
     /* ---- outputs (written by macm_step / macm_observe) ---- */
     float* obs;               /* Flock polar [E,N,4] = nn_dist nn_theta tgt_r tgt_theta;
                                  Flock cartesian [E,N,6] = nn_dist nn_cos nn_sin tgt_r tgt_cos tgt_sin;
-                                 TDM [E,N,N,4] = r theta phi type(1 ally, 0 enemy, -1 no entry)   16-byte aligned */
+                                 TDM [E,N,N,4] = r theta phi type(1 ally, 0 enemy, -1 no entry)   16-byte aligned.
+                                 With a 16-bit obs_dtype the member points at fp16 / bf16 elements of the same layout,
+                                 and the alignment is that of one record: 8 bytes (Flock polar, TDM) or 4 bytes (Flock
+                                 cartesian, 12-byte records).  The same holds for every other `obs` pointer below */
     int32_t* nn_idx;          /* [E,N] id of the nearest other agent (mvmnt.py:187-196); TDM: unused */
     float* rewards;           /* [E,N] */
     uint8_t* collided;        /* [E,N] agent appears in some world contact (mvmnt.py:162-164) */
@@ -158,7 +165,7 @@ typedef struct macm_buffers {
 typedef struct macm_buffer_sizes {
     uint64_t posvel, angsleep, fat, contact_ab, contact_imp, contact_count, env_state, targets,
              target_idx, tdm_state, team, obs, nn_idx, rewards, collided, done, touch_scratch;
-    int32_t obs_dim;          /* floats per agent in `obs` */
+    int32_t obs_dim;          /* values per agent in `obs` (`obs` bytes = E * N * obs_dim * element size of obs_dtype) */
     int32_t action_bytes;     /* bytes per agent in the `actions` argument of macm_step */
     int32_t max_contacts, max_touching;
 } macm_buffer_sizes;
@@ -226,7 +233,7 @@ int macm_reset_masked(macm_sim* sim, const uint8_t* mask, uint64_t seed, void* s
  * observation (a time-limit end is a truncation: a learner bootstraps from it) and its outcome (step count, overflow
  * bits, TDM winner; TDM health / alive).  Rows of envs that are not reset are left untouched.  Any member may be NULL. */
 typedef struct macm_final_out {
-    float* obs;        /* [E,N,obs_dim]  16-byte aligned */
+    float* obs;        /* [E,N,obs_dim]  obs_dtype elements, aligned as macm_buffers.obs (16 bytes in fp32) */
     int32_t* nn_idx;   /* [E,N]          Flock only */
     float* tdm_state;  /* [E,N,4]        TDM only, 16-byte aligned */
     int32_t* env_state;/* [E,4]          16-byte aligned */
@@ -251,14 +258,14 @@ int macm_step(macm_sim* sim, const void* actions, void* stream);
 
 /* Per-step outputs of macm_rollout: caller-owned device arrays with a leading step axis; any member may be NULL. */
 typedef struct macm_rollout_out {
-    float* obs;        /* [K,E,N,obs_dim]  16-byte aligned */
+    float* obs;        /* [K,E,N,obs_dim]  obs_dtype elements, aligned as macm_buffers.obs (16 bytes in fp32) */
     int32_t* nn_idx;   /* [K,E,N]          (Flock) */
     float* rewards;    /* [K,E,N] */
     uint8_t* collided; /* [K,E,N] */
     uint8_t* done;     /* [K,E] */
     /* Terminal rows of the envs reset after step k (MACM_FLAG_AUTO_RESET on and done[k][e] set), as macm_bind_final
      * describes; row [k][e] is written iff env e was reset after step k, every other row is left untouched. */
-    float* final_obs;        /* [K,E,N,obs_dim]  16-byte aligned */
+    float* final_obs;        /* [K,E,N,obs_dim]  obs_dtype elements, aligned as macm_buffers.obs (16 bytes in fp32) */
     int32_t* final_nn_idx;   /* [K,E,N]          Flock only */
     float* final_tdm_state;  /* [K,E,N,4]        TDM only, 16-byte aligned */
     int32_t* final_env_state;/* [K,E,4]          16-byte aligned */
@@ -276,7 +283,9 @@ typedef struct macm_rollout_out {
  *                     its own last observation, policy = MACM_BOT_* as in macm_bot_actions (MACM_BOT_FLOCK: Flock
  *                     with polar coordinates; MACM_BOT_COMBAT: TDM), draws keyed by (seed, env, agent, step_count).
  * With out == NULL or out->obs == NULL the observation pass only runs after the last step (action repeat /
- * frame skip); rewards of the intermediate steps are still available through out->rewards. */
+ * frame skip); rewards of the intermediate steps are still available through out->rewards.
+ * With a 16-bit obs_dtype, policy MACM_BOT_FLOCK returns MACM_E_UNSUPPORTED: its first step would steer by the rounded
+ * stored observation and so leave the fp32 trajectory.  MACM_BOT_COMBAT recomputes its row in fp32 and stays. */
 int macm_rollout(macm_sim* sim, const void* actions, int32_t n_steps, int32_t policy, uint64_t seed,
                  const macm_rollout_out* out, void* stream);
 
@@ -286,7 +295,9 @@ int macm_observe(macm_sim* sim, void* stream);
 /* test_scripts/bots.py on the device: writes one action per agent from the current `obs`
  * buffer (`actions=None` mode, mvmnt.py:86-92).  MACM_BOT_RANDOM draws U{0,1,2}^3 (x U{0,1}) and
  * MACM_BOT_CIRCLE its coin keyed by (seed, env, agent, step_count); MACM_BOT_COMBAT (TDM) faces, approaches and
- * strikes the nearest enemy of the agent's observation row (bots.py:3-16). */
+ * strikes the nearest enemy of the agent's observation row (bots.py:3-16).
+ * MACM_BOT_FLOCK and MACM_BOT_COMBAT read the stored `obs`; with a 16-bit obs_dtype they return MACM_E_UNSUPPORTED
+ * (a rounded observation would change their decisions).  The other policies do not read it and stay supported. */
 int macm_bot_actions(macm_sim* sim, int policy, uint64_t seed, void* actions_out, void* stream);
 
 /* Any little-endian integer array [E,N,width] (width 3 = a0 a1 a2, or 4 = + attack; elements of 1, 2, 4 or 8
