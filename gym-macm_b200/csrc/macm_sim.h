@@ -147,6 +147,13 @@ __device__ __forceinline__ float2 sample_target(const SampleConst& sc, uint64_t 
 }
 #endif
 
+// What the frame kernel (macm_render.cu) reads: the bound state and the geometry the Python settings hold in float64.
+struct RenderConst {
+    int E, N, T, kind;
+    double radius, reward_radius;    // macm_params.radius / reward_radius, metres
+    const float4* posvel; const float2* angsleep; const uint8_t* collided; const float4* tdm; const float2* targets;
+};
+
 // implemented in macm_kernels.cu
 cudaError_t macm_launch_cfg(const SimConst& P, int sm_count, LaunchCfg* cfg);
 cudaError_t macm_prepare_kernels(const SimConst& P, const LaunchCfg& cfg, int* blocks_per_sm);
@@ -163,3 +170,5 @@ cudaError_t macm_launch_sample(const SimConst& P, const SampleConst& sc, cudaStr
 cudaError_t macm_launch_overflow_count(const SimConst& P, int* d_out2, cudaStream_t s);
 cudaError_t macm_launch_pack_actions(const void* src, int elem_bytes, int width, uint64_t n_agents, void* out, cudaStream_t s);
 cudaError_t macm_launch_bot(const SimConst& P, int policy, uint64_t seed, void* actions_out, cudaStream_t s);
+// implemented in macm_render.cu (a translation unit of its own: the step kernels keep their register allocation)
+cudaError_t macm_launch_render(const RenderConst& R, const macm_render_args& a, cudaStream_t s);

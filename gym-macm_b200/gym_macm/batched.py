@@ -269,6 +269,13 @@ class Engine(object):
         _lib.check(_lib.lib().macm_bot_actions(self._h, int(policy), C.c_uint64(int(seed) & (2 ** 64 - 1)),
                                                C.c_void_p(out.data_ptr()), self._stream()), self._h)
 
+    def render(self, n_frames, height, width, envs, views, palette, out, stream=None):
+        """macm_render: `n_frames` frames [B,H,W,3] into `out`; envs (int32 [B] or None), views (float32 [B,3]),
+        palette (uint8 [N,2,3]) and out are device tensors."""
+        a = _lib.MacmRenderArgs(int(n_frames), int(height), int(width), None if envs is None else envs.data_ptr(),
+                                views.data_ptr(), palette.data_ptr(), out.data_ptr())
+        _lib.check(_lib.lib().macm_render(self._h, C.byref(a), self._stream(stream)), self._h)
+
     def pinned(self):
         """Pinned host mirrors of the action input and of every per-step output (for step_host)."""
         if self._pinned is None:
@@ -359,6 +366,36 @@ class _BatchedCommon(object):
         left, combat.py:171-182).  Fresh states drawn on the device, keyed by (seed, env, agent, episode)."""
         self.engine.reset_masked(mask, seed)
         return self.obs
+
+    def render(self, size, envs=None, views=None, out=None):
+        """Top-down RGB frames of envs of the batch, drawn on the device (macm_render): uint8 [B,H,W,3], row 0 at the
+        top, on the batch's stream.  Agents are solid circles (fill at half the colour, outline and heading axis in the
+        colour of gym_macm.render.palette), Flock targets white rings of radius `reward_radius`.
+
+        size:  (H, W), each 1..4096.
+        envs:  None = every env (frame b draws env b), or a list / range / int tensor of env indices (any order,
+               repeats allowed).  A CUDA tensor costs one host synchronisation to check.
+        views: None = render.fit_views (each frame holds its env's agents and targets), or [B,3] centre x, centre y,
+               half-width in metres.  A CUDA tensor costs one host synchronisation to check.
+        out:   a uint8 [B,H,W,3] CUDA tensor to draw into (reuse one frame buffer across steps), or None."""
+        from gym_macm import render
+        torch = _torch()
+        H, W = (int(x) for x in size)
+        if not (1 <= H <= 4096 and 1 <= W <= 4096):
+            raise ValueError("size must be (H, W) with each side in 1..4096, got %r" % (size,))
+        eng = self.engine
+        with torch.cuda.stream(eng.stream):   # None: torch's current stream
+            idx, B = render.env_index(self, envs)
+            v = render.fit_views(self, idx, (H, W)) if views is None else render.check_views(views, B, self.device)
+            if out is None:
+                out = torch.empty((B, H, W, 3), dtype=torch.uint8, device=self.device)
+            elif not (torch.is_tensor(out) and out.dtype == torch.uint8 and out.device == self.device and
+                      tuple(out.shape) == (B, H, W, 3) and out.is_contiguous()):
+                raise ValueError("out must be a contiguous uint8 tensor [%d, %d, %d, 3] on %s" % (B, H, W, self.device))
+            if getattr(self, "_palette", None) is None:
+                self._palette = torch.from_numpy(render.palette(self)).to(self.device)
+            eng.render(B, H, W, idx, v, self._palette, out)
+        return out
 
     def render_state(self, env=0):
         """One env of the batch as the objects the reference's CPU renderer reads

@@ -245,6 +245,15 @@ class Flock(_Base):
     def BeginContact(self, agent1, agent2):
         pass
 
+    def render(self, mode="rgb_array", size=(480, 640), view=None):
+        """This env as a top-down RGB picture drawn on the device: numpy uint8 [H,W,3] (size = (H, W)), row 0 at the
+        top.  view = (centre x, centre y, half-width in metres), or None to fit every agent and target.  Only mode
+        "rgb_array": the reference's pyglet window stays with its CPU backends."""
+        if mode != "rgb_array":
+            raise NotImplementedError("only render(mode=\"rgb_array\") is drawn here; the reference's pyglet window "
+                                      "stays with its CPU backends")
+        return self._batch.render(size, views=None if view is None else [view])[0].cpu().numpy()
+
     def render_state(self):
         """The objects the reference's CPU renderer reads (pyglet_framework.py:122-180), see gym_macm.render."""
         return self._batch.render_state(0)

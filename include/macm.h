@@ -31,7 +31,7 @@
 extern "C" {
 #endif
 
-#define MACM_ABI_VERSION 6
+#define MACM_ABI_VERSION 7
 #define MACM_MAX_AGENTS 128  /* per environment (the reference has no cap, mvmnt.py:61); up to 64: two agents per lane,
                                 beyond: four, with 128-bit contact adjacency rows */
 #define MACM_MAX_TARGETS 16
@@ -334,6 +334,32 @@ int macm_device_free(void* p);
  * cudaIpcMemHandle_t) for kernels running on `device`; *out receives the base address of the allocation. */
 int macm_ipc_open(const void* handle, int device, void** out);
 int macm_ipc_close(void* base);
+
+/* Top-down RGB frames of some envs of the batch: what the reference's renderer shows (bodies as solid circles with their
+ * heading axis, targets as white circles; see gym_macm/render.py), drawn on the device from the bound state.
+ * Frame b draws env e = envs[b] with view (cx, cy, hw) = views[b]: s = W / (2 hw) pixels per metre, a world point
+ * (x, y) lands on u = (x - cx) s + W/2, v = (cy - y) s + H/2 (world +y up, row 0 at the top), and pixel (row i,
+ * column j) is sampled at its centre (j + 0.5, i + 0.5).  The background is black; a pixel takes the colour of the last
+ * primitive that covers it, in this order:
+ *   every agent i = 0..N-1, centre c, radius rho = radius s, colour col = palette[i][alt] (alt: Flock `collided`,
+ *   TDM dead): the disc |p - c|^2 <= rho^2 in col >> 1 per channel, the outline (rho - 1)^2 < |p - c|^2 <= rho^2 in
+ *   col (rho < 1: the whole disc), then the heading axis, the pixels within 0.5 px of the segment from c to
+ *   c + rho (cos angle, -sin angle), in col;
+ *   Flock: every target t = 0..T-1 as an outline ring of radius reward_radius s in white.
+ * A frame whose env index lies outside [0, n_envs), or whose half-width is not a finite value > 0, is left black
+ * (envs and views are device data: the call does not read them on the host).  Reads the bound state, writes only
+ * `out`; one launch, no host synchronisation.  MACM_E_INVALID: a size out of range, a NULL views / palette / out, or
+ * envs == NULL with n_frames > n_envs; MACM_E_ALIGN: views or envs not 4-byte aligned; MACM_E_UNBOUND: before
+ * macm_bind. */
+typedef struct macm_render_args {
+    int32_t n_frames;        /* B >= 1 */
+    int32_t height, width;   /* H, W in 1..4096 */
+    const int32_t* envs;     /* [B] device: the env drawn in frame b; NULL = frame b draws env b (B <= n_envs) */
+    const float* views;      /* [B,3] device: centre x, centre y, half-width in metres of frame b (half-width > 0) */
+    const uint8_t* palette;  /* [N,2,3] device: per agent, the RGB bytes of its normal and of its alternate colour */
+    uint8_t* out;            /* [B,H,W,3] device, row 0 at the top */
+} macm_render_args;
+int macm_render(macm_sim* sim, const macm_render_args* a, void* stream);
 
 /* Number of kernels this handle has launched so far. */
 int64_t macm_launch_count(const macm_sim* sim);
