@@ -615,6 +615,26 @@ extern "C" int macm_render(macm_sim* sim, const macm_render_args* a, void* strea
     return MACM_OK;
 }
 
+extern "C" int macm_render_agents(macm_sim* sim, const macm_agent_frames_args* a, void* stream)
+{
+    if (!sim || !a) return MACM_E_INVALID;
+    if (!sim->bound) return MACM_E_UNBOUND;
+    if (a->n_envs < 1 || a->height < 1 || a->height > 1024 || a->width < 1 || a->width > 1024) return MACM_E_INVALID;
+    if (!(a->half_width > 0.0 && isfinite(a->half_width))) return MACM_E_INVALID;
+    if (!a->palette || !a->out || (!a->envs && a->n_envs > sim->K.E)) return MACM_E_INVALID;
+    if (a->envs && !aligned(a->envs, 4)) return MACM_E_ALIGN;
+    GUARD();
+    if (int rc = order_after_host(sim, (cudaStream_t)stream)) return rc;
+    const SimConst& K = sim->K;
+    const bool flock = K.kind == MACM_ENV_FLOCK;
+    const RenderConst R = {K.E, K.N, flock ? K.T : 0, K.kind, sim->params.radius, sim->params.reward_radius,
+                           K.posvel, K.angsleep, K.collided, K.tdm, K.targets};
+    CU(macm_launch_render_agents(R, *a, (cudaStream_t)stream));
+    sim->launches += 1;
+    note_device_work(sim, (cudaStream_t)stream);   // the host path must not overwrite the state before it is drawn
+    return MACM_OK;
+}
+
 extern "C" int macm_step_host_async(macm_sim* sim, const void* actions, float* obs, float* rewards, int32_t* nn_idx,
                                     uint8_t* collided, uint8_t* done)
 {

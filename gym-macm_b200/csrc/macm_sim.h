@@ -147,7 +147,7 @@ __device__ __forceinline__ float2 sample_target(const SampleConst& sc, uint64_t 
 }
 #endif
 
-// What the frame kernel (macm_render.cu) reads: the bound state and the geometry the Python settings hold in float64.
+// What the frame kernels (macm_render.cu) read: the bound state and the geometry the Python settings hold in float64.
 struct RenderConst {
     int E, N, T, kind;
     double radius, reward_radius;    // macm_params.radius / reward_radius, metres
@@ -172,3 +172,4 @@ cudaError_t macm_launch_pack_actions(const void* src, int elem_bytes, int width,
 cudaError_t macm_launch_bot(const SimConst& P, int policy, uint64_t seed, void* actions_out, cudaStream_t s);
 // implemented in macm_render.cu (a translation unit of its own: the step kernels keep their register allocation)
 cudaError_t macm_launch_render(const RenderConst& R, const macm_render_args& a, cudaStream_t s);
+cudaError_t macm_launch_render_agents(const RenderConst& R, const macm_agent_frames_args& a, cudaStream_t s);

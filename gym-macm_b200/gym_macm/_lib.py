@@ -18,7 +18,7 @@ ENV_FRESH, ENV_CONTACT_OVERFLOW, ENV_TOUCH_OVERFLOW = 1, 2, 4
 BOTS = {"idle": 0, "forward": 1, "rotate": 2, "diag": 3, "flock": 4, "random": 5, "combat": 6, "circle": 7}
 FLAG_REPAIR_MOV_COOLDOWN, FLAG_AUTO_RESET = 1, 2
 ENV_EPISODE_SHIFT = 8
-ABI_VERSION = 7
+ABI_VERSION = 8
 
 i32, f64, u64 = C.c_int32, C.c_double, C.c_uint64
 
@@ -78,13 +78,19 @@ class MacmRenderArgs(C.Structure):
                 ("envs", C.c_void_p), ("views", C.c_void_p), ("palette", C.c_void_p), ("out", C.c_void_p)]
 
 
+class MacmAgentFramesArgs(C.Structure):
+    _fields_ = [("n_envs", i32), ("height", i32), ("width", i32), ("half_width", f64),
+                ("envs", C.c_void_p), ("palette", C.c_void_p), ("out", C.c_void_p)]
+
+
 EXPORTS = ("macm_abi_version", "macm_strerror", "macm_last_cuda_error", "macm_params_default", "macm_create",
            "macm_destroy", "macm_get_buffer_sizes", "macm_get_launch_info", "macm_bind", "macm_reset",
            "macm_sample_reset", "macm_reset_masked", "macm_bind_final", "macm_set_auto_reset_seed", "macm_overflow_count", "macm_pack_actions",
            "macm_step", "macm_rollout", "macm_observe", "macm_bot_actions", "macm_step_host", "macm_step_host_async", "macm_host_sync",
            "macm_host_alloc",
            "macm_host_free", "macm_launch_count", "macm_set_trace", "macm_enable_peer_access", "macm_ipc_open",
-           "macm_ipc_close", "macm_device_alloc", "macm_device_free", "macm_render")
+           "macm_ipc_close", "macm_device_alloc", "macm_device_free", "macm_render",
+           "macm_render_agents")
 
 
 class MacmError(RuntimeError):
@@ -126,6 +132,7 @@ def lib():
         L.macm_observe.argtypes = [vp, vp]
         L.macm_bot_actions.argtypes = [vp, C.c_int, u64, vp, vp]
         L.macm_render.argtypes = [vp, C.POINTER(MacmRenderArgs), vp]
+        L.macm_render_agents.argtypes = [vp, C.POINTER(MacmAgentFramesArgs), vp]
         L.macm_step_host.argtypes = [vp] * 7
         L.macm_step_host_async.argtypes = [vp] * 7
         L.macm_host_sync.argtypes = [vp]

@@ -7,6 +7,7 @@ torch tensors (SoA, env-major) that the C ABI reads and writes in place; this mo
 arithmetic of its own and has no CPU path.
 """
 import ctypes as C
+import math
 
 import numpy as np
 
@@ -276,6 +277,13 @@ class Engine(object):
                                 views.data_ptr(), palette.data_ptr(), out.data_ptr())
         _lib.check(_lib.lib().macm_render(self._h, C.byref(a), self._stream(stream)), self._h)
 
+    def render_agents(self, n_envs, height, width, half_width, envs, palette, out, stream=None):
+        """macm_render_agents: every agent's frame of `n_envs` envs, [B,N,H,W,3] into `out`; envs (int32 [B] or
+        None), palette (uint8 [N,2,3]) and out are device tensors."""
+        a = _lib.MacmAgentFramesArgs(int(n_envs), int(height), int(width), float(half_width),
+                                     None if envs is None else envs.data_ptr(), palette.data_ptr(), out.data_ptr())
+        _lib.check(_lib.lib().macm_render_agents(self._h, C.byref(a), self._stream(stream)), self._h)
+
     def pinned(self):
         """Pinned host mirrors of the action input and of every per-step output (for step_host)."""
         if self._pinned is None:
@@ -395,6 +403,40 @@ class _BatchedCommon(object):
             if getattr(self, "_palette", None) is None:
                 self._palette = torch.from_numpy(render.palette(self)).to(self.device)
             eng.render(B, H, W, idx, v, self._palette, out)
+        return out
+
+    def render_agents(self, size, half_width, envs=None, out=None):
+        """Agent-centred RGB frames, drawn on the device (macm_render_agents): every agent's own view of its env,
+        centred on it with its heading pointing up and its right-hand side on the right -- uint8 [B,N,H,W,3], frame
+        (b, i) seen by agent i of env b (or envs[b]), row 0 at the top, on the batch's stream.  The drawing is that of
+        render(): agents as solid circles with their heading axis, Flock targets as white rings; a dead TDM agent keeps
+        its frame.  `gym_macm.render.write_gif(frames[:, b, i])` over a stack of steps animates one agent's view.
+
+        size:       (H, W), each 1..1024.
+        half_width: metres from the frame's centre to its left / right edge (finite, > 0); H / W sets the height.
+        envs:       None = every env, or a list / range / int tensor of env indices (any order, repeats allowed).  A
+                    CUDA tensor costs one host synchronisation to check.
+        out:        a uint8 [B,N,H,W,3] CUDA tensor to draw into (reuse one frame buffer across steps), or None."""
+        from gym_macm import render
+        torch = _torch()
+        H, W = (int(x) for x in size)
+        if not (1 <= H <= 1024 and 1 <= W <= 1024):
+            raise ValueError("size must be (H, W) with each side in 1..1024, got %r" % (size,))
+        hw = float(half_width)
+        if not (math.isfinite(hw) and hw > 0):
+            raise ValueError("half_width must be a finite value > 0, got %r" % (half_width,))
+        eng = self.engine
+        with torch.cuda.stream(eng.stream):   # None: torch's current stream
+            idx, B = render.env_index(self, envs)
+            shape = (B, eng.N, H, W, 3)
+            if out is None:
+                out = torch.empty(shape, dtype=torch.uint8, device=self.device)
+            elif not (torch.is_tensor(out) and out.dtype == torch.uint8 and out.device == self.device and
+                      tuple(out.shape) == shape and out.is_contiguous()):
+                raise ValueError("out must be a contiguous uint8 tensor %s on %s" % (list(shape), self.device))
+            if getattr(self, "_palette", None) is None:
+                self._palette = torch.from_numpy(render.palette(self)).to(self.device)
+            eng.render_agents(B, H, W, hw, idx, self._palette, out)
         return out
 
     def render_state(self, env=0):

@@ -31,7 +31,7 @@
 extern "C" {
 #endif
 
-#define MACM_ABI_VERSION 7
+#define MACM_ABI_VERSION 8
 #define MACM_MAX_AGENTS 128  /* per environment (the reference has no cap, mvmnt.py:61); up to 64: two agents per lane,
                                 beyond: four, with 128-bit contact adjacency rows */
 #define MACM_MAX_TARGETS 16
@@ -360,6 +360,32 @@ typedef struct macm_render_args {
     uint8_t* out;            /* [B,H,W,3] device, row 0 at the top */
 } macm_render_args;
 int macm_render(macm_sim* sim, const macm_render_args* a, void* stream);
+
+/* Agent-centred RGB frames: every agent's own view of its env, heading up, drawn on the device from the bound state
+ * (what a decentralised pixel policy sees).  Frame (b, i) looks at env e = envs[b] from agent i: its centre (cx, cy)
+ * is the agent's fp32 position, its heading ci = cos a_i, si = sin a_i (float64, of the fp32 body angle), and
+ * s = W / (2 half_width) pixels per metre.  A world point (x, y), dx = x - cx, dy = y - cy, lands on
+ *   u = W/2 + s (dx si - dy ci),   v = H/2 - s (dx ci + dy si),
+ * so the agent's heading points to the top of the frame and its right-hand side is on the right.  The heading axis
+ * of agent k (ck, sk) runs along the pixel direction (ck si - sk ci, -(ck ci + sk si)): agent i's own points straight
+ * up.  Everything else is macm_render's rules: pixel centres at (j + 0.5, r + 0.5); agents as discs at half the
+ * colour with an outline and a heading axis within 0.5 px, of radius rho = radius s and axis length rho; Flock
+ * targets as white rings of radius reward_radius s; palette[i][1] for a Flock agent in a contact or a dead TDM agent;
+ * a black background; the last primitive in painter's order (agents 0..N-1, then targets 0..T-1) wins.  A dead TDM
+ * agent still gets its frame: its body stays in the world.
+ * An env index outside [0, n_envs) gives N black frames and reads no state for that row (envs is device data: the
+ * call does not read it on the host).  Reads the bound state, writes only `out`; one launch, no host synchronisation.
+ * MACM_E_INVALID: a size out of range, a half_width that is not finite and > 0, a NULL palette / out, or envs == NULL
+ * with B > n_envs; MACM_E_ALIGN: envs not 4-byte aligned; MACM_E_UNBOUND: before macm_bind. */
+typedef struct macm_agent_frames_args {
+    int32_t n_envs;          /* B >= 1 envs; every agent of each gets a frame */
+    int32_t height, width;   /* H, W in 1..1024 */
+    double half_width;       /* metres from the frame centre to its left / right edge; finite, > 0 */
+    const int32_t* envs;     /* [B] device: env of frame row b; NULL = env b (B <= n_envs of the sim) */
+    const uint8_t* palette;  /* [N,2,3] device, as macm_render */
+    uint8_t* out;            /* [B,N,H,W,3] device: frame (b, i) is agent i of env envs[b], row 0 at the top */
+} macm_agent_frames_args;
+int macm_render_agents(macm_sim* sim, const macm_agent_frames_args* a, void* stream);
 
 /* Number of kernels this handle has launched so far. */
 int64_t macm_launch_count(const macm_sim* sim);
