@@ -635,6 +635,28 @@ extern "C" int macm_render_agents(macm_sim* sim, const macm_agent_frames_args* a
     return MACM_OK;
 }
 
+extern "C" int macm_lidar(macm_sim* sim, const macm_lidar_args* a, void* stream)
+{
+    if (!sim || !a) return MACM_E_INVALID;
+    if (!sim->bound) return MACM_E_UNBOUND;
+    if (a->n_envs < 1 || a->n_rays < 1 || a->n_rays > MACM_MAX_RAYS) return MACM_E_INVALID;
+    if (!(isfinite(a->max_range) && a->max_range > 0.0 && a->max_range <= 1e6)) return MACM_E_INVALID;
+    if (!(isfinite(a->fov) && a->fov > 0.0 && a->fov <= 2.0 * NP_PI)) return MACM_E_INVALID;
+    if (!a->fraction || (!a->envs && a->n_envs > sim->K.E)) return MACM_E_INVALID;
+    const SimConst& K = sim->K;
+    if ((a->envs && !aligned(a->envs, 4)) || (a->hit && !aligned(a->hit, 4)) ||
+        !aligned(a->fraction, K.obs_dtype == MACM_OBS_F32 ? 4 : 2))
+        return MACM_E_ALIGN;
+    GUARD();
+    if (int rc = order_after_host(sim, (cudaStream_t)stream)) return rc;
+    const RenderConst R = {K.E, K.N, K.kind == MACM_ENV_FLOCK ? K.T : 0, K.kind, sim->params.radius,
+                           sim->params.reward_radius, K.posvel, K.angsleep, K.collided, K.tdm, K.targets};
+    CU(macm_launch_lidar(R, *a, K.obs_dtype, (cudaStream_t)stream));
+    sim->launches += 1;
+    note_device_work(sim, (cudaStream_t)stream);   // the host path must not overwrite the state before it is scanned
+    return MACM_OK;
+}
+
 extern "C" int macm_step_host_async(macm_sim* sim, const void* actions, float* obs, float* rewards, int32_t* nn_idx,
                                     uint8_t* collided, uint8_t* done)
 {

@@ -173,3 +173,5 @@ cudaError_t macm_launch_bot(const SimConst& P, int policy, uint64_t seed, void* 
 // implemented in macm_render.cu (a translation unit of its own: the step kernels keep their register allocation)
 cudaError_t macm_launch_render(const RenderConst& R, const macm_render_args& a, cudaStream_t s);
 cudaError_t macm_launch_render_agents(const RenderConst& R, const macm_agent_frames_args& a, cudaStream_t s);
+// implemented in macm_lidar.cu (a translation unit of its own, for the same reason); obs_dtype: MACM_OBS_* of fraction
+cudaError_t macm_launch_lidar(const RenderConst& R, const macm_lidar_args& a, int obs_dtype, cudaStream_t s);

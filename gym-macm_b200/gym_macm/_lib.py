@@ -19,6 +19,7 @@ BOTS = {"idle": 0, "forward": 1, "rotate": 2, "diag": 3, "flock": 4, "random": 5
 FLAG_REPAIR_MOV_COOLDOWN, FLAG_AUTO_RESET = 1, 2
 ENV_EPISODE_SHIFT = 8
 ABI_VERSION = 8
+MAX_RAYS = 1024   # MACM_MAX_RAYS
 
 i32, f64, u64 = C.c_int32, C.c_double, C.c_uint64
 
@@ -83,6 +84,11 @@ class MacmAgentFramesArgs(C.Structure):
                 ("envs", C.c_void_p), ("palette", C.c_void_p), ("out", C.c_void_p)]
 
 
+class MacmLidarArgs(C.Structure):
+    _fields_ = [("n_envs", i32), ("n_rays", i32), ("max_range", f64), ("fov", f64),
+                ("envs", C.c_void_p), ("fraction", C.c_void_p), ("hit", C.c_void_p)]
+
+
 EXPORTS = ("macm_abi_version", "macm_strerror", "macm_last_cuda_error", "macm_params_default", "macm_create",
            "macm_destroy", "macm_get_buffer_sizes", "macm_get_launch_info", "macm_bind", "macm_reset",
            "macm_sample_reset", "macm_reset_masked", "macm_bind_final", "macm_set_auto_reset_seed", "macm_overflow_count", "macm_pack_actions",
@@ -90,7 +96,7 @@ EXPORTS = ("macm_abi_version", "macm_strerror", "macm_last_cuda_error", "macm_pa
            "macm_host_alloc",
            "macm_host_free", "macm_launch_count", "macm_set_trace", "macm_enable_peer_access", "macm_ipc_open",
            "macm_ipc_close", "macm_device_alloc", "macm_device_free", "macm_render",
-           "macm_render_agents")
+           "macm_render_agents", "macm_lidar")
 
 
 class MacmError(RuntimeError):
@@ -133,6 +139,7 @@ def lib():
         L.macm_bot_actions.argtypes = [vp, C.c_int, u64, vp, vp]
         L.macm_render.argtypes = [vp, C.POINTER(MacmRenderArgs), vp]
         L.macm_render_agents.argtypes = [vp, C.POINTER(MacmAgentFramesArgs), vp]
+        L.macm_lidar.argtypes = [vp, C.POINTER(MacmLidarArgs), vp]
         L.macm_step_host.argtypes = [vp] * 7
         L.macm_step_host_async.argtypes = [vp] * 7
         L.macm_host_sync.argtypes = [vp]

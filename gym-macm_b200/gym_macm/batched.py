@@ -284,6 +284,14 @@ class Engine(object):
                                      None if envs is None else envs.data_ptr(), palette.data_ptr(), out.data_ptr())
         _lib.check(_lib.lib().macm_render_agents(self._h, C.byref(a), self._stream(stream)), self._h)
 
+    def lidar(self, n_envs, n_rays, max_range, fov, envs, fraction, hit, stream=None):
+        """macm_lidar: every agent's scan of `n_envs` env rows into `fraction` [B,N,R] (obs dtype) and `hit` [B,N,R]
+        int32 (or None); envs (int32 [B] or None), fraction and hit are device tensors."""
+        a = _lib.MacmLidarArgs(int(n_envs), int(n_rays), float(max_range), float(fov),
+                               None if envs is None else envs.data_ptr(), fraction.data_ptr(),
+                               None if hit is None else hit.data_ptr())
+        _lib.check(_lib.lib().macm_lidar(self._h, C.byref(a), self._stream(stream)), self._h)
+
     def pinned(self):
         """Pinned host mirrors of the action input and of every per-step output (for step_host)."""
         if self._pinned is None:
@@ -438,6 +446,54 @@ class _BatchedCommon(object):
                 self._palette = torch.from_numpy(render.palette(self)).to(self.device)
             eng.render_agents(B, H, W, hw, idx, self._palette, out)
         return out
+
+    def lidar(self, n_rays, max_range, fov=2 * math.pi, envs=None, out=None, hits=True):
+        """Lidar scans, cast on the device (macm_lidar): every agent's fan of `n_rays` closest-hit ray casts around its
+        heading, each reporting how far it got and which agent it hit -- the TDM attack's ray cast (cm_framework.py:
+        56-86), once per ray.  Returns (fraction, hit) on the batch's stream: fraction [B,N,R] in the obs dtype, the
+        hit distance over max_range in [0, 1] with 1 for no hit; hit int32 [B,N,R], the agent id or -1 (None when
+        hits=False).  Row b scans env b (or envs[b]); ray r points at heading + fov * ((2r + 1 - R) / (2R)), counter-
+        clockwise, so with an odd R the middle ray points straight ahead.  A ray never reports the disc its origin
+        lies in; dead TDM agents are transparent, and still scan.  include/macm.h states the rule.
+
+        n_rays:    R in 1..1024.
+        max_range: L, metres (finite, > 0, at most 1e6).
+        fov:       the fan's width in radians (finite, 0 < fov <= 2 pi); 2 pi spaces the rays evenly all round.
+        envs:      None = every env, or a list / range / int tensor of env indices (any order, repeats allowed).  A
+                   CUDA tensor costs one host synchronisation to check.
+        out:       (fraction, hit) tensors to write into (reuse them across steps; hit None when hits=False), or None."""
+        from gym_macm import render
+        torch = _torch()
+        if isinstance(n_rays, bool) or not isinstance(n_rays, (int, np.integer)) or not 1 <= n_rays <= _lib.MAX_RAYS:
+            raise ValueError("n_rays must be an int in 1..%d, got %r" % (_lib.MAX_RAYS, n_rays))
+        L, fv = float(max_range), float(fov)
+        if not (math.isfinite(L) and 0 < L <= 1e6):
+            raise ValueError("max_range must be a finite value in (0, 1e6], got %r" % (max_range,))
+        if not (math.isfinite(fv) and 0 < fv <= 2 * math.pi):
+            raise ValueError("fov must be a finite value in (0, 2 pi], got %r" % (fov,))
+        if out is not None and not (isinstance(out, (tuple, list)) and len(out) == 2):
+            raise ValueError("out must be a (fraction, hit) pair")
+        eng = self.engine
+        with torch.cuda.stream(eng.stream):   # None: torch's current stream
+            idx, B = render.env_index(self, envs)
+            shape = (B, eng.N, int(n_rays))
+            def ok(t, dt):
+                return (torch.is_tensor(t) and t.dtype == dt and t.device == self.device and tuple(t.shape) == shape
+                        and t.is_contiguous())
+            fdt = eng.t["obs"].dtype
+            if out is None:
+                fraction = torch.empty(shape, dtype=fdt, device=self.device)
+                hit = torch.empty(shape, dtype=torch.int32, device=self.device) if hits else None
+            else:
+                fraction, hit = out
+                if not ok(fraction, fdt):
+                    raise ValueError("out[0] must be a contiguous %s tensor %s on %s" % (fdt, list(shape), self.device))
+                if hits and not ok(hit, torch.int32):
+                    raise ValueError("out[1] must be a contiguous int32 tensor %s on %s" % (list(shape), self.device))
+                if not hits:
+                    hit = None
+            eng.lidar(B, n_rays, L, fv, idx, fraction, hit)
+        return fraction, hit
 
     def render_state(self, env=0):
         """One env of the batch as the objects the reference's CPU renderer reads

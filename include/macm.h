@@ -387,6 +387,41 @@ typedef struct macm_agent_frames_args {
 } macm_agent_frames_args;
 int macm_render_agents(macm_sim* sim, const macm_agent_frames_args* a, void* stream);
 
+/* Lidar scans: every agent's fan of R closest-hit ray casts around its heading, cast on the device from the bound
+ * state (the range sensor of swarm policies).  Row b scans env e = envs[b] (env b when envs is NULL).  For agent i of
+ * that env and ray r = 0..R-1:
+ *   origin     p1 = the agent's fp32 centre (x, y);
+ *   direction  float64, in this order: o_r = fov * ((double)(2r + 1 - R) / (double)(2R)), th = (double)a_i + o_r
+ *              (a_i the fp32 body angle), dx = (float)(L * cos(th)), dy = (float)(L * sin(th)), L = max_range;
+ *   end        p2 = (x + dx, y + dy), added in fp32 (the TDM attack's ray, with L for melee_range).
+ * The fan is symmetric about the heading (cos a_i, sin a_i); r counts counter-clockwise, and with an odd R the middle
+ * ray points straight ahead.  The hit is the closest-hit cast of the step's TDM attack (cm_framework.py:56-86):
+ * b2CircleShape::RayCast in fp32 and Box2D's operation order, with the fp32 radius and maxFraction 1, against every
+ * body that has a proxy -- a dead TDM agent has none, so rays pass through it (a dead agent still scans: its body
+ * stays in the world).  The smallest fraction wins; among equal fractions, the lowest agent index.  Nothing special-
+ * cases the caster: a ray whose origin lies inside a disc (in the fp32 arithmetic, |p1 - c|^2 < radius^2) gets
+ * a = -(c + sqrt(sigma)) <= 0 from it, so the disc is never reported at a fraction above 0.  The caster's own disc
+ * (p1 - c = 0, a < 0) is never reported at all; a neighbour's disc holding the origin is reported only at fraction
+ * +-0, when the origin sits on its rim to within rounding.
+ * Output: fraction[b][i][r] in [0, 1], 1 = no hit, computed in fp32 and rounded once, to nearest even, to the sim's
+ * obs_dtype at the store (it is an observation); hit[b][i][r] = the agent id hit, or -1 (int32, like nn_idx).
+ * An env index outside [0, n_envs) gives a row of misses (fraction 1, hit -1) and reads no state for that row (envs
+ * is device data: the call does not read it on the host).  Reads the bound state, writes only its outputs; one
+ * launch, no host synchronisation.
+ * MACM_E_INVALID: an argument out of range, a NULL fraction, or envs == NULL with B > n_envs; MACM_E_ALIGN: envs or
+ * hit not 4-byte aligned, or fraction not aligned to its element; MACM_E_UNBOUND: before macm_bind. */
+#define MACM_MAX_RAYS 1024
+typedef struct macm_lidar_args {
+    int32_t n_envs;          /* B >= 1 env rows; every agent of each gets a scan */
+    int32_t n_rays;          /* R in 1..MACM_MAX_RAYS */
+    double max_range;        /* L, metres: finite, > 0, <= 1e6 */
+    double fov;              /* radians: finite, 0 < fov <= 2 pi */
+    const int32_t* envs;     /* [B] device, or NULL = env b (B <= n_envs of the sim) */
+    void* fraction;          /* [B,N,R] obs_dtype elements */
+    int32_t* hit;            /* [B,N,R] device, or NULL */
+} macm_lidar_args;
+int macm_lidar(macm_sim* sim, const macm_lidar_args* a, void* stream);
+
 /* Number of kernels this handle has launched so far. */
 int64_t macm_launch_count(const macm_sim* sim);
 
